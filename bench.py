@@ -15,6 +15,10 @@ batch of B = 256 independent hyper-parameter draws per GPU on synthetic inputs (
 
 `--impl reference` times the reference's CPU path instead: the reference itself (R + Stan Math +
 Eigen) cannot be built or run in this image, so this is the oracle port (kind "port").
+
+`--dump-outputs DIR` writes what the last timed step returned to DIR/lml.npy (draws,), DIR/grad.npy
+(draws, 3) and DIR/info.npy (draws,), all float64, draws of every rank in rank order.  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -210,6 +214,31 @@ def cpu_reference_evals_per_sec(n_evals, threads):
     return n_evals / dt, dt, out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, outputs, world, rank):
+    """Writes the device tensors `outputs` (name -> tensor with the draws on axis 0) as float64 .npy files under
+    `path`, each gathered over the ranks in rank order; rank 0 writes."""
+    import numpy as np
+    import torch
+    import torch.distributed as dist
+    host = {}
+    for name, t in outputs.items():
+        if world > 1:
+            parts = [torch.empty_like(t) for _ in range(world)]
+            dist.all_gather(parts, t.contiguous())
+            t = torch.cat(parts)
+        host[name] = t.cpu().numpy().astype(np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit; use fewer --draws" % (total, DUMP_LIMIT_BYTES))
+    if rank == 0:
+        os.makedirs(path, exist_ok=True)
+        for name, a in host.items():
+            np.save(os.path.join(path, name + ".npy"), a)
+
+
 def run_reference(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
@@ -249,7 +278,11 @@ def main():
     ap.add_argument("--impl", default="gpb200", choices=["gpb200", "reference"])
     ap.add_argument("--draws", type=int, default=DRAWS_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write lml, grad and info of the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -324,6 +357,8 @@ def main():
     value = world * B * K / (ms_max * 1e-3)
     assert int(dinfo.abs().sum().item()) == 0, "a synthetic draw was not positive definite"
     lml_dev = dlml.cpu().numpy().copy()
+    if args.dump_outputs:   # before the LML-only pass below overwrites dlml
+        dump_outputs(args.dump_outputs, {"lml": dlml, "grad": dgrad, "info": dinfo}, world, rank)
 
     # ---------------- second half of BASELINE's metric: Cholesky FP64 TFLOP/s vs peak ------------
     # the LML-only pass (Gram -> tiled Cholesky -> forward substitution -> log-det/quadratic form) of
