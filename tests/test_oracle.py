@@ -286,3 +286,66 @@ def test_oracle_properties_hold_for_random_inputs():
         assert info == 0 and abs(cv - v) <= 1e-10 * max(1.0, abs(v)) and np.max(np.abs(cg - g)) <= 1e-8 * max(1.0, np.max(np.abs(g)))
 
     check()
+
+
+# ---- extended-precision references of the Cholesky derivatives (oracle/chol_deriv_ext.py) ---------------------
+def _need_longdouble():
+    from oracle import chol_deriv_ext as X
+    if not X.LONGDOUBLE_OK:
+        pytest.skip("np.longdouble has %d mantissa bits here; the dual LLT reference needs 63" % np.finfo(np.longdouble).nmant)
+    return X
+
+
+def test_longdouble_dual_llt_matches_float64_duals_and_mpmath():
+    X = _need_longdouble()
+    from oracle import gp_oracle_mp as m
+    # rbf_cov_chol's inputs: the float64 literal duals agree to rounding
+    xs = np.random.default_rng(4).permutation(30).astype(float)
+    L, dL = X.chol_tangent(xs, 1.0, 0.7, o.RBF_JITTER, "rho")
+    L2, dL2 = o.rbf_cov_chol_dual(xs, 0.7)
+    assert relerr(L, L2) < 1e-14 and relerr(dL, dL2) < 1e-13
+    # dense SE inputs, both tangents: the 50-digit duals agree to the float64 rounding of the result
+    x = np.sort(np.random.default_rng(5).uniform(0, 10, 36))
+    for wrt in ("alpha", "rho"):
+        L, dL = X.chol_tangent(x, 1.3, 2.0, 0.1, wrt)
+        Lm, dLm = m.chol_tangent(x, 1.3, 2.0, 0.1, wrt)
+        assert relerr(L, Lm) < 4e-16 and relerr(dL, dLm) < 4e-16, wrt
+        assert np.all(np.triu(L, 1) == 0) and np.all(np.triu(dL, 1) == 0)
+
+
+def test_longdouble_dual_llt_matches_closed_form_at_n300():
+    X = _need_longdouble()
+    x = np.sort(np.random.default_rng(6).uniform(0, 10, 300))
+    for wrt in ("alpha", "rho"):
+        L, dL = X.chol_tangent(x, 1.3, 2.0, 0.1, wrt)
+        Lc, dLc = X.chol_tangent_closed_form(*X.se_gram_tangent(x, 1.3, 2.0, 0.1, wrt))
+        assert relerr(L, Lc) < 1e-13 and relerr(dL, dLc) < 1e-12, wrt
+    assert X.far_tile_share(L) >= 1e-2 and X.far_tile_share(dL) >= 1e-2
+
+
+def test_latent_adjoint_matches_central_differences():
+    from oracle import chol_deriv_ext as X
+    rng = np.random.default_rng(7)
+    n, theta, da = 200, np.array([1.3, 1.5]), 0.1
+    x = np.sort(rng.uniform(0, 10, n))
+    z = rng.standard_normal((3, n)); fbar = rng.standard_normal((3, n))
+    r = X.latent_adjoint(x, *theta, da, z, fbar)
+    L = o.cholesky_decompose(o.gram_se(x, *theta, da))
+    assert relerr(r["L"], L) == 0.0 and relerr(r["f"], z @ L.T) < 1e-15 and relerr(r["zbar"], fbar @ L) < 1e-15
+
+    def objective(th):   # sum_m fbar_m^T L(theta) z_m
+        Lt = o.cholesky_decompose(o.gram_se(x, th[0], th[1], da))
+        return float(np.sum(fbar * (z @ Lt.T)))
+    for k in range(2):
+        h = 1e-6 * theta[k]
+        tp, tm = theta.copy(), theta.copy()
+        tp[k] += h; tm[k] -= h
+        fd = (objective(tp) - objective(tm)) / (2 * h)
+        assert abs(fd - r["theta_bar"][k]) <= 1e-6 * r["scale"][k], (k, fd, r["theta_bar"][k], r["scale"][k])
+        assert r["scale"][k] >= abs(r["theta_bar"][k])
+    # the symmetrised adjoint of gp_oracle.exact_gp_lp_grad gives the same rho component for nvec = 1
+    y = rng.standard_normal(n)
+    _, g = o.exact_gp_lp_grad(x, y, 1.0, 0.3, z[0], jitter=da)
+    f = o.cholesky_decompose(o.gram_se(x, 1.0, 1.0, da)) @ z[0]
+    r1 = X.latent_adjoint(x, 1.0, 1.0, da, z[0], (y - f) / 0.3 ** 2)
+    assert abs(r1["theta_bar"][1] - (g["l"] - 3.0 + 4.0)) <= 1e-10 * r1["scale"][1]
