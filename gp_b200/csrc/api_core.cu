@@ -27,6 +27,7 @@ void free_handle(gpb200_handle_s *h) {
   if (h->latent_L) cudaFree(h->latent_L);
   if (h->info_slot) cudaFree(h->info_slot);
   if (h->panel_flags) cudaFree(h->panel_flags);
+  if (h->flops_dev) cudaFree(h->flops_dev);
   for (auto &kv : h->task_cache) cudaFree(kv.second.first);
   for (auto &kv : h->split_cache) if (kv.second.reg) cudaFree(kv.second.reg);
   delete h;
@@ -86,6 +87,10 @@ extern "C" int gpb200_create(gpb200_handle_t *out, int device) {
   if (fc && fc[0] == '0') h->fine_cfg = 0;
   const char *pf = getenv("GPB200_PANEL_FUSED");
   if (pf && pf[0] == '0') h->panel_fused = 0;
+  const char *ev = getenv("GPB200_ENVELOPE");  // 0: the dense SE route (reference for tests)
+  if (ev && ev[0] == '0') h->envelope = 0;
+  const char *sm = getenv("GPB200_SINV_MINB");
+  if (sm && sm[0] >= '0' && sm[0] <= '9') h->sinv_min_batch = atoi(sm);
   const char *ng = getenv("GPB200_NO_GRAPH");
   if (ng && ng[0] == '1') h->graphs_enabled = 0;
   *out = h;
@@ -578,12 +583,26 @@ extern "C" int gpb200_debug_panel_trace(gpb200_handle_t h, long long *out2048) {
   return panel_trace_fetch(out2048);
 }
 
-// Accounting of the flops the DMMA GEMM launches really execute (host-side, from the task lists: 2 * tile area * k per CTA
-// after the CTA-uniform skipping).  on != 0 resets the counter and starts counting; the getter returns the running total.
+// Accounting of the flops the DMMA GEMM launches really execute: 2 * tile area * k per CTA after the CTA-uniform skipping.
+// Launches whose skipping is fixed by the task lists are counted on the host; launches that skip tiles outside an item's
+// envelope count on the device, per CTA, into a counter the getter reads back (it waits for the handle's stream).
+// on != 0 resets the counter and starts counting; the getter returns the running total.
 extern "C" int gpb200_set_flop_counting(gpb200_handle_t h, int on) {
-  if (!h) return -1;
+  CHECK_H(h);
   h->count_flops = on ? 1 : 0;
   h->executed_gemm_flops = 0.0;
+  if (on) {
+    if (!h->flops_dev) GPB_CUDA(h, cudaMalloc(&h->flops_dev, sizeof(unsigned long long)));
+    GPB_CUDA(h, cudaMemsetAsync(h->flops_dev, 0, sizeof(unsigned long long), h->stream));
+  }
   return 0;
 }
-extern "C" double gpb200_executed_gemm_flops(gpb200_handle_t h) { return h ? h->executed_gemm_flops : 0.0; }
+extern "C" double gpb200_executed_gemm_flops(gpb200_handle_t h) {
+  if (!h) return 0.0;
+  DeviceGuard guard(h->device);
+  unsigned long long dev = 0;
+  if (h->flops_dev && (cudaMemcpyAsync(&dev, h->flops_dev, sizeof(dev), cudaMemcpyDeviceToHost, h->stream) != cudaSuccess ||
+                       cudaStreamSynchronize(h->stream) != cudaSuccess))
+    dev = 0;
+  return h->executed_gemm_flops + (double)dev;
+}

@@ -37,9 +37,20 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
     return launch_lml_small(h, n, x, x_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info, B);
   }
   const int zks = trmv_split_chunks(np, B);  // k-chunks of the split z = W y (small batches only)
-  const size_t per_item = small ? 0 : pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * pw * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) + 64;
+  // SE covariance: the tile envelope of every item (F, E; solve.cu) bounds the Cholesky, and larger batches compute the
+  // gradient from the selected inverse instead of the explicit inverse + W^T W.  Measured on a B200 (1000 W), LML +
+  // gradient per call on the bench.py family, dense / envelope + explicit inverse / envelope + selected inverse, ms:
+  //   N = 1024: B = 1 0.452 / 0.458 / 0.85,  B = 32 2.10 / 1.98 / 2.12   (nt = 8: the band covers the matrix, the
+  //             profile costs its launch; no envelope below 16 tile rows)
+  //   N = 2048: B = 1 0.948 / 0.949 / 2.34,  B = 8 3.46 / 2.93 / 3.70,  B = 16 6.26 / 5.20 / 4.96,  B = 32 11.0 / 9.59 / 7.67
+  //   N = 4096: B = 1 3.36 / 2.98 / 4.59,    B = 4 10.19 / 7.91 / 8.36,  B = 8 19.3 / 14.4 / 8.2,  B = 32 70.9 / 53.4 / 22.0
+  // The selected inverse is a chain of 2 nt launches of a few tiles per item: it wins once B * nt >= 256.
+  const bool use_env = !sp.deriv && h->envelope && !small && nt >= 16 && nt <= ENV_MAX_NT;
+  const bool sinv = use_env && want_grad && (h->sinv_min_batch > 0 ? B >= h->sinv_min_batch : (long long)B * nt >= 256);
+  const size_t per_item = small ? 0 : pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * pw * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) + 64 +
+                                      (use_env ? (size_t)2 * nt * sizeof(int) : 0);
   const size_t fixed = pad256((size_t)B * (x_stride ? ng : 0) * 8 + ng * 8) + pad256((size_t)B * (y_stride ? n : 0) * 8 + n * 8) +
-                       2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096;
+                       2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096 + (use_env ? 256 : 0);
   int Bc = B;
   if (!small && (h->ws_limit > 0 || fixed + per_item * (size_t)B + 8192 > h->ws_bytes)) {
     size_t limit = (size_t)h->ws_limit;
@@ -62,11 +73,13 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   double *dlml = a.take<double>(B), *dgrad = a.take<double>((size_t)B * ts);
   int *dinfo = a.take<int>(B);
   double *Lbuf = nullptr, *Sbuf = nullptr, *zbuf = nullptr, *abuf = nullptr, *dvec = nullptr, *partial = nullptr, *zpart = nullptr;
+  int *env = nullptr;
   if (!small) {
     Lbuf = a.take<double>((size_t)Bc * mat); Sbuf = a.take<double>((size_t)Bc * mat);
     zbuf = a.take<double>((size_t)Bc * np); abuf = a.take<double>((size_t)Bc * np); dvec = a.take<double>((size_t)Bc * np);
     partial = a.take<double>((size_t)Bc * nparts * pw);
     zpart = zks > 1 ? a.take<double>((size_t)Bc * zks * np) : nullptr;
+    if (use_env && !(env = a.take<int>((size_t)Bc * 2 * nt))) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
     if (!partial) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
   }
   if (!dinfo) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
@@ -79,10 +92,22 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       const int bc = std::min(Bc, B - b0);
       const double *cx = dx + (long long)b0 * xs, *cy = dy + (long long)b0 * ys, *cth = dth + (long long)b0 * ts;
       if (sp.deriv) RC(launch_gram_deriv_batched(h, ng, sp.order0, sp.nblocks, np, cx, xs, cth, ts, jitter, 1, Lbuf, mat, bc));
-      else RC(launch_gram_se_batched(h, n, np, cx, xs, cth, jitter, 1, Lbuf, mat, bc));
-      RC(chol_batched(h, Lbuf, np, mat, n, bc, dinfo + b0));
+      else {
+        if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
+        RC(launch_gram_se_batched(h, n, np, cx, xs, cth, jitter, 1, Lbuf, mat, bc, env));
+        if (env) RC(launch_envelope_profile(h, nt, env, bc));
+      }
+      RC(chol_batched(h, Lbuf, np, mat, n, bc, dinfo + b0, env));
       RC(extract_diag(h, np, Lbuf, mat, dvec, bc));
-      if (want_grad) {
+      int n1 = 0, n2 = 0;
+      if (sinv) {
+        RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
+        RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, np, bc, env));
+        RC(launch_backsub_band(h, np, Lbuf, Sbuf, mat, env, zbuf, abuf, bc));
+        RC(sinv_batched(h, Lbuf, Sbuf, np, mat, env, bc));
+        RC(launch_trace_sinv(h, n, np, Lbuf, mat, env, cx, xs, abuf, cth, partial, bc));
+        n1 = ntasks;
+      } else if (want_grad) {
         RC(trtri_batched(h, Lbuf, Sbuf, np, mat, bc));
         if (zks > 1 && zpart) RC(launch_trmv_lower_n_split(h, np, zks, Lbuf, mat, cy, ys, n, zpart, zbuf, np, bc));
         else RC(launch_trmv_lower_n(h, np, Lbuf, mat, cy, ys, n, zbuf, np, bc));
@@ -102,11 +127,10 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
         RC(launch_gemm(h, LAYOUT_TN, sp.deriv ? EPI_TRACE_DERIV : EPI_TRACE, p, ntasks, bc));
       } else {
         RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
-        if (bc >= 32) RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, np, bc));
+        if (bc >= 32) RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, np, bc, env));
         else RC(launch_trsv_sweep(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, abuf, np, bc));
       }
-      int n1 = 0, n2 = 0;
-      RC(gemm_partial_layout(h, tl.at(0), ntasks, bc, &n1, &n2));
+      if (!sinv) RC(gemm_partial_layout(h, tl.at(0), ntasks, bc, &n1, &n2));
       if (sp.deriv)
         RC(launch_finalize_deriv(h, ng, sp.nblocks, np, want_grad, dvec, zbuf, abuf, partial, n1, n2, cth, dlml + b0,
                                  dgrad + (long long)b0 * ts, bc));
@@ -139,7 +163,8 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       memcpy(&jbits, &jitter, sizeof(jbits));
       const std::vector<long long> key = {n, B, want_grad, xs, ys, jbits, (long long)(uintptr_t)h->ws, h->chol_panel_override,
                                           sp.deriv, sp.order0, sp.nblocks, h->gemm_cfg_override, h->lookahead, h->lookahead_max_batch,
-                                          h->panel_impl, h->trsm_mt_override, h->quarter_below_waves, h->trsm_pipelined, h->panel_fused, h->fine_cfg};
+                                          h->panel_impl, h->trsm_mt_override, h->quarter_below_waves, h->trsm_pipelined, h->panel_fused, h->fine_cfg,
+                                          h->envelope, h->sinv_min_batch};
       auto it = h->graphs.find(key);
       if (it == h->graphs.end()) {
         // task lists allocate and synchronise on first use, which a capture does not allow: a first uncaptured

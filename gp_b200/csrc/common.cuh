@@ -11,6 +11,7 @@ namespace gpb {
 
 constexpr int PANEL_FUSED_MAX_BATCH = 148;  // matrices per panel_fused_kernel launch (flag slots in the handle)
 constexpr int TILE = 128;  // tile edge of every tiled algorithm (internal matrices are padded to it)
+constexpr int ENV_MAX_NT = 512;  // tile rows of a matrix with a tile envelope (the GEMM stages one half of it in shared memory)
 
 inline int round_up(int n, int m) { return (n + m - 1) / m * m; }
 
@@ -61,7 +62,18 @@ struct GemmParams {
   // n_grid x n_grid; block b carries derivative order order0 + b; theta is B x theta_stride
   int n_grid, order0, theta_stride;
   int latency_hint;   // 1: this launch sits on a dependent chain (look-ahead Cholesky): small launches take the 16-warp fine tiles
+  // tile envelope of a banded covariance (ENV_* below): per item env[0..nt) = F (first nonzero tile column of each
+  // tile row), env[nt..2nt) = E (last tile row I with F_I <= J, per tile column J); item stride 2 * env_nt
+  const int *env;
+  int env_nt, env_mode;
+  MatRef CT;                    // EPI_AXPBY: when CT.p is set the transpose of the output tile is written there too
+  unsigned long long *flops;    // when set: every CTA adds the flops it executes (after all skipping)
 };
+// envelope modes of the tile GEMM.  Only products with an exactly-zero operand tile are dropped, and the k order of
+// the rest is kept, so a result is bit-identical to the dense launch (up to the sign of an all-zero tile).
+enum { ENV_NONE = 0,
+       ENV_CHOL = 1,   // C(I,J) -= L(I,k) L(J,k)^T: exit when J < F_I (tile outside the profile), k starts at max(F_I, F_J)
+       ENV_BAND = 2 }; // selected inverse: exit when I > E_J, the contraction ends at tile E_J
 
 struct Handle {
   int device = 0;
@@ -89,6 +101,9 @@ struct Handle {
   int diag_split = 1;           // large batches: symmetric diagonal tiles run as 64x64 quarter CTAs in their own launch (env GPB200_DIAG_SPLIT)
   int count_flops = 0;
   double executed_gemm_flops = 0.0;  // flops the DMMA GEMM launches actually executed (after CTA-level skipping)
+  unsigned long long *flops_dev = nullptr;  // the same for launches whose skipping is decided on the device (envelope)
+  int envelope = 1;             // SE path: envelope Cholesky and selected inverse (env GPB200_ENVELOPE=0: dense reference route)
+  int sinv_min_batch = 0;       // 0: selected inverse for the gradient when B * nt >= 256 (api_gp.cu); > 0: from this batch size (env GPB200_SINV_MINB)
   // CUDA graphs of the launch sequence of small (launch-latency-bound) LML evaluations, keyed by the
   // problem signature; replayed on a handle-owned stream (the caller's stream may be the legacy
   // default stream, which cannot be captured).  Invalidated when the workspace moves.
@@ -217,6 +232,13 @@ int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int 
                       int *info);
 int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l_off, long long l_step, double *W,
                            long long w_off, long long w_step, long long stride, int ntiles, int batch);
+// tile envelope of the SE path (solve.cu): E from F (F filled by gram_se_batched), the trace of the selected inverse
+// and the band-limited back substitution
+int launch_envelope_profile(Handle *h, int nt, int *env, int batch);
+int launch_trace_sinv(Handle *h, int n, int np, const double *Z, long long stride, const int *env, const double *x,
+                      long long x_stride, const double *a, const double *theta, double *partial, int batch);
+int launch_backsub_band(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const int *env,
+                        const double *z, double *a, int batch);
 int panel_smem_setup(Handle *h);
 int panel_trace_fetch(long long *out2048);  // instrumented builds (-DGPB_PANEL_TRACE) only
 

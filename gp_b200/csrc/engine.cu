@@ -165,7 +165,15 @@ int tasks_lauum(Handle *h, int nt, TaskList *out) {
 // engines on padded device buffers
 // ---------------------------------------------------------------------------------------------
 
-// Batched tiled Cholesky, in place on Lbuf (np x np per item, lower tiles valid on entry).
+static void set_env(GemmParams &p, const int *env, int nt, int mode) {
+  p.env = env;
+  p.env_nt = nt;
+  p.env_mode = env ? mode : ENV_NONE;
+}
+
+// Batched tiled Cholesky, in place on Lbuf (np x np per item, lower tiles valid on entry).  With a tile envelope
+// (env, see ENV_CHOL) every update CTA starts its contraction at the first tile where both operand rows can be nonzero
+// and exits when its output tile lies left of the profile: L is bit-identical to the dense factorisation.
 // Panel width: pure left-looking when the batch alone fills the GPU, 8-tile (1024-column) panels
 // with right-looking trailing updates otherwise.
 int chol_panel_tiles(int nt, int batch) {
@@ -216,7 +224,7 @@ int chol_lookahead_panel(const Handle *h, int nt) {
 // so panel p+1 is factored while the bulk of panel p's trailing update still runs.  Every write to a block column
 // is ordered: before P updates the next panel's columns it waits for T's previous trailing update, which was the
 // last launch to write them; T's updates follow one another in stream order.
-static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev) {
+static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env) {
   const int nt = np / TILE, pt = chol_lookahead_panel(h, nt);
   TaskList tl, tr, la1, la2;
   int rc = tasks_chol(h, nt, pt, &tl, &tr);
@@ -230,6 +238,7 @@ static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int
   p.C0 = mref(Lbuf, np, stride);
   p.alpha = -1.0;
   p.beta = 1.0;
+  set_env(p, env, nt, ENV_CHOL);
   GemmParams pc = p;      // launches on the panel chain
   pc.latency_hint = 1;
   cudaStream_t T = h->stream, P = h->pstream;
@@ -269,9 +278,9 @@ static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int
   return 0;  // T has waited for the last panel (which follows every launch on P): the side stream is joined
 }
 
-int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev) {
+int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env) {
   const int nt = np / TILE;
-  if (chol_uses_lookahead(h, nt, batch)) return chol_lookahead(h, Lbuf, np, stride, n, batch, info_dev);
+  if (chol_uses_lookahead(h, nt, batch)) return chol_lookahead(h, Lbuf, np, stride, n, batch, info_dev, env);
   const int pt = h->chol_panel_override > 0 ? std::min(nt, h->chol_panel_override) : chol_panel_tiles(nt, batch);
   TaskList tl, tr;
   int rc = tasks_chol(h, nt, pt, &tl, &tr);
@@ -283,6 +292,7 @@ int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int b
   p.C0 = mref(Lbuf, np, stride);
   p.alpha = -1.0;
   p.beta = 1.0;
+  set_env(p, env, nt, ENV_CHOL);
   for (int j = 0; j < nt; j++) {
     if (tl.count(j) > 0) {
       p.tasks = tl.at(j);
@@ -332,6 +342,73 @@ int trtri_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long strid
     q.tasks = tw.at(lvl);
     rc = launch_gemm(h, LAYOUT_TN, EPI_AXPBY, q, tw.count(lvl), batch);
     if (rc) return rc;
+  }
+  return 0;
+}
+
+// Selected inverse (Takahashi recurrence) of a factor with a tile envelope: Z = K^-1 on the tiles (I, J) with
+// J <= I <= E_J, which hold every tile where the SE covariance or its derivatives are nonzero.  With Y = L W
+// (W_JJ = L_JJ^-1, the block column scaled by its diagonal inverse) and S = J+1..E_J:
+//   Z[S,J] = -Z[S,S] Y[S,J],    Z[J,J] = W_JJ^T W_JJ - Y[S,J]^T Z[S,J]
+// For K in S, E_K >= E_J, so every Z[S,S] tile the contraction reads was produced by an earlier step.
+//   Y    all block columns in one launch (Sbuf, lower tiles)
+//   D    W_JJ^T W_JJ over the diagonal tiles of Lbuf (full tiles)
+//   per J from the last: Z[S,J] into Lbuf (lower tiles) and its transpose into the upper tiles, so that Z[S,S] is
+//   read with one layout; then Z[J,J].
+// On entry Lbuf holds L (lower tiles) and Sbuf W_JJ on its diagonal tiles; L is consumed.
+static int tasks_sinv(Handle *h, int nt, TaskList *ty, TaskList *td, TaskList *tz, TaskList *tzd) {
+  const long long k1 = tkey(TK_SINV_Y, nt), k2 = tkey(TK_SINV_D, nt), k3 = tkey(TK_SINV_Z, nt), k4 = tkey(TK_SINV_ZD, nt);
+  if (cached(h, k1, ty) && cached(h, k2, td) && cached(h, k3, tz) && cached(h, k4, tzd)) return 0;
+  std::vector<TileTask> y, d, z, zd;
+  std::vector<int> oz(1, 0), ozd(1, 0);
+  for (int j = 0; j < nt; j++) {
+    // NN: Y[i,j] = L[i,j] W[j,j] (W lower: B zero where k < n)
+    for (int i = j + 1; i < nt; i++) y.push_back({i * TILE, j * TILE, j * TILE, j * TILE, i * TILE, j * TILE, TILE, TF_B_TRI_FIRST});
+    // TN: D[j,j] = W[j,j]^T W[j,j]
+    d.push_back({j * TILE, j * TILE, j * TILE, j * TILE, j * TILE, j * TILE, TILE, TF_A_TRI_FIRST | TF_B_TRI_FIRST});
+  }
+  for (int j = 0; j < nt; j++) {  // step j of the lists: block column j
+    const int k = (nt - 1 - j) * TILE;
+    // NN: Z[i,j] = -sum_{k>j} Z[i,k] Y[k,j]
+    for (int i = j + 1; i < nt; i++) z.push_back({i * TILE, (j + 1) * TILE, (j + 1) * TILE, j * TILE, i * TILE, j * TILE, k, 0});
+    oz.push_back((int)z.size());
+    // TN: Z[j,j] = D[j,j] - sum_{k>j} Y[k,j]^T Z[k,j]
+    if (j + 1 < nt) zd.push_back({(j + 1) * TILE, j * TILE, (j + 1) * TILE, j * TILE, j * TILE, j * TILE, k, 0});
+    ozd.push_back((int)zd.size());
+  }
+  std::vector<int> oy = {0, (int)y.size()}, od = {0, (int)d.size()};
+  RC(upload_tasks(h, k1, y, oy, ty));
+  RC(upload_tasks(h, k2, d, od, td));
+  RC(upload_tasks(h, k3, z, oz, tz));
+  return upload_tasks(h, k4, zd, ozd, tzd);
+}
+
+int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, int batch) {
+  const int nt = np / TILE;
+  TaskList ty, td, tz, tzd;
+  RC(tasks_sinv(h, nt, &ty, &td, &tz, &tzd));
+  GemmParams p{};
+  set_env(p, env, nt, ENV_BAND);
+  p.alpha = 1.0;
+  if (nt > 1) {
+    p.A = mref(Lbuf, np, stride); p.B = mref(Sbuf, np, stride); p.C = mref(Sbuf, np, stride); p.tasks = ty.at(0);
+    RC(launch_gemm(h, LAYOUT_NN, EPI_AXPBY, p, ty.count(0), batch));
+  }
+  GemmParams q{};
+  q.A = mref(Sbuf, np, stride); q.B = mref(Sbuf, np, stride); q.C = mref(Lbuf, np, stride); q.alpha = 1.0; q.tasks = td.at(0);
+  RC(launch_gemm(h, LAYOUT_TN, EPI_AXPBY, q, td.count(0), batch));
+  for (int j = nt - 2; j >= 0; j--) {
+    GemmParams pz = p;
+    pz.alpha = -1.0;
+    pz.A = mref(Lbuf, np, stride); pz.B = mref(Sbuf, np, stride); pz.C = mref(Lbuf, np, stride); pz.CT = mref(Lbuf, np, stride);
+    pz.tasks = tz.at(j);
+    RC(launch_gemm(h, LAYOUT_NN, EPI_AXPBY, pz, tz.count(j), batch));
+    GemmParams pd = p;
+    pd.alpha = -1.0;
+    pd.beta = 1.0;
+    pd.A = mref(Sbuf, np, stride); pd.B = mref(Lbuf, np, stride); pd.C = mref(Lbuf, np, stride); pd.C0 = mref(Lbuf, np, stride);
+    pd.tasks = tzd.at(j);
+    RC(launch_gemm(h, LAYOUT_TN, EPI_AXPBY, pd, tzd.count(j), batch));
   }
   return 0;
 }

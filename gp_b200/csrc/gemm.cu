@@ -98,6 +98,14 @@ __global__ void __launch_bounds__(Cfg::NTHREADS, Cfg::MINB) gemm_tile_kernel(con
   extern __shared__ __align__(16) double smem[];
   constexpr int TM = Cfg::TM, LD_MC = Cfg::LD_MC_A;
   TileTask task = p.tasks[blockIdx.x / Cfg::NSPLIT];
+  // the half of the item's envelope this launch uses (F for ENV_CHOL, E for ENV_BAND), read beside the task rather
+  // than after it: on the dependent chain of the look-ahead Cholesky a second dependent load is a visible latency
+  __shared__ int s_env[ENV_MAX_NT];
+  if (p.env_mode != ENV_NONE) {
+    const int *src = p.env + (long long)blockIdx.y * 2 * p.env_nt + (p.env_mode == ENV_CHOL ? 0 : p.env_nt);
+    for (int q = threadIdx.x; q < p.env_nt; q += Cfg::NTHREADS) s_env[q] = src[q];
+    __syncthreads();
+  }
   const int split = (Cfg::NSPLIT > 1) ? (int)(blockIdx.x % Cfg::NSPLIT) : 0;
   const int m0 = (Cfg::NSPLIT_M > 1) ? (split / Cfg::NSPLIT_N) * TM : 0;
   const int n0 = (Cfg::NSPLIT_N > 1) ? (split % Cfg::NSPLIT_N) * TN : 0;
@@ -123,6 +131,30 @@ __global__ void __launch_bounds__(Cfg::NTHREADS, Cfg::MINB) gemm_tile_kernel(con
     if (sym_skip) task.k_len = 0;
   }
   const long long b = blockIdx.y;
+  if (p.env_mode != ENV_NONE) {  // the item's tile envelope: leave out the contraction over exactly-zero operand tiles
+    const int *F = s_env, *E = s_env;
+    const int ti = task.c_r / TILE, tj = task.c_c / TILE;
+    int k0 = A_KC ? task.a_r : task.a_c, k1 = k0 + task.k_len;
+    bool out;
+    if (p.env_mode == ENV_CHOL) {
+      out = tj < F[ti];
+      k0 = max(k0, max(F[ti], F[tj]) * TILE);
+    } else {
+      out = ti > E[tj];
+      k1 = min(k1, (E[tj] + 1) * TILE);
+    }
+    const int shift = k0 - (A_KC ? task.a_r : task.a_c);
+    if (A_KC) task.a_r += shift; else task.a_c += shift;
+    if (B_KC) task.b_r += shift; else task.b_c += shift;
+    task.k_len = max(k1 - k0, 0);
+    // an update of the factor in place with nothing left to add leaves C as it is
+    if (out || (p.env_mode == ENV_CHOL && task.k_len == 0)) {
+      if (EPI != EPI_AXPBY && threadIdx.x < (EPI == EPI_TRACE_DERIV ? 8 : 4))
+        p.partial[((long long)b * gridDim.x + blockIdx.x) * (EPI == EPI_TRACE_DERIV ? 8 : 4) + threadIdx.x] = 0.0;
+      return;
+    }
+  }
+  if (p.flops && threadIdx.x == 0 && task.k_len > 0) atomicAdd(p.flops, 2ull * TM * TN * (unsigned long long)task.k_len);
   const double *__restrict__ A = p.A.p + b * p.A.stride;
   const double *__restrict__ Bm = p.B.p + b * p.B.stride;
   const long long lda = p.A.ld, ldb = p.B.ld;
@@ -254,6 +286,11 @@ __global__ void __launch_bounds__(Cfg::NTHREADS, Cfg::MINB) gemm_tile_kernel(con
           v.y = fma(beta, c0.y, v.y);
         }
         *reinterpret_cast<double2 *>(C + m + (long long)n * p.C.ld) = v;
+        if (p.CT.p) {
+          double *CT = p.CT.p + b * p.CT.stride + n;
+          CT[(long long)m * p.CT.ld] = v.x;
+          CT[(long long)(m + 1) * p.CT.ld] = v.y;
+        }
       }
     }
   } else if (EPI == EPI_TRACE_DERIV) {
@@ -577,8 +614,12 @@ int gemm_partial_layout(Handle *h, const TileTask *tasks, int ntasks, int batch,
   return 0;
 }
 
-int launch_gemm(Handle *h, GemmLayout layout, GemmEpi epi, const GemmParams &p, int ntasks, int batch) {
+int launch_gemm(Handle *h, GemmLayout layout, GemmEpi epi, const GemmParams &p_in, int ntasks, int batch) {
   if (ntasks <= 0 || batch <= 0) return 0;
+  // which tiles an envelope launch skips is only known on the device: there the CTAs count what they execute
+  GemmParams p = p_in;
+  const bool count_here = h->count_flops && p.env_mode == ENV_NONE;
+  if (h->count_flops && p.env_mode != ENV_NONE) p.flops = h->flops_dev;
   const int c = gemm_pick_cfg(h, ntasks, batch);
   if (diag_split_applies(h, ntasks, batch, c)) {
     SplitLists sl;
@@ -591,15 +632,13 @@ int launch_gemm(Handle *h, GemmLayout layout, GemmEpi epi, const GemmParams &p, 
       pd.tasks = sl.diag;
       pd.ntasks = sl.ndiag;
       if (epi != EPI_AXPBY && p.partial) pd.partial = p.partial + (long long)batch * sl.nreg * CfgHalf8::NSPLIT * (epi == EPI_TRACE_DERIV ? 8 : 4);
-      if (h->count_flops) {
-        h->executed_gemm_flops += executed_flops_host(h, p.tasks, ntasks, batch, 2, 3);
-      }
+      if (count_here) h->executed_gemm_flops += executed_flops_host(h, p.tasks, ntasks, batch, 2, 3);
       rc = launch_cfg<CfgHalf8>(h, layout, epi, pr, sl.nreg, batch);
       if (rc) return rc;
       return launch_cfg<CfgQuarter>(h, layout, epi, pd, sl.ndiag, batch);
     }
   }
-  if (h->count_flops) h->executed_gemm_flops += executed_flops_host(h, p.tasks, ntasks, batch, c, c);
+  if (count_here) h->executed_gemm_flops += executed_flops_host(h, p.tasks, ntasks, batch, c, c);
   if (c == 3 && p.latency_hint && h->fine_cfg && epi == EPI_AXPBY && layout != LAYOUT_NN &&
       (long long)ntasks * batch * CfgFine::NSPLIT <= 148) {
     if (layout == LAYOUT_NT) return launch_one<CfgFine, false, false, EPI_AXPBY>(h, p, ntasks, batch);

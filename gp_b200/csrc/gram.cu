@@ -75,10 +75,14 @@ __global__ void __launch_bounds__(256) gram_outer_kernel(int kind, int n, int m,
 __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n, int np, const double *__restrict__ x,
                                                              long long x_stride, const double *__restrict__ theta,
                                                              double jitter, int lower_only,
-                                                             double *__restrict__ K, long long stride) {
+                                                             double *__restrict__ K, long long stride,
+                                                             int *__restrict__ envF) {
   const int nt = np / TILE;
   const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
   if (lower_only && tr < tc) return;
+  // envF (optional, item stride 2 nt, preset to INT_MAX per tile row): the first tile column of each tile row whose exp(-d^2/2rho^2) is
+  // not exactly zero somewhere (NaN counts as nonzero).  That set holds the support of K and of dK/dtheta.
+  bool nz = tr == tc;
   __shared__ double xs[TILE], ys[TILE];
   const long long b = blockIdx.y;
   const double *xb = x + b * x_stride;
@@ -98,9 +102,12 @@ __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n, int np, con
     for (int s = 0; s < 32; s++) {
       const double yc = ys[cq + 4 * s];
       const double d0 = x0 - yc, d1 = x1 - yc;
-      *reinterpret_cast<double2 *>(dst) = make_double2(a2 * exp_nonpos(d0 * d0 * nh), a2 * exp_nonpos(d1 * d1 * nh));
+      const double e0 = exp_nonpos(d0 * d0 * nh), e1 = exp_nonpos(d1 * d1 * nh);
+      nz |= e0 != 0.0 || e1 != 0.0;
+      *reinterpret_cast<double2 *>(dst) = make_double2(a2 * e0, a2 * e1);
       dst += 4LL * np;
     }
+    if (envF && __syncthreads_or(nz) && tid == 0) atomicMin(envF + b * 2 * nt + tr, tc);
     return;
   }
 #pragma unroll 2
@@ -113,13 +120,16 @@ __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n, int np, con
       const int i = r0 + rl + e;
       if (i < n && j < n) {
         const double d = xs[rl + e] - ys[cl];
-        v[e] = (i == j) ? a2 + dadd : a2 * exp_nonpos(d * d * nh);
+        const double ek = exp_nonpos(d * d * nh);
+        nz |= ek != 0.0;
+        v[e] = (i == j) ? a2 + dadd : a2 * ek;
       } else {
         v[e] = (i == j) ? 1.0 : 0.0;
       }
     }
     *reinterpret_cast<double2 *>(Kb + (r0 + rl) + (long long)j * np) = make_double2(v[0], v[1]);
   }
+  if (envF && __syncthreads_or(nz) && tid == 0) atomicMin(envF + b * 2 * nt + tr, tc);
 }
 
 // ---- block-column panel of the padded SE Gram for the block-cyclic multi-GPU Cholesky ----------
@@ -361,11 +371,11 @@ int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const 
 }
 
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch) {
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF) {
   const int nt = np / TILE;
   dim3 grid(nt * nt, batch);
   ProfScope ps__(h, PC_GRAM);
-  gram_se_batched_kernel<<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride);
+  gram_se_batched_kernel<<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

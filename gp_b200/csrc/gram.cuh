@@ -11,7 +11,7 @@ int launch_kernel_eval(Handle *h, int kind, long long len, const double *tj, con
 int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const double *y, double amp2, double l,
                       double *K, long long ldk);
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch);
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF = nullptr);
 int launch_gram_tangent(Handle *h, int n, int np, const double *x, double alpha, const double *ls, double dadd, int mode,
                         double *S, double *Sdot, long long stride, int batch);
 int launch_gram_deriv(Handle *h, int n, int nblocks, const double *t, double alpha, double rho, const double *noise,
@@ -34,7 +34,8 @@ int launch_trmv_lower_n_split(Handle *h, int np, int ks, const double *W, long l
 int launch_trmv_lower_t(Handle *h, int np, const double *W, long long stride, const double *z, long long z_stride,
                         double *a, long long a_stride, int batch);
 int launch_trsv_blocked(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const double *y,
-                        long long y_stride, const double *mu, int n_valid, double *z, long long z_stride, int batch);
+                        long long y_stride, const double *mu, int n_valid, double *z, long long z_stride, int batch,
+                        const int *env = nullptr);
 int launch_trsv_diag(Handle *h, long long ldw, long long w_off, int row0, const double *Wdiag, long long stride,
                      const double *y, long long y_stride, const double *mu, int n_valid, const double *acc, double *z,
                      long long z_stride, int batch);

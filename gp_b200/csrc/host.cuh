@@ -35,7 +35,7 @@ int ws_reserve(Handle *h, size_t bytes, Arena *a);
 
 // ---- tile task lists (host-built once per tile count, cached on the device) ---------------------
 enum TaskKind { TK_CHOL = 1, TK_CHOL_TRAIL, TK_CHOL_LA1, TK_CHOL_LA2, TK_TRTRI_S, TK_TRTRI_W, TK_LAUUM, TK_TAN_T1, TK_TAN_A, TK_TAN_LDOT, TK_COND_V,
-                TK_COND_COV, TK_MUL_WB, TK_MUL_WTB, TK_MUL_LZ };
+                TK_COND_COV, TK_MUL_WB, TK_MUL_WTB, TK_MUL_LZ, TK_SINV_Y, TK_SINV_D, TK_SINV_Z, TK_SINV_ZD };
 
 struct TaskList {
   const TileTask *dev = nullptr;
@@ -59,7 +59,8 @@ inline MatRef mref(double *p, long long ld, long long stride) { return MatRef{p,
 int chol_panel_tiles(int nt, int batch);
 bool chol_uses_lookahead(const Handle *h, int nt, int batch);
 int chol_lookahead_panel(const Handle *h, int nt);
-int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev);
+int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env = nullptr);
+int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, int batch);
 int trtri_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, int batch);
 int extract_diag(Handle *h, int np, const double *L, long long stride, double *dvec, int batch);
 

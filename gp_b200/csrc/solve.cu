@@ -11,6 +11,7 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "fastexp.cuh"
 #include "gram.cuh"
 
 namespace gpb {
@@ -129,13 +130,15 @@ __global__ void __launch_bounds__(256) trmv_lower_t_kernel(int np, const double 
 // Blocked forward substitution L z = (y - mu), one CTA per batch item.  Per 128-row block:
 // s = rhs_j - L[j, 0:j] z[0:j] (two k-halves per row), then z_j = Wdiag_j s with the pre-inverted
 // diagonal tile.  z lives in global memory (written and re-read by this CTA only, ordered by the
-// block barriers), so any n fits.
+// block barriers), so any n fits.  With a tile envelope (env: F, the first nonzero tile column per tile row) the
+// contraction of block j starts at tile F_j: L is exactly zero to its left, and since F_j * 128 is a multiple of the
+// k stride every product still lands in the same partial sum, so z is bit-identical to the dense sweep.
 constexpr int TRSV_KSPLIT = 8;  // k-groups per row: 1024 threads per item keep enough loads in flight to approach HBM speed
 __global__ void __launch_bounds__(TILE * TRSV_KSPLIT) trsv_blocked_kernel(int np, const double *__restrict__ L,
                                                           const double *__restrict__ Wdiag, long long stride,
                                                           const double *__restrict__ y, long long y_stride,
                                                           const double *__restrict__ mu, int n_valid,
-                                                          double *z, long long z_stride) {
+                                                          double *z, long long z_stride, const int *__restrict__ env) {
   constexpr int KS = TRSV_KSPLIT;
   __shared__ double part[KS][TILE];
   __shared__ double sv[TILE];
@@ -148,9 +151,10 @@ __global__ void __launch_bounds__(TILE * TRSV_KSPLIT) trsv_blocked_kernel(int np
   for (int j = 0; j < nt; j++) {
     const int i = j * TILE + r;
     const int kmax = j * TILE;  // multiple of 128, so every group's strided range has the same length
+    const int kmin = env ? env[b * 2 * nt + j] * TILE : 0;
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
-    const double *lp = Lb + i + (long long)grp * np;
-    for (int k = grp; k < kmax; k += 4 * KS) {
+    const double *lp = Lb + i + (long long)(kmin + grp) * np;
+    for (int k = kmin + grp; k < kmax; k += 4 * KS) {
       s0 = fma(lp[0], zb[k], s0);
       s1 = fma(lp[(long long)KS * np], zb[k + KS], s1);
       s2 = fma(lp[2LL * KS * np], zb[k + 2 * KS], s2);
@@ -487,9 +491,10 @@ int launch_trmv_lower_t(Handle *h, int np, const double *W, long long stride, co
 }
 
 int launch_trsv_blocked(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const double *y,
-                        long long y_stride, const double *mu, int n_valid, double *z, long long z_stride, int batch) {
+                        long long y_stride, const double *mu, int n_valid, double *z, long long z_stride, int batch,
+                        const int *env) {
   ProfScope ps__(h, PC_SOLVE);
-  trsv_blocked_kernel<<<batch, TILE * TRSV_KSPLIT, 0, h->stream>>>(np, L, Wdiag, stride, y, y_stride, mu, n_valid, z, z_stride);
+  trsv_blocked_kernel<<<batch, TILE * TRSV_KSPLIT, 0, h->stream>>>(np, L, Wdiag, stride, y, y_stride, mu, n_valid, z, z_stride, env);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }
@@ -526,6 +531,154 @@ int launch_trsv_sweep(Handle *h, int np, const double *L, const double *Wdiag, l
     rc = launch_trsv_update(h, np, doff + TILE, j * TILE, (j + 1) * TILE, nt - 1 - j, L, stride, z, acc, z_stride, batch);
     if (rc) return rc;
   }
+  return 0;
+}
+
+// ---- tile envelope of the SE covariance ------------------------------------------------------------------------------
+// env per item: F[0..nt) (first nonzero tile column of each tile row, filled by gram_se_batched; F_I <= I) and
+// E[0..nt): E_J = the last tile row I with F_I <= J.  F need not be monotone (x unsorted).  For K > J, E_K >= E_J,
+// which is what closes the selected-inverse recurrence over the contiguous range J+1..E_J.
+__global__ void __launch_bounds__(256) envelope_profile_kernel(int nt, int *__restrict__ env) {
+  extern __shared__ int sF[];
+  int *F = env + (long long)blockIdx.x * 2 * nt, *E = F + nt;
+  for (int i = threadIdx.x; i < nt; i += blockDim.x) sF[i] = min(F[i], i);
+  __syncthreads();
+  for (int j = threadIdx.x; j < nt; j += blockDim.x) {
+    int e = j;
+    for (int i = nt - 1; i > j; i--)
+      if (sF[i] <= j) { e = i; break; }
+    F[j] = sF[j];
+    E[j] = e;
+  }
+}
+
+int launch_envelope_profile(Handle *h, int nt, int *env, int batch) {
+  ProfScope ps__(h, PC_OTHER);
+  envelope_profile_kernel<<<batch, 256, nt * sizeof(int), h->stream>>>(nt, env);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+// Trace partials of the gradient from the selected inverse Z = K^-1 (lower tiles and full diagonal tiles, valid on
+// the envelope): one CTA per lower tile (I, J) of one item, the same sums as the EPI_TRACE epilogue of the dense route
+//   [0] w sum (a_i a_j - Z_ij) e_ij,  [1] w sum (a_i a_j - Z_ij) e_ij d_ij^2,  [2] tr Z on diagonal tiles
+// with w = 2 off the diagonal (the tile stands for its transpose too).  Outside the envelope e_ij is exactly zero:
+// those CTAs only write zeros.
+__global__ void __launch_bounds__(256) trace_sinv_kernel(int n, int np, const double *__restrict__ Z, long long stride,
+                                                        const int *__restrict__ env, const double *__restrict__ x,
+                                                        long long x_stride, const double *__restrict__ a,
+                                                        const double *__restrict__ theta, double *__restrict__ partial) {
+  __shared__ double xr[TILE], xc[TILE], ar[TILE], ac[TILE], red[8][3];
+  const int nt = np / TILE, q = blockIdx.x, tid = threadIdx.x;
+  const long long b = blockIdx.y;
+  int I = (int)((sqrt(8.0 * q + 1.0) - 1.0) * 0.5);
+  while (I * (I + 1) / 2 > q) I--;
+  while ((I + 1) * (I + 2) / 2 <= q) I++;
+  const int J = q - I * (I + 1) / 2;
+  double *o = partial + (b * gridDim.x + q) * 4;
+  if (J < env[b * 2 * nt + I]) {
+    if (tid < 4) o[tid] = 0.0;
+    return;
+  }
+  const double *xb = x + b * x_stride, *ab = a + b * np;
+  if (tid < TILE) {
+    const int i = I * TILE + tid;
+    xr[tid] = i < n ? xb[i] : 0.0;
+    ar[tid] = i < n ? ab[i] : 0.0;
+  } else {
+    const int j = J * TILE + tid - TILE;
+    xc[tid - TILE] = j < n ? xb[j] : 0.0;
+    ac[tid - TILE] = j < n ? ab[j] : 0.0;
+  }
+  __syncthreads();
+  const double rho = theta[b * 3 + 1], nh = -0.5 / (rho * rho);
+  const int r = tid & 127, cq = tid >> 7, i = I * TILE + r;
+  const double *Zb = Z + b * stride + i + (long long)J * TILE * np;
+  double s_se = 0.0, s_d2 = 0.0, s_tr = 0.0;
+  if (i < n) {
+    for (int c = cq; c < TILE; c += 2) {
+      const int j = J * TILE + c;
+      if (j >= n) break;
+      const double G = Zb[(long long)c * np];
+      const double d = xr[r] - xc[c], d2 = d * d, ek = exp_nonpos(d2 * nh);
+      const double M = ar[r] * ac[c] - G;
+      s_se += M * ek;
+      s_d2 += M * ek * d2;
+      if (i == j) s_tr += G;
+    }
+  }
+  const double w = I == J ? 1.0 : 2.0;
+  s_se = warp_sum(s_se * w);
+  s_d2 = warp_sum(s_d2 * w);
+  s_tr = warp_sum(s_tr);
+  if ((tid & 31) == 0) { red[tid >> 5][0] = s_se; red[tid >> 5][1] = s_d2; red[tid >> 5][2] = s_tr; }
+  __syncthreads();
+  if (tid < 3) {
+    double s = 0.0;
+    for (int w8 = 0; w8 < 8; w8++) s += red[w8][tid];
+    o[tid] = s;
+  } else if (tid == 3) {
+    o[3] = 0.0;
+  }
+}
+
+int launch_trace_sinv(Handle *h, int n, int np, const double *Z, long long stride, const int *env, const double *x,
+                      long long x_stride, const double *a, const double *theta, double *partial, int batch) {
+  const int nt = np / TILE;
+  dim3 grid(nt * (nt + 1) / 2, batch);
+  ProfScope ps__(h, PC_OTHER);
+  trace_sinv_kernel<<<grid, 256, 0, h->stream>>>(n, np, Z, stride, env, x, x_stride, a, theta, partial);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+// Band-limited blocked back substitution a = L^-T z, one CTA of 32 warps per item, block rows from the last:
+//   s = z_J - sum_{I=J+1..E_J} L[I,J]^T a_I,   a_J = Wdiag_J^T s
+// Rows below E_J are exactly zero in block column J.  A warp owns four columns; its lanes run down a column
+// (16-byte loads), so every read of L is coalesced.
+__global__ void __launch_bounds__(1024) backsub_band_kernel(int np, const double *__restrict__ L, const double *__restrict__ Wdiag,
+                                                           long long stride, const int *__restrict__ env,
+                                                           const double *__restrict__ z, double *a) {
+  __shared__ double sv[TILE];
+  const long long b = blockIdx.x;
+  const int nt = np / TILE, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const double *Lb = L + b * stride, *Wb = Wdiag + b * stride, *zb = z + b * np;
+  const int *E = env + b * 2 * nt + nt;
+  double *ab = a + b * np;
+  for (int J = nt - 1; J >= 0; J--) {
+    const int i0 = (J + 1) * TILE, i1 = (E[J] + 1) * TILE;
+    for (int c = warp; c < TILE; c += 32) {
+      const int col = J * TILE + c;
+      const double *lc = Lb + (long long)col * np;
+      double s0 = 0.0, s1 = 0.0;
+      for (int i = i0 + 2 * lane; i < i1; i += 64) {
+        const double2 l2 = *reinterpret_cast<const double2 *>(lc + i);
+        const double2 a2 = *reinterpret_cast<const double2 *>(ab + i);
+        s0 = fma(l2.x, a2.x, s0);
+        s1 = fma(l2.y, a2.y, s1);
+      }
+      const double s = warp_sum(s0 + s1);
+      if (lane == 0) sv[c] = zb[col] - s;
+    }
+    __syncthreads();
+    for (int c = warp; c < TILE; c += 32) {
+      const double *wc = Wb + (long long)J * TILE * (np + 1) + (long long)c * np;  // column c of the diagonal tile inverse
+      const double2 w2 = *reinterpret_cast<const double2 *>(wc + 2 * lane);
+      const double2 w3 = *reinterpret_cast<const double2 *>(wc + 64 + 2 * lane);
+      double s = fma(w2.x, sv[2 * lane], w2.y * sv[2 * lane + 1]);
+      s = fma(w3.x, sv[64 + 2 * lane], fma(w3.y, sv[65 + 2 * lane], s));
+      s = warp_sum(s);
+      if (lane == 0) ab[J * TILE + c] = s;
+    }
+    __syncthreads();
+  }
+}
+
+int launch_backsub_band(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const int *env,
+                        const double *z, double *a, int batch) {
+  ProfScope ps__(h, PC_SOLVE);
+  backsub_band_kernel<<<batch, 1024, 0, h->stream>>>(np, L, Wdiag, stride, env, z, a);
+  GPB_LAUNCH_CHECK(h);
   return 0;
 }
 

@@ -71,8 +71,9 @@ GPB200_API int gpb200_set_gemm_config(gpb200_handle_t h, int cfg);
 GPB200_API int gpb200_set_profiling(gpb200_handle_t h, int on);
 GPB200_API int gpb200_get_profile(gpb200_handle_t h, double *ms_out6, long long *count_out6);
 
-/* flops the DMMA tile-GEMM launches really executed since counting was switched on (host-side accounting from the task
- * lists: 2 x CTA tile area x contraction length per CTA, after the skipping of triangular / symmetric tile parts);
+/* flops the DMMA tile-GEMM launches really executed since counting was switched on: 2 x CTA tile area x contraction
+ * length per CTA, after the skipping of triangular / symmetric tile parts (host-side, from the task lists) and of the
+ * tiles outside an item's envelope (counted by the CTAs on the device; the getter waits for the handle's stream);
  * bench.py reports it against the algorithmic count */
 GPB200_API int gpb200_set_flop_counting(gpb200_handle_t h, int on);
 GPB200_API double gpb200_executed_gemm_flops(gpb200_handle_t h);
