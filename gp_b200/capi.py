@@ -83,6 +83,9 @@ SIGNATURES = {
     "gpb200_normal_fill": (C.c_int, [_h, C.c_ulonglong, C.c_ulonglong, _ll, C.c_void_p]),
     "gpb200_mvrnorm": (C.c_int, [_h, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_double, C.c_ulonglong,
                                  C.c_void_p, C.c_int]),
+    "gpb200_posterior_draws_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, _ll,
+                                                 C.c_void_p, _ll, C.c_void_p, C.c_double, C.c_void_p, C.c_ulonglong,
+                                                 C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_mg_gram_panel": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                        C.c_void_p, _ll]),
     "gpb200_mg_panel_factor": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p]),
@@ -499,6 +502,46 @@ class Handle:
         self._check(self.lib.gpb200_mvrnorm(self._h, int(ndraws), m, _ptr(mu_a), _ptr(S), max(m, 1), float(jitter),
                                             int(seed), _ptr(out), max(ndraws, 1)), "mvrnorm")
         return out[0].copy() if ndraws == 1 else np.ascontiguousarray(out)
+
+    def posterior_draws_batched(self, t, y, theta, order=1, s=None, jitter=1e-8, seed=None, z=None):
+        """One posterior draw of f^(order) on s (on t when s is None) per hyper-parameter row theta[b] =
+        (alpha, rho, sigma), given y observed on t (include/gpb200.h: gpb200_posterior_draws_batched).
+        t: (n,) or (B, n); s: (m,) or (B, m); y: (n,) or (B, n); z: (B, m) normals, else the device
+        stream of `seed` (0 when None).  Returns draws (B, m), mu (B, m), info (B,)."""
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        if th.ndim != 2 or th.shape[1] != 3:
+            raise ValueError("theta must be (B, 3) = (alpha, rho, sigma) per row")
+        B = th.shape[0]
+        t = np.ascontiguousarray(t, dtype=np.float64); y = np.ascontiguousarray(y, dtype=np.float64)
+        if t.ndim not in (1, 2) or y.ndim not in (1, 2):
+            raise ValueError("t and y must be (n,) or (B, n)")
+        n = t.shape[-1]
+        if y.shape[-1] != n or (t.ndim == 2 and t.shape[0] != B) or (y.ndim == 2 and y.shape[0] != B):
+            raise ValueError("t and y must be (n,) or (B, n) with the same n")
+        s_a = None if s is None else np.ascontiguousarray(s, dtype=np.float64)
+        if s_a is not None and (s_a.ndim not in (1, 2) or (s_a.ndim == 2 and s_a.shape[0] != B)):
+            raise ValueError("s must be (m,) or (B, m)")
+        m = n if s_a is None else s_a.shape[-1]
+        z_a = None
+        if z is not None:
+            z_a = np.ascontiguousarray(z, dtype=np.float64)
+            if z_a.shape != (B, m):
+                raise ValueError("z must be (B, m)")
+        draws = np.empty((B, m)); mu = np.empty((B, m)); info = np.zeros(B, dtype=np.int32)
+        self._check(self.lib.gpb200_posterior_draws_batched(
+            self._h, n, m, int(order), B, _ptr(t), n if t.ndim == 2 else 0, _ptr(s_a),
+            m if s_a is not None and s_a.ndim == 2 else 0, _ptr(y), n if y.ndim == 2 else 0, _ptr(th), float(jitter),
+            _ptr(z_a), int(seed or 0), _ptr(draws), _ptr(mu), _ptr(info)), "posterior_draws_batched")
+        return draws, mu, info
+
+    def posterior_draws_batched_device(self, n, m, order, B, t, t_stride, s, s_stride, y, y_stride, theta, jitter, z, seed,
+                                       draws, mu, info):
+        """Device-pointer variant: every array argument is a torch CUDA tensor (float64 / int32) or None; the
+        handle must be in device-pointer mode.  Asynchronous on the handle's stream."""
+        assert self.device_pointers
+        self._check(self.lib.gpb200_posterior_draws_batched(self._h, n, m, order, B, _ptr(t), t_stride, _ptr(s), s_stride,
+                                                            _ptr(y), y_stride, _ptr(theta), jitter, _ptr(z), int(seed),
+                                                            _ptr(draws), _ptr(mu), _ptr(info)), "posterior_draws_batched")
 
 
 _default = {}

@@ -82,3 +82,89 @@ extern "C" int gpb200_mvrnorm(gpb200_handle_t h, int ndraws, int m, const double
   RC(finish(h));
   return 0;
 }
+
+// Posterior draws for B hyper-parameter draws, one joint factorisation per item.  The Cholesky factor of
+//   J = [[K, Ks^T], [Ks, Kss + jitter I]]  is  [[L11, 0], [L21, L22]]  with L21 = Ks L11^-T and L22 L22^T = cov,
+// so with z1 = L11^-1 y the lower block of  L [z1; eps]  is  L21 z1 + L22 eps = mu + chol(cov) eps.
+// The pivot index of the joint factorisation already is the item's info (1..n: K, n+1..n+m: cov).
+extern "C" int gpb200_posterior_draws_batched(gpb200_handle_t h, int n, int m, int order, int B, const double *t,
+                                              long long t_stride, const double *s, long long s_stride, const double *y,
+                                              long long y_stride, const double *theta, double jitter, const double *z,
+                                              unsigned long long seed, double *draws, double *mu, int *info) {
+  CHECK_H(h);
+  if (n < 1) BAD_ARG(h, 2, "posterior_draws_batched: n must be >= 1");
+  if (m < 1) BAD_ARG(h, 3, "posterior_draws_batched: m must be >= 1");
+  if (order < 0 || order > 2) BAD_ARG(h, 4, "posterior_draws_batched: derivative order must be 0, 1 or 2");
+  if (B < 0) BAD_ARG(h, 5, "posterior_draws_batched: negative batch");
+  if ((long long)n + m > MAX_DENSE_N) BAD_ARG(h, 3, "posterior_draws_batched: n + m above 65407 is not supported");
+  if (t_stride != 0 && t_stride < n) BAD_ARG(h, 7, "posterior_draws_batched: t_stride < n");
+  if (!s && m != n) BAD_ARG(h, 8, "posterior_draws_batched: s == NULL predicts on t and needs m == n");
+  if (s && s_stride != 0 && s_stride < m) BAD_ARG(h, 9, "posterior_draws_batched: s_stride < m");
+  if (y_stride != 0 && y_stride < n) BAD_ARG(h, 11, "posterior_draws_batched: y_stride < n");
+  if (B == 0) return 0;
+  if (!t || !y || !theta || !draws || !info) BAD_ARG(h, 6, "posterior_draws_batched: t, y, theta, draws and info are required");
+  if (!s) { s = t; s_stride = t_stride; }
+
+  const int N = n + m, np = round_up(N, TILE), nt = np / TILE;
+  const long long mat = (long long)np * np;
+  const long long tl = t_stride ? n : 0, sl = s_stride ? m : 0, yl = y_stride ? n : 0;
+  const size_t per_item = 2 * (size_t)mat * 8 + 2 * (size_t)np * 8;
+  const size_t fixed = pad256((size_t)(B * tl + n) * 8) + pad256((size_t)(B * sl + m) * 8) + pad256((size_t)(B * yl + n) * 8) +
+                       pad256((size_t)B * 3 * 8) + (z ? pad256((size_t)B * m * 8) : 0) + (mu ? 2 : 1) * pad256((size_t)B * m * 8) +
+                       pad256((size_t)B * 4) + 6 * 256 + 4096;
+  // chunk the batch under the workspace limit, sized like the fused LML path
+  int Bc = B;
+  if (h->ws_limit > 0 || fixed + per_item * (size_t)B + 8192 > h->ws_bytes) {
+    size_t limit = (size_t)h->ws_limit;
+    if (h->ws_limit <= 0) {
+      size_t freeb = 0, totalb = 0;
+      GPB_CUDA(h, cudaMemGetInfo(&freeb, &totalb));
+      limit = (size_t)((freeb + h->ws_bytes) * 0.85);
+    }
+    if (limit < fixed + per_item + 8192) BAD_ARG(h, 1002, "posterior_draws_batched: workspace limit too small for one item");
+    Bc = (int)std::min<size_t>((size_t)B, (limit - fixed - 8192) / per_item);
+  }
+  Bc = std::min(Bc, 65535);  // gridDim.y of the batched launches
+  Arena a;
+  RC(ws_reserve(h, fixed + per_item * (size_t)Bc + 8192, &a));
+  double *dt = a.take<double>((size_t)B * tl + n), *ds = a.take<double>((size_t)B * sl + m), *dy = a.take<double>((size_t)B * yl + n);
+  double *dth = a.take<double>((size_t)B * 3), *dz = z ? a.take<double>((size_t)B * m) : nullptr;
+  double *ddraw = a.take<double>((size_t)B * m), *dmu = mu ? a.take<double>((size_t)B * m) : nullptr;
+  int *dinfo = a.take<int>(B);
+  double *Lbuf = a.take<double>((size_t)Bc * mat), *Sbuf = a.take<double>((size_t)Bc * mat);
+  double *zbuf = a.take<double>((size_t)Bc * np), *vbuf = a.take<double>((size_t)Bc * np);
+  if (!vbuf) BAD_ARG(h, 1002, "posterior_draws_batched: workspace arithmetic error");
+
+  if (t_stride) RC(to_device_2d(h, t, t_stride, dt, n, n, B)); else RC(to_device(h, t, dt, n));
+  if (s_stride) RC(to_device_2d(h, s, s_stride, ds, m, m, B)); else RC(to_device(h, s, ds, m));
+  if (y_stride) RC(to_device_2d(h, y, y_stride, dy, n, n, B)); else RC(to_device(h, y, dy, n));
+  RC(to_device(h, theta, dth, (size_t)B * 3));
+  if (z) RC(to_device(h, z, dz, (size_t)B * m));
+  GPB_CUDA(h, cudaMemsetAsync(dinfo, 0, (size_t)B * sizeof(int), h->stream));
+  for (int b0 = 0; b0 < B; b0 += Bc) {
+    const int bc = std::min(Bc, B - b0);
+    const double *cy = dy + (long long)b0 * yl;
+    int *cinfo = dinfo + b0;
+    RC(launch_gram_cond_batched(h, n, m, order, np, dt + (long long)b0 * tl, tl, ds + (long long)b0 * sl, sl, dth + (long long)b0 * 3,
+                                jitter, Lbuf, mat, bc));
+    RC(chol_batched(h, Lbuf, np, mat, N, bc, cinfo));
+    // z[0, n) = L11^-1 y (the rhs is read as zero from row n on)
+    RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
+    if (bc >= 32) RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, yl, nullptr, n, zbuf, np, bc));
+    else RC(launch_trsv_sweep(h, np, Lbuf, Sbuf, mat, cy, yl, nullptr, n, zbuf, vbuf, np, bc));
+    if (dmu) {  // rows [n, n+m) of L [z1; 0] = L21 z1 = mu
+      RC(launch_trmv_lower_n(h, np, Lbuf, mat, zbuf, np, n, vbuf, np, bc));
+      RC(launch_rows_or_nan(h, n, m, vbuf, np, cinfo, dmu + (long long)b0 * m, bc));
+    }
+    // z[n, n+m) = eps_b: the caller's normals, or normals [b*m, (b+1)*m) of the stream (independent of the chunking)
+    if (dz) GPB_CUDA(h, cudaMemcpy2DAsync(zbuf + n, (size_t)np * 8, dz + (long long)b0 * m, (size_t)m * 8, (size_t)m * 8, bc,
+                                          cudaMemcpyDeviceToDevice, h->stream));
+    else RC(launch_normal_fill(h, seed, (unsigned long long)b0 * m, (long long)bc * m, m, np, zbuf + n));
+    RC(launch_trmv_lower_n(h, np, Lbuf, mat, zbuf, np, N, vbuf, np, bc));
+    RC(launch_rows_or_nan(h, n, m, vbuf, np, cinfo, ddraw + (long long)b0 * m, bc));
+  }
+  RC(from_device(h, ddraw, draws, (size_t)B * m * sizeof(double)));
+  if (mu) RC(from_device(h, dmu, mu, (size_t)B * m * sizeof(double)));
+  RC(from_device(h, dinfo, info, (size_t)B * sizeof(int)));
+  return finish(h);
+}

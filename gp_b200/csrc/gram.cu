@@ -288,6 +288,58 @@ __global__ void __launch_bounds__(256) gram_deriv_batched_kernel(int n, int orde
   }
 }
 
+// Joint prior covariance of the noisy values f(t) + noise and the derivative f^(p)(s) of a GP, for
+// conditioning and drawing in one factorisation (gpb200_posterior_draws_batched):
+//   J = [[alpha^2 QQ(t, t) + sigma^2 I,  .                          ],
+//        [alpha^2 k_{p,0}(s, t),        alpha^2 k_{p,p}(s, s) + jitter I]]
+// rows [0, n) from t, rows [n, n+m) from s; padded np x np per item with identity in the padding, lower tiles only.
+// Lower-triangle elements come from kern_value / c_joint_kind exactly as gram_outer evaluates them (row point first);
+// the strict upper part of a diagonal tile mirrors them.  theta = (alpha, rho, sigma) per item.
+__global__ void __launch_bounds__(256) gram_cond_batched_kernel(int n, int m, int order, int np,
+                                                               const double *__restrict__ t, long long t_stride,
+                                                               const double *__restrict__ s, long long s_stride,
+                                                               const double *__restrict__ theta, double jitter,
+                                                               double *__restrict__ K, long long stride) {
+  const int nt = np / TILE;
+  const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
+  if (tr < tc) return;
+  __shared__ double xs[TILE], ys[TILE];
+  const long long b = blockIdx.y;
+  const double *tb = t + b * t_stride, *sb = s + b * s_stride;
+  const int N = n + m;
+  const int r0 = tr * TILE, c0 = tc * TILE, tid = threadIdx.x;
+  {
+    const int I = (tid < TILE) ? r0 + tid : c0 + tid - TILE;
+    const double v = (I < n) ? tb[I] : (I < N) ? sb[I - n] : 0.0;
+    if (tid < TILE) xs[tid] = v;
+    else ys[tid - TILE] = v;
+  }
+  __syncthreads();
+  const double alpha = theta[b * 3 + 0], rho = theta[b * 3 + 1], sigma = theta[b * 3 + 2];
+  const double amp2 = alpha * alpha;
+  double *Kb = K + b * stride;
+  const int rl = 2 * (tid & 63), cq = tid >> 6;
+  for (int q = 0; q < 32; q++) {
+    const int cl = cq + 4 * q;
+    const int J = c0 + cl;
+    double v[2];
+#pragma unroll
+    for (int e = 0; e < 2; e++) {
+      const int I = r0 + rl + e;
+      if (I < N && J < N) {
+        const bool up = I < J;  // only inside a diagonal tile
+        const int Ir = up ? J : I, Jc = up ? I : J;
+        const double xr = up ? ys[cl] : xs[rl + e], xc = up ? xs[rl + e] : ys[cl];
+        v[e] = kern_value(c_joint_kind[Ir < n ? 0 : order][Jc < n ? 0 : order], xr, xc, rho, amp2);
+        if (I == J) v[e] += (I < n) ? sigma * sigma : jitter;
+      } else {
+        v[e] = (I == J) ? 1.0 : 0.0;
+      }
+    }
+    *reinterpret_cast<double2 *>(Kb + (r0 + rl) + (long long)J * np) = make_double2(v[0], v[1]);
+  }
+}
+
 // ---- QQard (R/kernels.R:19) ---------------------------------------------------------------------
 __global__ void __launch_bounds__(256) gram_ard_kernel(int n, int m, int D, const double *__restrict__ X, long long ldx,
                                                       const double *__restrict__ Y, long long ldy, double alpha,
@@ -417,6 +469,17 @@ int launch_gram_deriv_batched(Handle *h, int n, int order0, int nblocks, int np,
   ProfScope ps__(h, PC_GRAM);
   gram_deriv_batched_kernel<<<grid, 256, 0, h->stream>>>(n, order0, nblocks, np, t, t_stride, theta, theta_stride, jitter,
                                                         lower_only, K, stride);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+int launch_gram_cond_batched(Handle *h, int n, int m, int order, int np, const double *t, long long t_stride,
+                             const double *s, long long s_stride, const double *theta, double jitter, double *K,
+                             long long stride, int batch) {
+  const int nt = np / TILE;
+  dim3 grid(nt * nt, batch);
+  ProfScope ps__(h, PC_GRAM);
+  gram_cond_batched_kernel<<<grid, 256, 0, h->stream>>>(n, m, order, np, t, t_stride, s, s_stride, theta, jitter, K, stride);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

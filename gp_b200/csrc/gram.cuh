@@ -19,6 +19,9 @@ int launch_gram_deriv(Handle *h, int n, int nblocks, const double *t, double alp
 int launch_gram_deriv_batched(Handle *h, int n, int order0, int nblocks, int np, const double *t, long long t_stride,
                               const double *theta, int theta_stride, double jitter, int lower_only, double *K,
                               long long stride, int batch);
+int launch_gram_cond_batched(Handle *h, int n, int m, int order, int np, const double *t, long long t_stride,
+                             const double *s, long long s_stride, const double *theta, double jitter, double *K,
+                             long long stride, int batch);
 int launch_gram_ard(Handle *h, int n, int m, int D, const double *X, long long ldx, const double *Y, long long ldy,
                     double alpha, const double *rho, int rho_len, double *K, long long ldk);
 
@@ -76,5 +79,7 @@ int launch_normal_fill(Handle *h, unsigned long long seed, unsigned long long of
                        long long ld, double *out);
 int launch_add_mean_transpose(Handle *h, int m, int ndraws, const double *X, long long ldx, const double *mu,
                               double *out, long long ldo);
+int launch_rows_or_nan(Handle *h, int row0, int rows, const double *src, long long src_stride, const int *info,
+                       double *dst, int batch);
 
 }  // namespace gpb

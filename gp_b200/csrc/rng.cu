@@ -30,22 +30,24 @@ __device__ __forceinline__ double u53(unsigned a, unsigned b) {
   return ((double)m + 0.5) * (1.0 / 9007199254740992.0);
 }
 
-// out[e] for e in [0, len): normal number e of stream `seed` (+ `offset` elements).  Counter q = e / 2
-// yields the Box-Muller pair (e even: cos branch, e odd: sin branch).  ld / rows lay the stream out as
-// a column-major matrix with padding rows left untouched (rows == ld for a flat vector).
+// out[e] for e in [0, len): normal number offset + e of stream `seed`.  Counter q = (offset + e) / 2
+// yields the Box-Muller pair (offset + e even: cos branch, odd: sin branch).  ld / rows lay the stream out as
+// a column-major matrix with padding rows left untouched (rows == ld for a flat vector).  An odd offset
+// (a chunk of draws of odd length starting mid-pair) regenerates the pair it starts in and keeps its sin half.
 __global__ void normal_fill_kernel(unsigned long long seed, unsigned long long offset, long long len, long long rows,
                                    long long ld, double *__restrict__ out) {
-  const long long npairs = (len + 1) / 2;
+  const long long first = (long long)(offset & 1ULL);
+  const long long npairs = (len + first + 1) / 2;
   for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < npairs; q += (long long)gridDim.x * blockDim.x) {
-    const unsigned long long ctr = (offset >> 1) + (unsigned long long)q;   // offset is even (checked by the host)
+    const unsigned long long ctr = (offset >> 1) + (unsigned long long)q;
     unsigned r[4];
     philox4x32_10((unsigned)ctr, (unsigned)(ctr >> 32), 0u, 0u, (unsigned)seed, (unsigned)(seed >> 32), r);
     const double u1 = u53(r[0], r[1]), u2 = u53(r[2], r[3]);
     const double rad = sqrt(-2.0 * log(u1));
     double s, c;
     sincospi(2.0 * u2, &s, &c);
-    const long long e0 = 2 * q, e1 = 2 * q + 1;
-    out[(e0 / rows) * ld + (e0 % rows)] = rad * c;
+    const long long e0 = 2 * q - first, e1 = e0 + 1;
+    if (e0 >= 0) out[(e0 / rows) * ld + (e0 % rows)] = rad * c;
     if (e1 < len) out[(e1 / rows) * ld + (e1 % rows)] = rad * s;
   }
 }
@@ -53,7 +55,7 @@ __global__ void normal_fill_kernel(unsigned long long seed, unsigned long long o
 int launch_normal_fill(Handle *h, unsigned long long seed, unsigned long long offset, long long len, long long rows,
                        long long ld, double *out) {
   if (len <= 0) return 0;
-  const long long npairs = (len + 1) / 2;
+  const long long npairs = (len + (long long)(offset & 1ULL) + 1) / 2;
   const int blocks = (int)std::min<long long>((npairs + 255) / 256, 148 * 8);
   ProfScope ps__(h, PC_OTHER);
   normal_fill_kernel<<<blocks, 256, 0, h->stream>>>(seed, offset, len, rows, ld, out);
@@ -83,6 +85,24 @@ int launch_add_mean_transpose(Handle *h, int m, int ndraws, const double *X, lon
   dim3 grid((m + 31) / 32, (ndraws + 31) / 32), block(32, 8);
   ProfScope ps__(h, PC_OTHER);
   add_mean_transpose_kernel<<<grid, block, 0, h->stream>>>(m, ndraws, X, ldx, mu, out, ldo);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+// dst[b*rows + i] = src[b*src_stride + row0 + i], or NaN for every i when info[b] != 0 (a failed item)
+__global__ void rows_or_nan_kernel(int row0, int rows, const double *__restrict__ src, long long src_stride,
+                                   const int *__restrict__ info, double *__restrict__ dst) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const long long b = blockIdx.y;
+  if (i >= rows) return;
+  dst[b * rows + i] = info[b] ? __longlong_as_double(0x7ff8000000000000LL) : src[b * src_stride + row0 + i];
+}
+
+int launch_rows_or_nan(Handle *h, int row0, int rows, const double *src, long long src_stride, const int *info,
+                       double *dst, int batch) {
+  dim3 grid((rows + 255) / 256, batch);
+  ProfScope ps__(h, PC_OTHER);
+  rows_or_nan_kernel<<<grid, 256, 0, h->stream>>>(row0, rows, src, src_stride, info, dst);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

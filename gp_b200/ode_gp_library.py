@@ -84,6 +84,30 @@ def sample_derivs(params, ynoise, ti, rng=None, seed=None, handle=None):
     return mu + h.trmv_lower(L, rng.standard_normal(mu.shape[0]))
 
 
+def sample_derivs_draws(params, ynoise, ti, seed=None, rng=None, handle=None):
+    """The loop of pendulum_fit.R:259-268 over sample_derivs, batched: one draw of the posterior derivative per
+    row of params = (l, a, sy) (B, 3), in one call (gpb200_posterior_draws_batched, order 1, predicting on ti,
+    jitter 1e-8).  ynoise: (n,) shared or (B, n).  Normals: the device stream of `seed`, or drawn on the host from
+    `rng` (a NumPy Generator; a fresh one when both are None).  Returns a (B, n) array."""
+    p = np.asarray(params, dtype=np.float64)
+    if p.ndim != 2 or p.shape[1] != 3:
+        raise ValueError("sample_derivs_draws: params must be (B, 3) = (l, a, sy) per row")
+    ti = np.asarray(ti, dtype=np.float64)
+    y = np.asarray(ynoise, dtype=np.float64)
+    if ti.ndim != 1 or y.ndim not in (1, 2) or y.shape[-1] != ti.shape[0] or (y.ndim == 2 and y.shape[0] != p.shape[0]):
+        raise ValueError("sample_derivs_draws: ynoise must be (n,) or (B, n) with n = len(ti)")
+    h = handle or capi.default_handle()
+    theta = p[:, [1, 0, 2]]  # (l, a, sy) -> (alpha, rho, sigma)
+    z = None
+    if seed is None:
+        z = (rng or np.random.default_rng()).standard_normal((p.shape[0], ti.shape[0]))
+    draws, _, info = h.posterior_draws_batched(ti, y, theta, order=1, jitter=1e-8, seed=seed, z=z)
+    bad = np.flatnonzero(info)
+    if bad.size:
+        raise capi.NotPositiveDefiniteError("sample_derivs_draws (item %d)" % bad[0], int(info[bad[0]]))
+    return draws
+
+
 def create_p_dotXnS(Xn_list, mn, Kn, theta, rng=None, handle=None, incremental=True):
     """R/ode_gp_library.R:43-93: closure that, given a new state x*, returns the conditional normal
     of the derivative there given the data and every derivative already drawn, then draws from it.

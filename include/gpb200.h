@@ -243,6 +243,25 @@ GPB200_API int gpb200_normal_fill(gpb200_handle_t h, unsigned long long seed, un
  * NULL (zeros).  (MASS uses an eigen-decomposition square root; both give N(mu, Sigma) draws.) */
 GPB200_API int gpb200_mvrnorm(gpb200_handle_t h, int ndraws, int m, const double *mu, const double *Sigma, int lds,
                               double jitter, unsigned long long seed, double *out, int ldo);
+/* B posterior draws, one per hyper-parameter draw theta_b = (alpha, rho, sigma), in one call that stays on the
+ * device: the loop of pendulum_fit.R:259-268 over sample_derivs (:227-255: three Grams, conditioning, one
+ * mvrnorm draw) and of lorenz.Rmd:58-68,80-107 (separate prediction grid, 1e-6 jitter).  For item b
+ *   K   = alpha^2 QQ(t, t) + sigma^2 I          n x n   (training grid t, observations y)
+ *   Ks  = alpha^2 k_{p,0}(s, t)                  m x n   (covariance of f^(p)(s_i) with f(t_j))
+ *   Kss = alpha^2 k_{p,p}(s, s)                  m x m
+ *   mu  = Ks K^-1 y,   cov = Kss - Ks K^-1 Ks^T + jitter I,   draw_b = mu + chol(cov) eps_b
+ * with k_{p,q} the kernels of derivative_kernels.R:39-73 and derivative order p = `order` in {0, 1, 2}:
+ * (QQ, QQ) as in ch2.py:36-45, (RQ, RR) as in pendulum_fit.R:238-240, (TQ, TT) as in gp_derivs.py on tts.
+ * s == NULL predicts on t (then m == n).  t, s, y: B strides in doubles (0 = shared; s == NULL takes t's);
+ * theta: B x 3 row-major.  eps_b = z + b*m when z != NULL, else the standard normals [b*m, (b+1)*m) of
+ * gpb200_normal_fill(seed) (B = 1: the normals of gpb200_mvrnorm(1, ..., seed)).  Outputs: draws[B*m] (column b
+ * = draw b), mu[B*m] (may be NULL), info[B]: 0 ok; k in 1..n: K is not positive definite at pivot k; n + k: cov is
+ * not positive definite at pivot k.  Items with info != 0 get NaN in draws and mu; the others are unaffected.
+ * Computed from one Cholesky factorisation of the joint (n+m)^2 prior covariance of (y, f^(p)(s)) per item. */
+GPB200_API int gpb200_posterior_draws_batched(gpb200_handle_t h, int n, int m, int order, int B, const double *t,
+                                              long long t_stride, const double *s, long long s_stride, const double *y,
+                                              long long y_stride, const double *theta, double jitter, const double *z,
+                                              unsigned long long seed, double *draws, double *mu, int *info);
 
 /* ---- (e) multi-GPU block-cyclic Cholesky of ONE large matrix: per-rank building blocks ------------
  * DEVICE pointers only.  A panel is a block column of the padded matrix (np = ceil(n/128)*128)

@@ -52,6 +52,13 @@ sample_derivs <- function(params, ynoise, ti, seed = NULL) {
   L <- gp_chol(m$cov)
   as.numeric(m$mu + L %*% rnorm(length(m$mu)))
 }
+# the mclapply loop of pendulum_fit.R:259-268 in one GPU call: params is 3 x B, one (l, a, sy) per COLUMN; ynoise a
+# vector or a length(ti) x B matrix; returns a length(ti) x B matrix, column b = sample_derivs(params[, b], ...)
+sample_derivs_draws <- function(params, ynoise, ti, seed = NULL) {
+  params <- as.matrix(params)
+  z <- if (is.null(seed)) matrix(rnorm(length(ti) * ncol(params)), length(ti), ncol(params)) else NULL
+  .Call("gp_sample_derivs_draws", params, ynoise, ti, seed, z)
+}
 mvrnorm <- function(n = 1, mu, Sigma, seed = sample.int(.Machine$integer.max, 1)) {   # MASS::mvrnorm signature + seed
   out <- .Call("gp_mvrnorm", as.integer(n), mu, Sigma, seed)
   if (n == 1) drop(out) else out

@@ -355,6 +355,45 @@ SEXP gp_mvrnorm(SEXP n_, SEXP mu_, SEXP Sigma_, SEXP seed) {
   return out;
 }
 
+/* The mclapply body of pendulum_fit.R:259-268 for all draws at once: one sample_derivs (:227-255) draw per COLUMN
+ * (l, a, sy) of the 3 x B matrix params; ynoise is a vector of length(ti) or a length(ti) x B matrix.  Normals: the
+ * device stream of `seed`, or the length(ti) x B matrix z when seed is NULL.  Returns a length(ti) x B matrix. */
+SEXP gp_sample_derivs_draws(SEXP params_, SEXP ynoise_, SEXP ti_, SEXP seed, SEXP z_) {
+  int np = 0;
+  SEXP params = as_real(params_, &np, "params"), y = as_real(ynoise_, &np, "ynoise"), ti = as_real(ti_, &np, "ti");
+  const int n = LENGTH(ti), B = Rf_ncols(params);
+  if (n < 1) Rf_error("sample_derivs_draws: ti must not be empty");
+  if (Rf_nrows(params) != 3)
+    Rf_error("sample_derivs_draws: params must be a 3 x B matrix, one (l, a, sy) per COLUMN (got %d x %d)", Rf_nrows(params), B);
+  const int y_mat = LENGTH(y) != n;
+  if (y_mat) need_matrix(y, n, B, "ynoise");
+  const double *z = NULL;
+  if (Rf_isNull(seed)) {
+    SEXP zr = as_real(z_, &np, "z (normals, needed when seed is NULL)");
+    need_matrix(zr, n, B, "z");
+    z = REAL(zr);
+  }
+  SEXP theta = PROTECT(Rf_allocVector(REALSXP, 3 * (R_xlen_t)B));
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, n, B));
+  SEXP info = PROTECT(Rf_allocVector(INTSXP, B));
+  np += 3;
+  const double *p = REAL(params);
+  double *th = REAL(theta);
+  for (int b = 0; b < B; b++) {  /* (l, a, sy) -> (alpha, rho, sigma) */
+    th[3 * b] = p[3 * b + 1];
+    th[3 * b + 1] = p[3 * b];
+    th[3 * b + 2] = p[3 * b + 2];
+  }
+  check(gpb200_posterior_draws_batched(handle(), n, n, 1, B, REAL(ti), 0, NULL, 0, REAL(y), y_mat ? n : 0, th, 1e-8, z,
+                                       z ? 0ULL : (unsigned long long)Rf_asReal(seed), REAL(out), NULL, INTEGER(info)),
+        "sample_derivs_draws");
+  for (int b = 0; b < B; b++)
+    if (INTEGER(info)[b]) Rf_error("sample_derivs_draws: draw %d: matrix is not positive definite (first non-positive pivot at %d)",
+                                   b + 1, INTEGER(info)[b]);
+  UNPROTECT(np);
+  return out;
+}
+
 /* mu = Ks (K + s2 I)^-1 y ; cov = Kss - Ks (K + s2 I)^-1 Ks^T + jitter I   [pendulum_fit.R:242-251] */
 SEXP gp_condition(SEXP K_, SEXP Ks_, SEXP Kss_, SEXP y_, SEXP noise_var, SEXP jitter) {
   int np = 0;
@@ -412,6 +451,7 @@ static const R_CallMethodDef call_methods[] = {
     {"gp_rbf_cov_chol_grid", (DL_FUNC)&gp_rbf_cov_chol_grid, 2}, {"gp_approx_L_basis", (DL_FUNC)&gp_approx_L_basis, 5},
     {"gp_se_chol_tangent", (DL_FUNC)&gp_se_chol_tangent, 5},
     {"gp_lml_grad_deriv_draws", (DL_FUNC)&gp_lml_grad_deriv_draws, 5}, {"gp_mvrnorm", (DL_FUNC)&gp_mvrnorm, 4},
+    {"gp_sample_derivs_draws", (DL_FUNC)&gp_sample_derivs_draws, 5},
     {NULL, NULL, 0}};
 
 void R_init_gpb200_r(DllInfo *dll) {
