@@ -349,3 +349,96 @@ def test_latent_adjoint_matches_central_differences():
     f = o.cholesky_decompose(o.gram_se(x, 1.0, 1.0, da)) @ z[0]
     r1 = X.latent_adjoint(x, 1.0, 1.0, da, z[0], (y - f) / 0.3 ** 2)
     assert abs(r1["theta_bar"][1] - (g["l"] - 3.0 + 4.0)) <= 1e-10 * r1["scale"][1]
+
+
+# ---- extended-precision reference of the batched posterior draws (oracle/posterior_ext.py) -------------------------
+def _joint_mp(t, s, theta, order, jitter):
+    """J of posterior_ext.joint_cov in 50-digit mpmath, with the kernel formulas of posterior_ext"""
+    import mpmath as mp
+    from oracle import posterior_ext as P
+    mp.mp.dps = 50
+    n, m = len(t), len(s)
+    pts = [mp.mpf(float(v)) for v in t] + [mp.mpf(float(v)) for v in s]
+    alpha, rho, sigma = (mp.mpf(float(v)) for v in theta)
+    J = mp.matrix(n + m, n + m)
+    for i in range(n + m):
+        for j in range(i + 1):
+            name = "QQ" if i < n else P.KINDS[order][0 if j < n else 1]
+            a, b = pts[i], pts[j]
+            if name in P._SWAPPED:
+                name, a, b = P._SWAPPED[name], b, a
+            d = a - b
+            J[i, j] = J[j, i] = alpha ** 2 * P._BASE[name](mp.exp(-(d ** 2 / (2 * rho ** 2))), d, rho)
+        J[i, i] += sigma ** 2 if i < n else mp.mpf(jitter)
+    return J
+
+
+@pytest.mark.parametrize("order", [0, 1, 2])
+def test_posterior_ext_matches_mpmath_llt(order):
+    _need_longdouble()
+    import mpmath as mp
+    from oracle import posterior_ext as P
+    rng = np.random.default_rng(10 + order)
+    for n, m in ((1, 1), (7, 12), (19, 21)):
+        t, s = np.sort(rng.uniform(0, 4, n)), np.sort(rng.uniform(-0.5, 4.5, m))
+        y = np.sin(t) + 0.1 * rng.standard_normal(n)
+        theta = (1.2, 0.8, 0.15)
+        J = _joint_mp(t, s, theta, order, 1e-8)
+        L = mp.cholesky(J)
+        z1 = mp.lu_solve(L[:n, :n], mp.matrix([mp.mpf(float(v)) for v in y]))
+        mu = np.array([float(v) for v in L[n:, :n] * z1])
+        L22 = np.array([[float(L[n + i, n + j]) for j in range(m)] for i in range(m)])
+        ext = P.posterior_ext(t, s, y, theta, order, 1e-8)
+        base = P.posterior_f64(t, s, y, theta, order, 1e-8)
+        assert ext.info == 0 and base.info == 0
+        assert np.all(np.triu(ext.L22, 1) == 0)
+        # with jitter 1e-8 the posterior block is ill-conditioned: the float64 baseline's L22 is off by up to 1e-8
+        # relative here, and the long-double factor must be at least 100 times closer (measured: about 2000 times)
+        for got, want, b in ((ext.mu, mu, base.mu), (ext.L22, L22, base.L22)):
+            assert relerr(got, want) <= 1e-2 * relerr(b, want) + 4e-16, (n, m, relerr(got, want), relerr(b, want))
+        # the long-double J is the 50-digit one to its own rounding
+        Jl = P.joint_cov(t, s, theta, order, 1e-8, np.longdouble)
+        Jm = np.array([[float(J[i, j]) for j in range(n + m)] for i in range(n + m)])
+        dJ = max(abs(mp.mpf(float(Jl[i, j])) + mp.mpf(float(Jl[i, j] - np.longdouble(float(Jl[i, j])))) - J[i, j])
+                 for i in range(n + m) for j in range(n + m))
+        assert float(dJ) <= 1e-18 * np.max(np.abs(Jm)), (n, m, float(dJ))
+        # the float64 J of the restated kernels is the oracle's blocks
+        Jf = P.joint_cov(t, s, theta, order, 1e-8)
+        a2 = theta[0] ** 2
+        assert relerr(Jf[n:, :n], a2 * o.outer_kernel(P.KINDS[order][0], s, t, theta[1])) < 1e-15
+        assert relerr(Jf[n:, n:] - 1e-8 * np.eye(m), a2 * o.outer_kernel(P.KINDS[order][1], s, s, theta[1])) < 1e-15
+
+
+def test_posterior_ext_matches_gp_condition_at_n300_m515():
+    _need_longdouble()
+    from oracle import posterior_ext as P
+    rng = np.random.default_rng(11)
+    t, s = np.sort(rng.uniform(0, 6, 300)), np.sort(rng.uniform(-0.5, 6.5, 515))
+    y = np.sin(t) + 0.1 * rng.standard_normal(300)
+    theta, jitter = (1.3, 0.9, 0.1), 1e-8
+    for order in (0, 1, 2):
+        a2 = theta[0] ** 2
+        mu, cov = o.gp_condition(a2 * o.outer_kernel("QQ", t, t, theta[1]),
+                                 a2 * o.outer_kernel(P.KINDS[order][0], s, t, theta[1]),
+                                 a2 * o.outer_kernel(P.KINDS[order][1], s, s, theta[1]), y, theta[2] ** 2, jitter)
+        ext = P.posterior_ext(t, s, y, theta, order, jitter)
+        assert ext.info == 0
+        assert relerr(ext.mu, mu) < 1e-11, order
+        assert relerr(ext.L22 @ ext.L22.T, cov) < 1e-11, order
+
+
+def test_posterior_ext_reports_the_first_bad_pivot():
+    _need_longdouble()
+    from oracle import posterior_ext as P
+    n, m = 30, 25
+    t, s = np.linspace(0, 3, n), np.linspace(-0.2, 3.2, m)
+    y = np.cos(t)
+    for order in (0, 1, 2):
+        for k in (0, 11, n - 1):
+            tt = t.copy(); tt[k] = np.nan
+            r = P.posterior_ext(tt, s, y, (1.0, 0.7, 0.1), order, 1e-8)
+            assert r.info == k + 1 and np.all(np.isnan(r.mu)) and np.all(np.isnan(r.L22)), (order, k)
+        for k in (0, 9, m - 1):
+            ss = s.copy(); ss[k] = np.nan
+            r = P.posterior_ext(t, ss, y, (1.0, 0.7, 0.1), order, 1e-8, eps=np.ones((2, m)))
+            assert r.info == n + k + 1 and np.all(np.isnan(r.draws)), (order, k)
