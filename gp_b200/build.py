@@ -17,7 +17,7 @@ TAG = os.environ.get("GPB_BUILD_TAG", "")            # experiment builds: libgpb
 SO = os.path.join(LIBDIR, "libgpb200%s.so" % ("_" + TAG if TAG else ""))
 EXTRA = os.environ.get("GPB_EXTRA_NVCC", "").split()
 SOURCES = ["gemm.cu", "panel.cu", "gram.cu", "solve.cu", "engine.cu", "api_core.cu", "api_gp.cu", "api_mg.cu", "rng.cu", "api_sample.cu", "small.cu", "api_latent.cu"]
-HEADERS = ["common.cuh", "gram.cuh", "host.cuh", "fastexp.cuh", "panel_ll.cuh", os.path.join("..", "..", "include", "gpb200.h")]
+HEADERS = ["common.cuh", "gemm_tile_body.cuh", "gram.cuh", "host.cuh", "fastexp.cuh", "panel_ll.cuh", os.path.join("..", "..", "include", "gpb200.h")]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "--expt-relaxed-constexpr"]

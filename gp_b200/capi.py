@@ -64,6 +64,8 @@ SIGNATURES = {
                                           C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_lml_grad_deriv_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, _ll,
                                                 C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gpb200_lml_grad_ard_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, _ll, C.c_void_p,
+                                              C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_rbf_cov_chol": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p]),
     "gpb200_rbf_cov_chol_batched": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p]),
@@ -391,6 +393,35 @@ class Handle:
                                                            _ptr(th), jitter, int(want_grad), _ptr(lml), _ptr(grad),
                                                            _ptr(info)), "lml_grad_deriv_batched")
         return lml, grad, info
+
+    def lml_grad_ard_batched(self, X, y, theta, jitter=0.0, want_grad=True):
+        """ARD squared-exponential covariance (QQard) in D = 1..8 input dimensions.
+        X: (n, D) shared or (B, n, D) per item; y: (n,) or (B, n); theta: (B, D + 2) = (alpha, rho_1 .. rho_D, sigma).
+        Returns lml[B], grad[B, D + 2], info[B]."""
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        X = np.asarray(X, dtype=np.float64); y = np.ascontiguousarray(y, dtype=np.float64)
+        if X.ndim not in (2, 3) or y.ndim not in (1, 2):
+            raise ValueError("X must be (n, D) or (B, n, D) and y (n,) or (B, n)")
+        n, D = X.shape[-2], X.shape[-1]
+        if th.ndim != 2 or th.shape[1] != D + 2:
+            raise ValueError("theta must be (B, D + 2) = (alpha, rho_1 .. rho_D, sigma) per row")
+        B = th.shape[0]
+        if y.shape[-1] != n or (X.ndim == 3 and X.shape[0] != B) or (y.ndim == 2 and y.shape[0] != B):
+            raise ValueError("X and y must hold n points, shared or one set per row of theta")
+        Xc = np.ascontiguousarray(np.swapaxes(X, -1, -2))  # each item column-major n x D
+        lml = np.empty(B); grad = np.empty((B, D + 2)); info = np.zeros(B, dtype=np.int32)
+        self._check(self.lib.gpb200_lml_grad_ard_batched(self._h, n, D, B, _ptr(Xc), n * D if X.ndim == 3 else 0, _ptr(y),
+                                                         n if y.ndim == 2 else 0, _ptr(th), jitter, int(want_grad),
+                                                         _ptr(lml), _ptr(grad), _ptr(info)), "lml_grad_ard_batched")
+        return lml, grad, info
+
+    def lml_grad_ard_batched_device(self, n, D, B, X, x_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info):
+        """Device-pointer variant: every array argument is a torch CUDA tensor (float64 / int32), X holding per item an
+        n x D column-major matrix; the handle must be in device-pointer mode.  Asynchronous on the handle's stream."""
+        assert self.device_pointers
+        self._check(self.lib.gpb200_lml_grad_ard_batched(self._h, n, D, B, _ptr(X), x_stride, _ptr(y), y_stride, _ptr(theta),
+                                                         jitter, int(want_grad), _ptr(lml), _ptr(grad), _ptr(info)),
+                    "lml_grad_ard_batched")
 
     # -- a1-a3 / f-1 ----------------------------------------------------------------------------
     def rbf_cov_chol(self, x1, l):

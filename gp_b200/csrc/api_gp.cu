@@ -10,15 +10,19 @@ using namespace gpb;
 // =================================================================================================
 namespace {
 // which covariance the fused path assembles: the SE kernel of fit_hyperparameters.stan (deriv = false,
-// theta = (alpha, rho, sigma)) or the joint derivative-observation covariance (deriv = true,
-// theta = (alpha, rho, noise[nblocks])) on a grid of n_grid points
-struct LmlSpec { bool deriv; int n_grid, order0, nblocks; };
+// theta = (alpha, rho, sigma)), the joint derivative-observation covariance (deriv = true,
+// theta = (alpha, rho, noise[nblocks])) on a grid of n_grid points, or the ARD kernel on n_grid points in
+// ard_d > 0 dimensions (theta = (alpha, rho[ard_d], sigma); x per item n_grid x ard_d column-major)
+struct LmlSpec { bool deriv; int n_grid, order0, nblocks; int ard_d; };
 
 int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long long x_stride,
              const double *y, long long y_stride, const double *theta, double jitter,
              int want_grad, double *lml, double *grad, int *info) {
-  const int ng = sp.n_grid, n = sp.n_grid * sp.nblocks, ts = sp.deriv ? 2 + sp.nblocks : 3;
-  const int pw = sp.deriv ? 8 : 4;  // doubles per tile partial
+  const bool ard = sp.ard_d > 0;
+  const int ng = sp.n_grid, n = sp.n_grid * sp.nblocks, ts = sp.deriv ? 2 + sp.nblocks : (ard ? 2 + sp.ard_d : 3);
+  const int xl = ard ? ng * sp.ard_d : ng;  // doubles of x per item
+  const GemmEpi epi = sp.deriv ? EPI_TRACE_DERIV : (ard ? EPI_TRACE_ARD : EPI_TRACE);
+  const int pw = epi_partial_width(epi);  // doubles per tile partial
   if (B == 0) return 0;
   const int np = round_up(n, TILE), nt = np / TILE;
   const long long mat = (long long)np * np;
@@ -30,7 +34,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   // chunk the batch so that the resident set fits the workspace limit.  cudaMemGetInfo costs
   // milliseconds with tens of GB allocated, so it is only consulted when the workspace must grow.
   // n <= 128: one CTA per item does the whole evaluation in shared memory (small.cu); no O(n^2) workspace at all
-  const bool small = !sp.deriv && lml_small_applies(h, n);
+  const bool small = !sp.deriv && !ard && lml_small_applies(h, n);
   if (small && h->device_ptrs && info && lml && (grad || !want_grad)) {
     // device-pointer mode: the kernel reads the caller's arrays and writes the caller's results in place --
     // ONE launch per call, no staging copies, no memset (the kernel writes every info word)
@@ -45,11 +49,11 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   //   N = 2048: B = 1 0.948 / 0.949 / 2.34,  B = 8 3.46 / 2.93 / 3.70,  B = 16 6.26 / 5.20 / 4.96,  B = 32 11.0 / 9.59 / 7.67
   //   N = 4096: B = 1 3.36 / 2.98 / 4.59,    B = 4 10.19 / 7.91 / 8.36,  B = 8 19.3 / 14.4 / 8.2,  B = 32 70.9 / 53.4 / 22.0
   // The selected inverse is a chain of 2 nt launches of a few tiles per item: it wins once B * nt >= 256.
-  const bool use_env = !sp.deriv && h->envelope && !small && nt >= 16 && nt <= ENV_MAX_NT;
+  const bool use_env = !sp.deriv && !ard && h->envelope && !small && nt >= 16 && nt <= ENV_MAX_NT;
   const bool sinv = use_env && want_grad && (h->sinv_min_batch > 0 ? B >= h->sinv_min_batch : (long long)B * nt >= 256);
   const size_t per_item = small ? 0 : pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * pw * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) + 64 +
                                       (use_env ? (size_t)2 * nt * sizeof(int) : 0);
-  const size_t fixed = pad256((size_t)B * (x_stride ? ng : 0) * 8 + ng * 8) + pad256((size_t)B * (y_stride ? n : 0) * 8 + n * 8) +
+  const size_t fixed = pad256((size_t)B * (x_stride ? xl : 0) * 8 + (size_t)xl * 8) + pad256((size_t)B * (y_stride ? n : 0) * 8 + n * 8) +
                        2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096 + (use_env ? 256 : 0);
   int Bc = B;
   if (!small && (h->ws_limit > 0 || fixed + per_item * (size_t)B + 8192 > h->ws_bytes)) {
@@ -66,8 +70,8 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   Arena a;
   RC(ws_reserve(h, fixed + per_item * (size_t)Bc + 8192, &a));
 
-  const long long xs = x_stride ? ng : 0, ys = y_stride ? n : 0;
-  double *dx = a.take<double>(x_stride ? (size_t)B * ng : ng);
+  const long long xs = x_stride ? xl : 0, ys = y_stride ? n : 0;
+  double *dx = a.take<double>(x_stride ? (size_t)B * xl : xl);
   double *dy = a.take<double>(y_stride ? (size_t)B * n : n);
   double *dth = a.take<double>((size_t)B * ts);
   double *dlml = a.take<double>(B), *dgrad = a.take<double>((size_t)B * ts);
@@ -92,6 +96,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       const int bc = std::min(Bc, B - b0);
       const double *cx = dx + (long long)b0 * xs, *cy = dy + (long long)b0 * ys, *cth = dth + (long long)b0 * ts;
       if (sp.deriv) RC(launch_gram_deriv_batched(h, ng, sp.order0, sp.nblocks, np, cx, xs, cth, ts, jitter, 1, Lbuf, mat, bc));
+      else if (ard) RC(launch_gram_ard_batched(h, n, sp.ard_d, np, cx, xs, cth, jitter, Lbuf, mat, bc));
       else {
         if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
         RC(launch_gram_se_batched(h, n, np, cx, xs, cth, jitter, 1, Lbuf, mat, bc, env));
@@ -124,14 +129,18 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
         p.n = n;
         p.ntasks = ntasks;
         p.n_grid = ng; p.order0 = sp.order0; p.theta_stride = ts;
-        RC(launch_gemm(h, LAYOUT_TN, sp.deriv ? EPI_TRACE_DERIV : EPI_TRACE, p, ntasks, bc));
+        p.ard_d = sp.ard_d;
+        RC(launch_gemm(h, LAYOUT_TN, epi, p, ntasks, bc));
       } else {
         RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
         if (bc >= 32) RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, np, bc, env));
         else RC(launch_trsv_sweep(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, abuf, np, bc));
       }
       if (!sinv) RC(gemm_partial_layout(h, tl.at(0), ntasks, bc, &n1, &n2));
-      if (sp.deriv)
+      if (ard)
+        RC(launch_finalize_ard(h, n, sp.ard_d, np, want_grad, dvec, zbuf, abuf, partial, n1, n2, cth, dlml + b0,
+                               dgrad + (long long)b0 * ts, bc));
+      else if (sp.deriv)
         RC(launch_finalize_deriv(h, ng, sp.nblocks, np, want_grad, dvec, zbuf, abuf, partial, n1, n2, cth, dlml + b0,
                                  dgrad + (long long)b0 * ts, bc));
       else
@@ -151,7 +160,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   }
   int rc = 0;
   do {
-    if (x_stride) rc = to_device_2d(h, x, x_stride, dx, ng, ng, B); else rc = to_device(h, x, dx, ng);
+    if (x_stride) rc = to_device_2d(h, x, x_stride, dx, xl, xl, B); else rc = to_device(h, x, dx, xl);
     if (rc) break;
     if (y_stride) rc = to_device_2d(h, y, y_stride, dy, n, n, B); else rc = to_device(h, y, dy, n);
     if (rc) break;
@@ -164,7 +173,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       const std::vector<long long> key = {n, B, want_grad, xs, ys, jbits, (long long)(uintptr_t)h->ws, h->chol_panel_override,
                                           sp.deriv, sp.order0, sp.nblocks, h->gemm_cfg_override, h->lookahead, h->lookahead_max_batch,
                                           h->panel_impl, h->trsm_mt_override, h->quarter_below_waves, h->trsm_pipelined, h->panel_fused, h->fine_cfg,
-                                          h->envelope, h->sinv_min_batch};
+                                          h->envelope, h->sinv_min_batch, sp.ard_d};
       auto it = h->graphs.find(key);
       if (it == h->graphs.end()) {
         // task lists allocate and synchronise on first use, which a capture does not allow: a first uncaptured
@@ -226,6 +235,19 @@ extern "C" int gpb200_lml_grad_deriv_batched(gpb200_handle_t h, int n, int order
   if (t_stride != 0 && t_stride < n) BAD_ARG(h, 7, "lml_grad_deriv_batched: t_stride < n");
   if (y_stride != 0 && y_stride < (long long)n * nblocks) BAD_ARG(h, 9, "lml_grad_deriv_batched: y_stride < n * nblocks");
   return lml_core(h, LmlSpec{true, n, order0, nblocks}, B, t, t_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info);
+}
+
+extern "C" int gpb200_lml_grad_ard_batched(gpb200_handle_t h, int n, int D, int B, const double *X, long long x_stride,
+                                           const double *y, long long y_stride, const double *theta, double jitter,
+                                           int want_grad, double *lml, double *grad, int *info) {
+  CHECK_H(h);
+  if (n < 1) BAD_ARG(h, 2, "lml_grad_ard_batched: n must be >= 1");
+  if (D < 1 || D > ARD_MAX_D) BAD_ARG(h, 3, "lml_grad_ard_batched: D must lie in 1..8");
+  if (B < 0) BAD_ARG(h, 4, "lml_grad_ard_batched: negative batch");
+  if ((long long)n * D > 2147483647LL / 2) BAD_ARG(h, 2, "lml_grad_ard_batched: n * D too large");
+  if (x_stride != 0 && x_stride < (long long)n * D) BAD_ARG(h, 6, "lml_grad_ard_batched: x_stride < n * D");
+  if (y_stride != 0 && y_stride < n) BAD_ARG(h, 8, "lml_grad_ard_batched: y_stride < n");
+  return lml_core(h, LmlSpec{false, n, 0, 1, D}, B, X, x_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info);
 }
 
 // number of CUDA-graph replays so far (small evaluations are replayed as one graph)

@@ -68,6 +68,7 @@ struct GemmParams {
   int env_nt, env_mode;
   MatRef CT;                    // EPI_AXPBY: when CT.p is set the transpose of the output tile is written there too
   unsigned long long *flops;    // when set: every CTA adds the flops it executes (after all skipping)
+  int ard_d;                    // EPI_TRACE_ARD: input dimensions D (x is n x D column-major per item, theta_stride = D + 2)
 };
 // envelope modes of the tile GEMM.  Only products with an exactly-zero operand tile are dropped, and the k order of
 // the rest is kept, so a result is bit-identical to the dense launch (up to the sign of an all-zero tile).
@@ -204,7 +205,13 @@ struct ProfScope {
 
 // ---- launchers implemented in the .cu files --------------------------------------------------
 enum GemmLayout { LAYOUT_NT = 0, LAYOUT_TN = 1, LAYOUT_NN = 2, LAYOUT_TT = 3 };  // TT: A k-contiguous, B n-contiguous
-enum GemmEpi { EPI_AXPBY = 0, EPI_TRACE = 1, EPI_TRACE_DERIV = 2 };
+enum GemmEpi { EPI_AXPBY = 0, EPI_TRACE = 1, EPI_TRACE_DERIV = 2, EPI_TRACE_ARD = 3 };
+constexpr int ARD_MAX_D = 8;  // input dimensions of the ARD covariance (gpb200_lml_grad_ard_batched)
+// doubles per CTA partial record of a trace epilogue: (S_se, S_d2, tr G, 0); (S_k, S_dk, tr G per block, ...);
+// (S_e, S_1 .. S_ARD_MAX_D, tr G)
+__host__ __device__ constexpr int epi_partial_width(int epi) {
+  return epi == EPI_TRACE_DERIV ? 8 : (epi == EPI_TRACE_ARD ? ARD_MAX_D + 2 : 4);
+}
 
 int launch_gemm(Handle *h, GemmLayout layout, GemmEpi epi, const GemmParams &p, int ntasks, int batch);
 int gemm_smem_setup(Handle *h);

@@ -359,6 +359,59 @@ __global__ void __launch_bounds__(256) gram_ard_kernel(int n, int m, int D, cons
   }
 }
 
+// ---- batched padded ARD Gram for the fused LML path (gpb200_lml_grad_ard_batched) -----------------
+// K = alpha^2 exp(-0.5 sum_d ((X_id - X_jd) / rho_d)^2) + c I: QQard of R/kernels.R:19 plus the noise diagonal.
+// X per item is n x D column-major (leading dimension n); theta per item (alpha, rho_1 .. rho_D, sigma).  Layout as
+// gram_se_batched_kernel: np x np per item, identity in the padding, lower tiles only.  The coordinates are staged
+// already divided by rho_d, with the same division the ARD trace epilogue (gemm.cu) uses.
+__global__ void __launch_bounds__(256) gram_ard_batched_kernel(int n, int D, int np, const double *__restrict__ X,
+                                                              long long x_stride, const double *__restrict__ theta,
+                                                              double jitter, double *__restrict__ K, long long stride) {
+  const int nt = np / TILE;
+  const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
+  if (tr < tc) return;
+  __shared__ double xs[ARD_MAX_D * TILE], ys[ARD_MAX_D * TILE];
+  const long long b = blockIdx.y;
+  const double *Xb = X + b * x_stride;
+  const double *th = theta + b * (D + 2);
+  const int r0 = tr * TILE, c0 = tc * TILE, tid = threadIdx.x;
+  for (int q = tid; q < D * 2 * TILE; q += 256) {
+    const int d = q / (2 * TILE), l = q % (2 * TILE);
+    const int i = (l < TILE) ? r0 + l : c0 + l - TILE;
+    const double v = (i < n) ? Xb[i + (long long)d * n] / th[1 + d] : 0.0;
+    if (l < TILE) xs[d * TILE + l] = v;
+    else ys[d * TILE + l - TILE] = v;
+  }
+  __syncthreads();
+  const double alpha = th[0], sigma = th[D + 1];
+  const double a2 = alpha * alpha, dadd = sigma * sigma + jitter;
+  double *Kb = K + b * stride;
+  const int rl = 2 * (tid & 63), cq = tid >> 6;
+#pragma unroll 2
+  for (int s = 0; s < 32; s++) {
+    const int cl = cq + 4 * s;
+    const int j = c0 + cl;
+    double v[2];
+#pragma unroll
+    for (int e = 0; e < 2; e++) {
+      const int i = r0 + rl + e;
+      if (i < n && j < n) {
+        double r2 = 0.0;
+        for (int d = 0; d < D; d++) {
+          const double dq = xs[d * TILE + rl + e] - ys[d * TILE + cl];
+          r2 = fma(dq, dq, r2);
+        }
+        // exp_nonpos clamps its argument with fmax, which drops a NaN: a NaN coordinate or length-scale must reach
+        // the factorisation (and fail its item) as it does in the reference
+        v[e] = (i == j) ? a2 + dadd : a2 * (isnan(r2) ? r2 : exp_nonpos(-0.5 * r2));
+      } else {
+        v[e] = (i == j) ? 1.0 : 0.0;
+      }
+    }
+    *reinterpret_cast<double2 *>(Kb + (r0 + rl) + (long long)j * np) = make_double2(v[0], v[1]);
+  }
+}
+
 // ---- f-3: Mercer / Hermite eigen-basis factor of the SE kernel ---------------------------------
 // approx_L(M, scale, x, sigma, l) of models/westbrook.stan:2-30 (copied into six other models;
 // spectral_test.R:6-27 `bH`): N x M matrix whose columns are scaled Hermite functions built by a
@@ -480,6 +533,16 @@ int launch_gram_cond_batched(Handle *h, int n, int m, int order, int np, const d
   dim3 grid(nt * nt, batch);
   ProfScope ps__(h, PC_GRAM);
   gram_cond_batched_kernel<<<grid, 256, 0, h->stream>>>(n, m, order, np, t, t_stride, s, s_stride, theta, jitter, K, stride);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+int launch_gram_ard_batched(Handle *h, int n, int D, int np, const double *X, long long x_stride, const double *theta,
+                            double jitter, double *K, long long stride, int batch) {
+  const int nt = np / TILE;
+  dim3 grid(nt * nt, batch);
+  ProfScope ps__(h, PC_GRAM);
+  gram_ard_batched_kernel<<<grid, 256, 0, h->stream>>>(n, D, np, X, x_stride, theta, jitter, K, stride);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

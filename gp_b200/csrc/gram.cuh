@@ -22,6 +22,8 @@ int launch_gram_deriv_batched(Handle *h, int n, int order0, int nblocks, int np,
 int launch_gram_cond_batched(Handle *h, int n, int m, int order, int np, const double *t, long long t_stride,
                              const double *s, long long s_stride, const double *theta, double jitter, double *K,
                              long long stride, int batch);
+int launch_gram_ard_batched(Handle *h, int n, int D, int np, const double *X, long long x_stride, const double *theta,
+                            double jitter, double *K, long long stride, int batch);
 int launch_gram_ard(Handle *h, int n, int m, int D, const double *X, long long ldx, const double *Y, long long ldy,
                     double alpha, const double *rho, int rho_len, double *K, long long ldk);
 
@@ -51,6 +53,8 @@ int launch_trsv_sweep(Handle *h, int np, const double *L, const double *Wdiag, l
                       int batch);
 int launch_finalize(Handle *h, int n, int np, int want_grad, const double *dvec, const double *z, const double *a,
                     const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch);
+int launch_finalize_ard(Handle *h, int n, int D, int np, int want_grad, const double *dvec, const double *z, const double *a,
+                        const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch);
 int launch_finalize_deriv(Handle *h, int n_grid, int nblocks, int np, int want_grad, const double *dvec, const double *z,
                           const double *a, const double *partial, int ntasks, int ntasks2, const double *theta, double *lml,
                           double *grad, int batch);

@@ -6,7 +6,8 @@
 //   trsv_blocked                  mdivide_left_tri_low inside multi_normal_cholesky
 //                                 (models/fit_hyperparameters.stan:31) when no inverse is wanted
 //   finalize                      lml = -n/2 log 2pi - sum log L_ii - 0.5 ||z||^2 and the three
-//                                 gradient components from the fused trace partials
+//                                 gradient components from the fused trace partials (and the ARD and
+//                                 derivative-observation forms of the same)
 //   hermite                       covariance.cpp:63-66,85-88 / cubic_interpolated_gp.hpp:63-70
 #include <algorithm>
 
@@ -686,6 +687,73 @@ int launch_finalize(Handle *h, int n, int np, int want_grad, const double *dvec,
                     const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch) {
   ProfScope ps__(h, PC_OTHER);
   finalize_kernel<<<batch, 256, 0, h->stream>>>(n, np, want_grad, dvec, z, a, partial, ntasks, ntasks2, theta, lml, grad);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+// The same for the ARD LML (EPI_TRACE_ARD partials: S_e = sum M e, S_d = sum M e q_d^2 on the coordinates divided by
+// rho_d, tr G); theta = (alpha, rho_1 .. rho_D, sigma) per item, grad in the same layout.  Every thread sums the first
+// region, then the second (diagonal-split) region, in a fixed order: the result does not depend on the schedule.
+__global__ void __launch_bounds__(256) finalize_ard_kernel(int n, int D, int np, int want_grad, const double *__restrict__ dvec,
+                                                          const double *__restrict__ z, const double *__restrict__ a,
+                                                          const double *__restrict__ partial, int ntasks, int ntasks2,
+                                                          const double *__restrict__ theta, double *__restrict__ lml,
+                                                          double *__restrict__ grad) {
+  constexpr int PW = epi_partial_width(EPI_TRACE_ARD), NV = 3 + PW;  // logdet, quad, aa, the partial record
+  __shared__ double red[8][NV];
+  const long long b = blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, ts = D + 2;
+  double v[NV];
+#pragma unroll
+  for (int c = 0; c < NV; c++) v[c] = 0.0;
+  for (int i = tid; i < n; i += 256) {
+    v[0] += log(dvec[b * np + i]);
+    const double zi = z[b * np + i];
+    v[1] = fma(zi, zi, v[1]);
+    if (want_grad) {
+      const double ai = a[b * np + i];
+      v[2] = fma(ai, ai, v[2]);
+    }
+  }
+  if (want_grad) {
+    for (int q = tid; q < ntasks; q += 256) {
+      const double *pp = partial + (b * ntasks + q) * PW;
+#pragma unroll
+      for (int c = 0; c < PW; c++) v[3 + c] += pp[c];
+    }
+    const double *part2 = partial + (long long)gridDim.x * ntasks * PW;
+    for (int q = tid; q < ntasks2; q += 256) {
+      const double *pp = part2 + (b * ntasks2 + q) * PW;
+#pragma unroll
+      for (int c = 0; c < PW; c++) v[3 + c] += pp[c];
+    }
+  }
+#pragma unroll
+  for (int c = 0; c < NV; c++) v[c] = warp_sum(v[c]);
+  if (lane == 0)
+#pragma unroll
+    for (int c = 0; c < NV; c++) red[warp][c] = v[c];
+  __syncthreads();
+  if (tid == 0) {
+    double s[NV];
+    for (int c = 0; c < NV; c++) s[c] = 0.0;
+    for (int w = 0; w < 8; w++)
+      for (int c = 0; c < NV; c++) s[c] += red[w][c];
+    lml[b] = -0.5 * n * 1.8378770664093454835606594728112 - s[0] - 0.5 * s[1];
+    if (want_grad) {
+      const double *th = theta + b * ts;
+      const double alpha = th[0], sigma = th[D + 1];
+      grad[b * ts + 0] = alpha * s[3];                                       // 0.5 sum M * 2 alpha e
+      for (int d = 0; d < D; d++) grad[b * ts + 1 + d] = 0.5 * alpha * alpha * s[4 + d] / th[1 + d];  // 0.5 sum M * alpha^2 e q_d^2 / rho_d
+      grad[b * ts + D + 1] = sigma * (s[2] - s[3 + PW - 1]);                // 0.5 tr(M) 2 sigma
+    }
+  }
+}
+
+int launch_finalize_ard(Handle *h, int n, int D, int np, int want_grad, const double *dvec, const double *z, const double *a,
+                        const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch) {
+  ProfScope ps__(h, PC_OTHER);
+  finalize_ard_kernel<<<batch, 256, 0, h->stream>>>(n, D, np, want_grad, dvec, z, a, partial, ntasks, ntasks2, theta, lml, grad);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

@@ -53,6 +53,12 @@ def gp_lml_grad_draws(x, y, theta, jitter=0.0, want_grad=True, handle=None):
     return (handle or capi.default_handle()).lml_grad_batched(x, y, theta, jitter, want_grad)
 
 
+def gp_lml_grad_ard_draws(X, y, theta, jitter=0.0, want_grad=True, handle=None):
+    """The same with the ARD covariance (QQard) on multi-column inputs: X (n, D) shared or (B, n, D) per item,
+    theta (B, D + 2) = (alpha, rho_1 .. rho_D, sigma); y (n,) or (B, n)."""
+    return (handle or capi.default_handle()).lml_grad_ard_batched(X, y, theta, jitter, want_grad)
+
+
 def fit_hyperparameters_lp(x, y, log_rho, log_alpha, log_sigma, handle=None):
     """lp__ and its gradient w.r.t. the unconstrained (log rho, log alpha, log sigma) for
     models/fit_hyperparameters.stan: `~` likelihood (constant dropped, :31), gamma(4,4) and

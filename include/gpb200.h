@@ -177,6 +177,16 @@ GPB200_API int gpb200_lml_grad_deriv_batched(gpb200_handle_t h, int n, int order
                                              long long y_stride, const double *theta, double jitter,
                                              int want_grad, double *lml, double *grad, int *info);
 
+/* LML + gradient of B GPs with the ARD squared-exponential covariance (QQard, R/kernels.R:19):
+ *   K = alpha^2 exp(-0.5 sum_d (X[i,d] - X[j,d])^2 / rho_d^2) + (sigma^2 + jitter) I,   1 <= D <= 8
+ * X: per item an n x D column-major matrix with leading dimension n (an R matrix); x_stride in doubles between items
+ * (0 = shared, else >= n*D); y, y_stride as in gpb200_lml_grad_batched; theta and grad: B x (D + 2) row-major,
+ * (alpha, rho_1 .. rho_D, sigma); lml[B], info[B] with the conventions of gpb200_lml_grad_batched.
+ * want_grad = 0 skips the inverse.  At D = 1 this is the model of gpb200_lml_grad_batched. */
+GPB200_API int gpb200_lml_grad_ard_batched(gpb200_handle_t h, int n, int D, int B, const double *X, long long x_stride,
+                                           const double *y, long long y_stride, const double *theta, double jitter,
+                                           int want_grad, double *lml, double *grad, int *info);
+
 /* ---- a1-a3: the reference's one native entry point ----------------------------------------- */
 /* Exact twin of rbf_cov_chol (covariance.cpp:9-47): Sigma = exp(-(xi-xj)^2/(2 l^2)) + 1e-10 I,
  * L = chol(Sigma), dLdl = d L / d l (forward mode); both n x n column-major with zero strict

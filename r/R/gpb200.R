@@ -67,6 +67,9 @@ mvrnorm <- function(n = 1, mu, Sigma, seed = sample.int(.Machine$integer.max, 1)
 # ---- batched LML + gradient over hyper-parameter draws (the mclapply axis, pendulum_fit.R:259-268) -
 # theta: 3 x B matrix, one (alpha, rho, sigma) per COLUMN
 gp_lml_grad_draws <- function(x, y, theta, jitter = 0) .Call("gp_lml_grad_draws", x, y, theta, jitter)
+# ARD covariance QQard(X, X, c(alpha, rho)) + (sigma^2 + jitter) I on the n x D matrix X (D <= 8): theta is
+# (D + 2) x B, one (alpha, rho_1 .. rho_D, sigma) per column; grad has the same layout
+gp_lml_grad_ard_draws <- function(X, y, theta, jitter = 0) .Call("gp_lml_grad_ard_draws", as.matrix(X), y, theta, jitter)
 
 # ---- GP observed through derivatives (the Stan model inside gpderivs.py:25-133; design_notes.Rmd:25-46) ----
 # theta: (2 + nblocks) x B matrix, columns (alpha, rho, noise_1..noise_nblocks); y = c(y, yp, ypp) stacked

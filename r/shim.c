@@ -312,6 +312,30 @@ SEXP gp_lml_grad_draws(SEXP x_, SEXP y_, SEXP theta_, SEXP jitter) {
   return out;
 }
 
+/* LML + gradient for B draws with the ARD covariance (QQard of R/kernels.R:19) on the n x D matrix X (1 <= D <= 8):
+ * theta is a (D + 2) x B matrix (alpha, rho_1 .. rho_D, sigma per column), grad has the same layout */
+SEXP gp_lml_grad_ard_draws(SEXP X_, SEXP y_, SEXP theta_, SEXP jitter) {
+  int np = 0;
+  SEXP X = as_real(X_, &np, "X"), y = as_real(y_, &np, "y"), theta = as_real(theta_, &np, "theta");
+  const int n = Rf_nrows(X), D = Rf_ncols(X), B = Rf_ncols(theta);
+  if (D < 1 || D > 8) Rf_error("gp_lml_grad_ard_draws: X must have 1 to 8 columns (got %d)", D);
+  if (LENGTH(y) != n) Rf_error("gp_lml_grad_ard_draws: length(y) = %d must equal nrow(X) = %d", LENGTH(y), n);
+  if (Rf_nrows(theta) != D + 2)
+    Rf_error("gp_lml_grad_ard_draws: theta must be a (ncol(X) + 2) x B matrix, one (alpha, rho[D], sigma) per COLUMN "
+             "(got %d x %d)", Rf_nrows(theta), B);
+  SEXP lml = PROTECT(Rf_allocVector(REALSXP, B));
+  SEXP grad = PROTECT(Rf_allocMatrix(REALSXP, D + 2, B));
+  SEXP info = PROTECT(Rf_allocVector(INTSXP, B));
+  np += 3;
+  check(gpb200_lml_grad_ard_batched(handle(), n, D, B, REAL(X), 0, REAL(y), 0, REAL(theta), Rf_asReal(jitter), 1,
+                                    REAL(lml), REAL(grad), INTEGER(info)), "lml_grad_ard_draws");
+  SEXP elts[3] = {lml, grad, info};
+  static const char *const names[3] = {"lml", "grad", "info"};
+  SEXP out = named_list(3, elts, names);
+  UNPROTECT(np);
+  return out;
+}
+
 /* LML + gradient of a GP observed through derivative orders order0 .. order0+nblocks-1 on the grid t
  * (gpderivs.py:62-83 is order0 = 1, nblocks = 1; design_notes.Rmd:25-46 is 0, 3); theta is a
  * (2 + nblocks) x B matrix (alpha, rho, noise[nblocks] per column), y the stacked observations */
@@ -446,7 +470,7 @@ static const R_CallMethodDef call_methods[] = {
     {"gp_gram_outer", (DL_FUNC)&gp_gram_outer, 5},     {"gp_kernel_eval", (DL_FUNC)&gp_kernel_eval, 5},
     {"gp_gram_ard", (DL_FUNC)&gp_gram_ard, 4},         {"gp_gram_deriv", (DL_FUNC)&gp_gram_deriv, 7},
     {"gp_potrf", (DL_FUNC)&gp_potrf, 1},               {"gp_potrs", (DL_FUNC)&gp_potrs, 2},
-    {"gp_lml_grad_draws", (DL_FUNC)&gp_lml_grad_draws, 4},
+    {"gp_lml_grad_draws", (DL_FUNC)&gp_lml_grad_draws, 4}, {"gp_lml_grad_ard_draws", (DL_FUNC)&gp_lml_grad_ard_draws, 4},
     {"gp_condition", (DL_FUNC)&gp_condition, 6},       {"gp_cond_mvn", (DL_FUNC)&gp_cond_mvn, 4},
     {"gp_rbf_cov_chol_grid", (DL_FUNC)&gp_rbf_cov_chol_grid, 2}, {"gp_approx_L_basis", (DL_FUNC)&gp_approx_L_basis, 5},
     {"gp_se_chol_tangent", (DL_FUNC)&gp_se_chol_tangent, 5},
