@@ -88,6 +88,9 @@ SIGNATURES = {
     "gpb200_posterior_draws_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, _ll,
                                                  C.c_void_p, _ll, C.c_void_p, C.c_double, C.c_void_p, C.c_ulonglong,
                                                  C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gpb200_posterior_draws_ard_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p,
+                                                     _ll, C.c_void_p, _ll, C.c_void_p, C.c_double, C.c_void_p, C.c_ulonglong,
+                                                     C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_mg_gram_panel": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_int, C.c_int,
                                        C.c_void_p, _ll]),
     "gpb200_mg_panel_factor": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p]),
@@ -573,6 +576,52 @@ class Handle:
         self._check(self.lib.gpb200_posterior_draws_batched(self._h, n, m, order, B, _ptr(t), t_stride, _ptr(s), s_stride,
                                                             _ptr(y), y_stride, _ptr(theta), jitter, _ptr(z), int(seed),
                                                             _ptr(draws), _ptr(mu), _ptr(info)), "posterior_draws_batched")
+
+    def posterior_draws_ard_batched(self, X, y, theta, Xs=None, jitter=1e-8, seed=None, z=None):
+        """One posterior draw of f on Xs (on X when Xs is None) per hyper-parameter row theta[b] = (alpha, rho_1 ..
+        rho_D, sigma) of the ARD kernel, given y observed on X (include/gpb200.h: gpb200_posterior_draws_ard_batched).
+        X: (n, D) or (B, n, D); Xs: (m, D) or (B, m, D); y: (n,) or (B, n); z: (B, m) normals, else the device stream of
+        `seed` (0 when None).  Returns draws (B, m), mu (B, m), info (B,)."""
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        X = np.asarray(X, dtype=np.float64); y = np.ascontiguousarray(y, dtype=np.float64)
+        if X.ndim not in (2, 3) or y.ndim not in (1, 2):
+            raise ValueError("X must be (n, D) or (B, n, D) and y (n,) or (B, n)")
+        n, D = X.shape[-2], X.shape[-1]
+        if th.ndim != 2 or th.shape[1] != D + 2:
+            raise ValueError("theta must be (B, D + 2) = (alpha, rho_1 .. rho_D, sigma) per row")
+        B = th.shape[0]
+        if y.shape[-1] != n or (X.ndim == 3 and X.shape[0] != B) or (y.ndim == 2 and y.shape[0] != B):
+            raise ValueError("X and y must hold n points, shared or one set per row of theta")
+        Xs_c = None
+        if Xs is not None:
+            Xs = np.asarray(Xs, dtype=np.float64)
+            if Xs.ndim not in (2, 3) or Xs.shape[-1] != D or (Xs.ndim == 3 and Xs.shape[0] != B):
+                raise ValueError("Xs must be (m, D) or (B, m, D) with the D columns of X")
+            Xs_c = np.ascontiguousarray(np.swapaxes(Xs, -1, -2))  # each item column-major m x D
+        m = n if Xs is None else Xs.shape[-2]
+        z_a = None
+        if z is not None:
+            z_a = np.ascontiguousarray(z, dtype=np.float64)
+            if z_a.shape != (B, m):
+                raise ValueError("z must be (B, m)")
+        Xc = np.ascontiguousarray(np.swapaxes(X, -1, -2))
+        draws = np.empty((B, m)); mu = np.empty((B, m)); info = np.zeros(B, dtype=np.int32)
+        self._check(self.lib.gpb200_posterior_draws_ard_batched(
+            self._h, n, m, D, B, _ptr(Xc), n * D if X.ndim == 3 else 0, _ptr(Xs_c),
+            m * D if Xs is not None and Xs.ndim == 3 else 0, _ptr(y), n if y.ndim == 2 else 0, _ptr(th), float(jitter),
+            _ptr(z_a), int(seed or 0), _ptr(draws), _ptr(mu), _ptr(info)), "posterior_draws_ard_batched")
+        return draws, mu, info
+
+    def posterior_draws_ard_batched_device(self, n, m, D, B, X, x_stride, Xs, xs_stride, y, y_stride, theta, jitter, z,
+                                           seed, draws, mu, info):
+        """Device-pointer variant: every array argument is a torch CUDA tensor (float64 / int32) or None, X and Xs
+        holding per item column-major n x D and m x D matrices; the handle must be in device-pointer mode.  Asynchronous
+        on the handle's stream."""
+        assert self.device_pointers
+        self._check(self.lib.gpb200_posterior_draws_ard_batched(self._h, n, m, D, B, _ptr(X), x_stride, _ptr(Xs), xs_stride,
+                                                                _ptr(y), y_stride, _ptr(theta), jitter, _ptr(z), int(seed),
+                                                                _ptr(draws), _ptr(mu), _ptr(info)),
+                    "posterior_draws_ard_batched")
 
 
 _default = {}

@@ -359,7 +359,22 @@ __global__ void __launch_bounds__(256) gram_ard_kernel(int n, int m, int D, cons
   }
 }
 
-// ---- batched padded ARD Gram for the fused LML path (gpb200_lml_grad_ard_batched) -----------------
+// ---- batched padded ARD Grams (gpb200_lml_grad_ard_batched, gpb200_posterior_draws_ard_batched) ----
+// Squared scaled distance r^2 = sum_d (xs[r] - ys[c])^2 between staged row point r and column point c (coordinates
+// already divided by rho_d, one dimension every TILE doubles), accumulated over d in order.  It is symmetric to the bit
+// ((a - b)^2 == (b - a)^2).  Both ARD Gram kernels turn it into alpha^2 exp(-r^2 / 2) themselves: written as one
+// helper, the whole element changes the register allocation of gram_ard_batched_kernel; this part leaves its SASS as
+// it was.  exp_nonpos clamps its argument with fmax, which drops a NaN: a NaN coordinate or length-scale must reach
+// the factorisation (and fail its item) as it does in the reference, hence the isnan pass-through in both kernels.
+__device__ __forceinline__ double ard_r2(const double *xs, const double *ys, int r, int c, int D) {
+  double r2 = 0.0;
+  for (int d = 0; d < D; d++) {
+    const double dq = xs[d * TILE + r] - ys[d * TILE + c];
+    r2 = fma(dq, dq, r2);
+  }
+  return r2;
+}
+
 // K = alpha^2 exp(-0.5 sum_d ((X_id - X_jd) / rho_d)^2) + c I: QQard of R/kernels.R:19 plus the noise diagonal.
 // X per item is n x D column-major (leading dimension n); theta per item (alpha, rho_1 .. rho_D, sigma).  Layout as
 // gram_se_batched_kernel: np x np per item, identity in the padding, lower tiles only.  The coordinates are staged
@@ -396,14 +411,61 @@ __global__ void __launch_bounds__(256) gram_ard_batched_kernel(int n, int D, int
     for (int e = 0; e < 2; e++) {
       const int i = r0 + rl + e;
       if (i < n && j < n) {
-        double r2 = 0.0;
-        for (int d = 0; d < D; d++) {
-          const double dq = xs[d * TILE + rl + e] - ys[d * TILE + cl];
-          r2 = fma(dq, dq, r2);
-        }
-        // exp_nonpos clamps its argument with fmax, which drops a NaN: a NaN coordinate or length-scale must reach
-        // the factorisation (and fail its item) as it does in the reference
+        const double r2 = ard_r2(xs, ys, rl + e, cl, D);
         v[e] = (i == j) ? a2 + dadd : a2 * (isnan(r2) ? r2 : exp_nonpos(-0.5 * r2));
+      } else {
+        v[e] = (i == j) ? 1.0 : 0.0;
+      }
+    }
+    *reinterpret_cast<double2 *>(Kb + (r0 + rl) + (long long)j * np) = make_double2(v[0], v[1]);
+  }
+}
+
+// Joint prior covariance of the noisy values f(X) + noise and f(Xs) under the ARD kernel, for conditioning and drawing
+// in one factorisation (gpb200_posterior_draws_ard_batched):
+//   J = [[QQard(X, X) + sigma^2 I,  .                       ],
+//        [QQard(Xs, X),             QQard(Xs, Xs) + jitter I]]
+// rows [0, n) from X (n x D per item, leading dimension n), rows [n, n+m) from Xs (m x D, leading dimension m);
+// theta = (alpha, rho_1 .. rho_D, sigma) per item.  Layout as gram_cond_batched_kernel: np x np per item, identity in
+// the padding, lower tiles only, the strict upper part of a diagonal tile mirrored (ard_r2 is symmetric).  The
+// elements are those of gram_ard_batched_kernel.
+__global__ void __launch_bounds__(256) gram_cond_ard_batched_kernel(int n, int m, int D, int np,
+                                                                   const double *__restrict__ X, long long x_stride,
+                                                                   const double *__restrict__ Xs, long long xs_stride,
+                                                                   const double *__restrict__ theta, double jitter,
+                                                                   double *__restrict__ K, long long stride) {
+  const int nt = np / TILE;
+  const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
+  if (tr < tc) return;
+  __shared__ double xs[ARD_MAX_D * TILE], ys[ARD_MAX_D * TILE];
+  const long long b = blockIdx.y;
+  const double *Xb = X + b * x_stride, *Sb = Xs + b * xs_stride;
+  const double *th = theta + b * (D + 2);
+  const int N = n + m;
+  const int r0 = tr * TILE, c0 = tc * TILE, tid = threadIdx.x;
+  for (int q = tid; q < D * 2 * TILE; q += 256) {
+    const int d = q / (2 * TILE), l = q % (2 * TILE);
+    const int i = (l < TILE) ? r0 + l : c0 + l - TILE;
+    const double v = (i < n) ? Xb[i + (long long)d * n] / th[1 + d] : (i < N) ? Sb[i - n + (long long)d * m] / th[1 + d] : 0.0;
+    if (l < TILE) xs[d * TILE + l] = v;
+    else ys[d * TILE + l - TILE] = v;
+  }
+  __syncthreads();
+  const double alpha = th[0], sigma = th[D + 1];
+  const double a2 = alpha * alpha;
+  double *Kb = K + b * stride;
+  const int rl = 2 * (tid & 63), cq = tid >> 6;
+#pragma unroll 2
+  for (int s = 0; s < 32; s++) {
+    const int cl = cq + 4 * s;
+    const int j = c0 + cl;
+    double v[2];
+#pragma unroll
+    for (int e = 0; e < 2; e++) {
+      const int i = r0 + rl + e;
+      if (i < N && j < N) {
+        const double r2 = ard_r2(xs, ys, rl + e, cl, D);
+        v[e] = (i == j) ? a2 + (i < n ? sigma * sigma : jitter) : a2 * (isnan(r2) ? r2 : exp_nonpos(-0.5 * r2));
       } else {
         v[e] = (i == j) ? 1.0 : 0.0;
       }
@@ -543,6 +605,18 @@ int launch_gram_ard_batched(Handle *h, int n, int D, int np, const double *X, lo
   dim3 grid(nt * nt, batch);
   ProfScope ps__(h, PC_GRAM);
   gram_ard_batched_kernel<<<grid, 256, 0, h->stream>>>(n, D, np, X, x_stride, theta, jitter, K, stride);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+int launch_gram_cond_ard_batched(Handle *h, int n, int m, int D, int np, const double *X, long long x_stride,
+                                 const double *Xs, long long xs_stride, const double *theta, double jitter, double *K,
+                                 long long stride, int batch) {
+  const int nt = np / TILE;
+  dim3 grid(nt * nt, batch);
+  ProfScope ps__(h, PC_GRAM);
+  gram_cond_ard_batched_kernel<<<grid, 256, 0, h->stream>>>(n, m, D, np, X, x_stride, Xs, xs_stride, theta, jitter, K,
+                                                            stride);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

@@ -24,6 +24,9 @@ int launch_gram_cond_batched(Handle *h, int n, int m, int order, int np, const d
                              long long stride, int batch);
 int launch_gram_ard_batched(Handle *h, int n, int D, int np, const double *X, long long x_stride, const double *theta,
                             double jitter, double *K, long long stride, int batch);
+int launch_gram_cond_ard_batched(Handle *h, int n, int m, int D, int np, const double *X, long long x_stride,
+                                 const double *Xs, long long xs_stride, const double *theta, double jitter, double *K,
+                                 long long stride, int batch);
 int launch_gram_ard(Handle *h, int n, int m, int D, const double *X, long long ldx, const double *Y, long long ldy,
                     double alpha, const double *rho, int rho_len, double *K, long long ldk);
 

@@ -272,6 +272,20 @@ GPB200_API int gpb200_posterior_draws_batched(gpb200_handle_t h, int n, int m, i
                                               long long t_stride, const double *s, long long s_stride, const double *y,
                                               long long y_stride, const double *theta, double jitter, const double *z,
                                               unsigned long long seed, double *draws, double *mu, int *info);
+/* The same B posterior draws for the ARD squared-exponential kernel (QQard, R/kernels.R:19) on D-column inputs,
+ * 1 <= D <= 8 (the states of create_p_dotXnS, R/ode_gp_library.R:43-93).  For item b, with
+ * k(p, q) = alpha^2 exp(-0.5 sum_d (p_d - q_d)^2 / rho_d^2):
+ *   K = k(X, X) + sigma^2 I  (n x n),  Ks = k(Xs, X)  (m x n),  Kss = k(Xs, Xs)  (m x m)
+ *   mu = Ks K^-1 y,   cov = Kss - Ks K^-1 Ks^T + jitter I,   draw_b = mu + chol(cov) eps_b
+ * X: per item n x D column-major with leading dimension n (an R matrix); Xs: per item m x D with leading dimension m;
+ * x_stride / xs_stride in doubles between items (0 = shared, else >= n*D / m*D); Xs == NULL predicts on X (then
+ * m == n).  theta: B x (D + 2) row-major, (alpha, rho_1 .. rho_D, sigma) as in gpb200_lml_grad_ard_batched.  y, z,
+ * seed, draws, mu and info as in gpb200_posterior_draws_batched.  At D = 1 this is its order-0 model. */
+GPB200_API int gpb200_posterior_draws_ard_batched(gpb200_handle_t h, int n, int m, int D, int B, const double *X,
+                                                  long long x_stride, const double *Xs, long long xs_stride,
+                                                  const double *y, long long y_stride, const double *theta, double jitter,
+                                                  const double *z, unsigned long long seed, double *draws, double *mu,
+                                                  int *info);
 
 /* ---- (e) multi-GPU block-cyclic Cholesky of ONE large matrix: per-rank building blocks ------------
  * DEVICE pointers only.  A panel is a block column of the padded matrix (np = ceil(n/128)*128)

@@ -59,6 +59,15 @@ sample_derivs_draws <- function(params, ynoise, ti, seed = NULL) {
   z <- if (is.null(seed)) matrix(rnorm(length(ti) * ncol(params)), length(ti), ncol(params)) else NULL
   .Call("gp_sample_derivs_draws", params, ynoise, ti, seed, z)
 }
+# one posterior draw of f on the states Xs (on X when Xs is NULL) per ARD hyper-parameter draw: theta is (D + 2) x B,
+# one (alpha, rho_1 .. rho_D, sigma) per COLUMN as gp_lml_grad_ard_draws takes it; returns an nrow(Xs) x B matrix
+gp_posterior_draws_ard <- function(X, y, theta, Xs = NULL, jitter = 1e-8, seed = NULL) {
+  X <- as.matrix(X); theta <- as.matrix(theta)
+  if (!is.null(Xs)) Xs <- as.matrix(Xs)
+  m <- if (is.null(Xs)) nrow(X) else nrow(Xs)
+  z <- if (is.null(seed)) matrix(rnorm(m * ncol(theta)), m, ncol(theta)) else NULL
+  .Call("gp_posterior_draws_ard", X, y, theta, Xs, jitter, seed, z)
+}
 mvrnorm <- function(n = 1, mu, Sigma, seed = sample.int(.Machine$integer.max, 1)) {   # MASS::mvrnorm signature + seed
   out <- .Call("gp_mvrnorm", as.integer(n), mu, Sigma, seed)
   if (n == 1) drop(out) else out

@@ -418,6 +418,49 @@ SEXP gp_sample_derivs_draws(SEXP params_, SEXP ynoise_, SEXP ti_, SEXP seed, SEX
   return out;
 }
 
+/* Posterior draws of f on the states Xs (on X when Xs is NULL) under the ARD covariance QQard (R/kernels.R:19), one per
+ * COLUMN (alpha, rho_1 .. rho_D, sigma) of the (D + 2) x B matrix theta, given y observed on the n x D matrix X (the
+ * states of create_p_dotXnS, R/ode_gp_library.R:43-93).  Normals: the device stream of `seed`, or the m x B matrix z when
+ * seed is NULL.  Returns an m x B matrix, column b = mu_b + chol(cov_b) eps_b. */
+SEXP gp_posterior_draws_ard(SEXP X_, SEXP y_, SEXP theta_, SEXP Xs_, SEXP jitter, SEXP seed, SEXP z_) {
+  int np = 0;
+  SEXP X = as_real(X_, &np, "X"), y = as_real(y_, &np, "y"), theta = as_real(theta_, &np, "theta");
+  const int n = Rf_nrows(X), D = Rf_ncols(X), B = Rf_ncols(theta);
+  if (n < 1) Rf_error("gp_posterior_draws_ard: X must have at least one row");
+  if (D < 1 || D > 8) Rf_error("gp_posterior_draws_ard: X must have 1 to 8 columns (got %d)", D);
+  if (LENGTH(y) != n) Rf_error("gp_posterior_draws_ard: length(y) = %d must equal nrow(X) = %d", LENGTH(y), n);
+  if (Rf_nrows(theta) != D + 2)
+    Rf_error("gp_posterior_draws_ard: theta must be a (ncol(X) + 2) x B matrix, one (alpha, rho[D], sigma) per COLUMN "
+             "(got %d x %d)", Rf_nrows(theta), B);
+  const double *xs = NULL;
+  int m = n;
+  if (!Rf_isNull(Xs_)) {
+    SEXP Xs = as_real(Xs_, &np, "Xs");
+    m = Rf_nrows(Xs);
+    if (m < 1 || Rf_ncols(Xs) != D)
+      Rf_error("gp_posterior_draws_ard: Xs must be a matrix with ncol(X) = %d columns and at least one row (got %d x %d)",
+               D, m, Rf_ncols(Xs));
+    xs = REAL(Xs);
+  }
+  const double *z = NULL;
+  if (Rf_isNull(seed)) {
+    SEXP zr = as_real(z_, &np, "z (normals, needed when seed is NULL)");
+    need_matrix(zr, m, B, "z");
+    z = REAL(zr);
+  }
+  SEXP out = PROTECT(Rf_allocMatrix(REALSXP, m, B));
+  SEXP info = PROTECT(Rf_allocVector(INTSXP, B));
+  np += 2;
+  check(gpb200_posterior_draws_ard_batched(handle(), n, m, D, B, REAL(X), 0, xs, 0, REAL(y), 0, REAL(theta), Rf_asReal(jitter),
+                                           z, z ? 0ULL : (unsigned long long)Rf_asReal(seed), REAL(out), NULL, INTEGER(info)),
+        "posterior_draws_ard");
+  for (int b = 0; b < B; b++)
+    if (INTEGER(info)[b]) Rf_error("gp_posterior_draws_ard: draw %d: matrix is not positive definite (first non-positive pivot at %d)",
+                                   b + 1, INTEGER(info)[b]);
+  UNPROTECT(np);
+  return out;
+}
+
 /* mu = Ks (K + s2 I)^-1 y ; cov = Kss - Ks (K + s2 I)^-1 Ks^T + jitter I   [pendulum_fit.R:242-251] */
 SEXP gp_condition(SEXP K_, SEXP Ks_, SEXP Kss_, SEXP y_, SEXP noise_var, SEXP jitter) {
   int np = 0;
@@ -476,6 +519,7 @@ static const R_CallMethodDef call_methods[] = {
     {"gp_se_chol_tangent", (DL_FUNC)&gp_se_chol_tangent, 5},
     {"gp_lml_grad_deriv_draws", (DL_FUNC)&gp_lml_grad_deriv_draws, 5}, {"gp_mvrnorm", (DL_FUNC)&gp_mvrnorm, 4},
     {"gp_sample_derivs_draws", (DL_FUNC)&gp_sample_derivs_draws, 5},
+    {"gp_posterior_draws_ard", (DL_FUNC)&gp_posterior_draws_ard, 7},
     {NULL, NULL, 0}};
 
 void R_init_gpb200_r(DllInfo *dll) {
