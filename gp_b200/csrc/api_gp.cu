@@ -52,9 +52,9 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   const bool use_env = !sp.deriv && !ard && h->envelope && !small && nt >= 16 && nt <= ENV_MAX_NT;
   const bool sinv = use_env && want_grad && (h->sinv_min_batch > 0 ? B >= h->sinv_min_batch : (long long)B * nt >= 256);
   const size_t per_item = small ? 0 : pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * pw * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) + 64 +
-                                      (use_env ? (size_t)2 * nt * sizeof(int) : 0);
+                                      (use_env ? (size_t)(2 * nt + 2) * sizeof(int) : 0);
   const size_t fixed = pad256((size_t)B * (x_stride ? xl : 0) * 8 + (size_t)xl * 8) + pad256((size_t)B * (y_stride ? n : 0) * 8 + n * 8) +
-                       2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096 + (use_env ? 256 : 0);
+                       2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096 + (use_env ? 512 : 0);
   int Bc = B;
   if (!small && (h->ws_limit > 0 || fixed + per_item * (size_t)B + 8192 > h->ws_bytes)) {
     size_t limit = (size_t)h->ws_limit;
@@ -77,13 +77,14 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   double *dlml = a.take<double>(B), *dgrad = a.take<double>((size_t)B * ts);
   int *dinfo = a.take<int>(B);
   double *Lbuf = nullptr, *Sbuf = nullptr, *zbuf = nullptr, *abuf = nullptr, *dvec = nullptr, *partial = nullptr, *zpart = nullptr;
-  int *env = nullptr;
+  int *env = nullptr, *order = nullptr;
   if (!small) {
     Lbuf = a.take<double>((size_t)Bc * mat); Sbuf = a.take<double>((size_t)Bc * mat);
     zbuf = a.take<double>((size_t)Bc * np); abuf = a.take<double>((size_t)Bc * np); dvec = a.take<double>((size_t)Bc * np);
     partial = a.take<double>((size_t)Bc * nparts * pw);
     zpart = zks > 1 ? a.take<double>((size_t)Bc * zks * np) : nullptr;
-    if (use_env && !(env = a.take<int>((size_t)Bc * 2 * nt))) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
+    if (use_env && (!(env = a.take<int>((size_t)Bc * 2 * nt)) || !(order = a.take<int>((size_t)Bc * 2))))
+      BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
     if (!partial) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
   }
   if (!dinfo) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
@@ -100,16 +101,16 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       else {
         if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
         RC(launch_gram_se_batched(h, n, np, cx, xs, cth, jitter, 1, Lbuf, mat, bc, env));
-        if (env) RC(launch_envelope_profile(h, nt, env, bc));
+        if (env) RC(launch_envelope_profile(h, nt, env, order, bc));
       }
-      RC(chol_batched(h, Lbuf, np, mat, n, bc, dinfo + b0, env));
+      RC(chol_batched(h, Lbuf, np, mat, n, bc, dinfo + b0, env, order));
       RC(extract_diag(h, np, Lbuf, mat, dvec, bc));
       int n1 = 0, n2 = 0;
       if (sinv) {
         RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
         RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, cy, ys, nullptr, n, zbuf, np, bc, env));
         RC(launch_backsub_band(h, np, Lbuf, Sbuf, mat, env, zbuf, abuf, bc));
-        RC(sinv_batched(h, Lbuf, Sbuf, np, mat, env, bc));
+        RC(sinv_batched(h, Lbuf, Sbuf, np, mat, env, order, bc));
         RC(launch_trace_sinv(h, n, np, Lbuf, mat, env, cx, xs, abuf, cth, partial, bc));
         n1 = ntasks;
       } else if (want_grad) {

@@ -66,6 +66,7 @@ struct GemmParams {
   // tile row), env[nt..2nt) = E (last tile row I with F_I <= J, per tile column J); item stride 2 * env_nt
   const int *env;
   int env_nt, env_mode;
+  const int *order;             // envelope launches: item of blockIdx.y (envelope_order_kernel); nullptr: blockIdx.y itself
   MatRef CT;                    // EPI_AXPBY: when CT.p is set the transpose of the output tile is written there too
   unsigned long long *flops;    // when set: every CTA adds the flops it executes (after all skipping)
   int ard_d;                    // EPI_TRACE_ARD: input dimensions D (x is n x D column-major per item, theta_stride = D + 2)
@@ -75,6 +76,16 @@ struct GemmParams {
 enum { ENV_NONE = 0,
        ENV_CHOL = 1,   // C(I,J) -= L(I,k) L(J,k)^T: exit when J < F_I (tile outside the profile), k starts at max(F_I, F_J)
        ENV_BAND = 2 }; // selected inverse: exit when I > E_J, the contraction ends at tile E_J
+
+// Tile envelope of the batched TRSM below diagonal tile `col` (the throughput TRSM kernels of panel.cu): F points at the
+// F entry of the first row tile of item 0, item stride `stride`.  Row tile r (counted from the first) is live when
+// F[r] <= col.  Any other C tile is exactly zero -- the Gram wrote +0.0 there and no update touched it -- and so would
+// its solution be, so it is left as it is.  F need not be monotone (unsorted inputs), so every tile is tested.
+struct TrsmEnv {
+  const int *F = nullptr;  // nullptr: every tile is live (dense route)
+  int stride = 0, col = 0;
+  __device__ bool live(int item, int r) const { return !F || F[(long long)item * stride + r] <= col; }
+};
 
 struct Handle {
   int device = 0;
@@ -230,18 +241,20 @@ int launch_tile_inverse(Handle *h, const double *L, double *W, long long ld, lon
 int launch_potrf_tile_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base,
                          int n, int batch, int *info);
 int launch_trsm_tiles_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, long long c_off,
-                         int ntiles, int batch);
+                         int ntiles, int batch, TrsmEnv env = TrsmEnv{});
 // POTRF of the diagonal tile at diag_off, then TRSM of the `ntiles` tiles from c_off down: one fused launch on the
-// latency path, otherwise the two launches above
+// latency path, otherwise the two launches above (whose TRSM solves only the tiles live under `env`)
 int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base, int n,
-                         long long c_off, int ntiles, int batch, int *info);
+                         long long c_off, int ntiles, int batch, int *info, TrsmEnv env = TrsmEnv{});
+// env: the tile envelope of each item (F, E with item stride 2 * ld / TILE, see GemmParams), or nullptr
 int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int tile_col, int ntiles_below, int n, int batch,
-                      int *info);
+                      int *info, const int *env = nullptr);
 int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l_off, long long l_step, double *W,
                            long long w_off, long long w_step, long long stride, int ntiles, int batch);
 // tile envelope of the SE path (solve.cu): E from F (F filled by gram_se_batched), the trace of the selected inverse
-// and the band-limited back substitution
-int launch_envelope_profile(Handle *h, int nt, int *env, int batch);
+// and the band-limited back substitution.  launch_envelope_profile also writes the dispatch order of the envelope GEMM
+// launches to order[0..batch) (order[batch..2 batch) is its scratch)
+int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch);
 int launch_trace_sinv(Handle *h, int n, int np, const double *Z, long long stride, const int *env, const double *x,
                       long long x_stride, const double *a, const double *theta, double *partial, int batch);
 int launch_backsub_band(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const int *env,

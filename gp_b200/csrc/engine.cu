@@ -165,8 +165,9 @@ int tasks_lauum(Handle *h, int nt, TaskList *out) {
 // engines on padded device buffers
 // ---------------------------------------------------------------------------------------------
 
-static void set_env(GemmParams &p, const int *env, int nt, int mode) {
+static void set_env(GemmParams &p, const int *env, const int *order, int nt, int mode) {
   p.env = env;
+  p.order = env ? order : nullptr;
   p.env_nt = nt;
   p.env_mode = env ? mode : ENV_NONE;
 }
@@ -238,7 +239,7 @@ static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int
   p.C0 = mref(Lbuf, np, stride);
   p.alpha = -1.0;
   p.beta = 1.0;
-  set_env(p, env, nt, ENV_CHOL);
+  set_env(p, env, nullptr, nt, ENV_CHOL);
   GemmParams pc = p;      // launches on the panel chain
   pc.latency_hint = 1;
   cudaStream_t T = h->stream, P = h->pstream;
@@ -278,7 +279,8 @@ static int chol_lookahead(Handle *h, double *Lbuf, int np, long long stride, int
   return 0;  // T has waited for the last panel (which follows every launch on P): the side stream is joined
 }
 
-int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env) {
+int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env,
+                 const int *order) {
   const int nt = np / TILE;
   if (chol_uses_lookahead(h, nt, batch)) return chol_lookahead(h, Lbuf, np, stride, n, batch, info_dev, env);
   const int pt = h->chol_panel_override > 0 ? std::min(nt, h->chol_panel_override) : chol_panel_tiles(nt, batch);
@@ -292,14 +294,14 @@ int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int b
   p.C0 = mref(Lbuf, np, stride);
   p.alpha = -1.0;
   p.beta = 1.0;
-  set_env(p, env, nt, ENV_CHOL);
+  set_env(p, env, order, nt, ENV_CHOL);
   for (int j = 0; j < nt; j++) {
     if (tl.count(j) > 0) {
       p.tasks = tl.at(j);
       rc = launch_gemm(h, LAYOUT_NT, EPI_AXPBY, p, tl.count(j), batch);
       if (rc) return rc;
     }
-    rc = launch_potrf_trsm(h, Lbuf, np, stride, j, nt - 1 - j, n, batch, info_dev);
+    rc = launch_potrf_trsm(h, Lbuf, np, stride, j, nt - 1 - j, n, batch, info_dev, env);
     if (rc) return rc;
     if ((j + 1) % pt == 0 && j + 1 < nt) {
       const int panel = j / pt;
@@ -383,12 +385,12 @@ static int tasks_sinv(Handle *h, int nt, TaskList *ty, TaskList *td, TaskList *t
   return upload_tasks(h, k4, zd, ozd, tzd);
 }
 
-int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, int batch) {
+int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, const int *order, int batch) {
   const int nt = np / TILE;
   TaskList ty, td, tz, tzd;
   RC(tasks_sinv(h, nt, &ty, &td, &tz, &tzd));
   GemmParams p{};
-  set_env(p, env, nt, ENV_BAND);
+  set_env(p, env, order, nt, ENV_BAND);
   p.alpha = 1.0;
   if (nt > 1) {
     p.A = mref(Lbuf, np, stride); p.B = mref(Sbuf, np, stride); p.C = mref(Sbuf, np, stride); p.tasks = ty.at(0);

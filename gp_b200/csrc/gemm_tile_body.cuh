@@ -12,8 +12,9 @@
   // the half of the item's envelope this launch uses (F for ENV_CHOL, E for ENV_BAND), read beside the task rather
   // than after it: on the dependent chain of the look-ahead Cholesky a second dependent load is a visible latency
   __shared__ int s_env[ENV_MAX_NT];
+  const long long b = p.order ? p.order[blockIdx.y] : blockIdx.y;  // the batch item
   if (p.env_mode != ENV_NONE) {
-    const int *src = p.env + (long long)blockIdx.y * 2 * p.env_nt + (p.env_mode == ENV_CHOL ? 0 : p.env_nt);
+    const int *src = p.env + b * 2 * p.env_nt + (p.env_mode == ENV_CHOL ? 0 : p.env_nt);
     for (int q = threadIdx.x; q < p.env_nt; q += Cfg::NTHREADS) s_env[q] = src[q];
     __syncthreads();
   }
@@ -41,7 +42,6 @@
     if (skip_last) task.k_len -= TILE / 2;
     if (sym_skip) task.k_len = 0;
   }
-  const long long b = blockIdx.y;
   if (p.env_mode != ENV_NONE) {  // the item's tile envelope: leave out the contraction over exactly-zero operand tiles
     const int *F = s_env, *E = s_env;
     const int ti = task.c_r / TILE, tj = task.c_c / TILE;

@@ -59,8 +59,9 @@ inline MatRef mref(double *p, long long ld, long long stride) { return MatRef{p,
 int chol_panel_tiles(int nt, int batch);
 bool chol_uses_lookahead(const Handle *h, int nt, int batch);
 int chol_lookahead_panel(const Handle *h, int nt);
-int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env = nullptr);
-int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, int batch);
+int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int batch, int *info_dev, const int *env = nullptr,
+                 const int *order = nullptr);
+int sinv_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, const int *env, const int *order, int batch);
 int trtri_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long stride, int batch);
 int extract_diag(Handle *h, int np, const double *L, long long stride, double *dvec, int batch);
 

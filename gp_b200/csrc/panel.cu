@@ -166,13 +166,14 @@ constexpr int TRSM_SMEM_BYTES = (TILE * LD_L + TILE) * (int)sizeof(double);
 template <int MODE>
 __global__ void __launch_bounds__(256, 1)
 trsm_tile_kernel(const double *Ldiag_base, double *Cbase, long long ld, long long stride, long long diag_off,
-                 long long diag_step, long long c_off, long long c_step) {
+                 long long diag_step, long long c_off, long long c_step, TrsmEnv env) {
   extern __shared__ __align__(16) double sm[];
   double *Ls = sm;                     // Ls[k*LD_L + n] = L[n][k]
   double *invd = sm + TILE * LD_L;     // 1 / L[n][n]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int item = blockIdx.y;
+  if (MODE == 0 && !env.live(item, blockIdx.x)) return;
   const double *Ld = Ldiag_base + (long long)item * stride + diag_off + (long long)blockIdx.x * diag_step;
   double *Ct = Cbase + (long long)item * stride + c_off + (long long)blockIdx.x * c_step;
 
@@ -290,7 +291,7 @@ constexpr int TRSM_PIPE_SMEM_BYTES = (LPK_DOUBLES + TILE + TILE * LD_CB) * (int)
 template <int MT>  // m8 row tiles per warp: 128 / (8 MT) warps per CTA
 __global__ void __launch_bounds__(32 * (16 / MT), 1)
 trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long ld, long long stride, long long diag_off,
-                            long long c_off, int ntiles, int tiles_per_cta) {
+                            long long c_off, int ntiles, int tiles_per_cta, TrsmEnv env) {
   extern __shared__ __align__(16) double sm[];
   double *Lp = sm;                      // packed: Lp[lpk_off(cb) + kk*lpk_ld(cb) + (n - 8cb)] = L[n][8cb + kk], n >= 8cb
   double *invd = sm + LPK_DOUBLES;      // 1 / L[n][n]
@@ -300,9 +301,15 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
   const int g = lane >> 2, t = lane & 3;
   const int item = blockIdx.y;
   const double *Ld = Ldiag_base + (long long)item * stride + diag_off;
-  const int t0 = blockIdx.x * tiles_per_cta;
-  const int t1 = min(ntiles, t0 + tiles_per_cta);
-  double *Ct = Cbase + (long long)item * stride + c_off + (long long)t0 * TILE;
+  const int t1 = min(ntiles, (int)blockIdx.x * tiles_per_cta + tiles_per_cta);
+  // only the live row tiles of this CTA's range are loaded, solved and stored; a CTA without one never stages L
+  auto next_live = [&](int ti) {
+    while (ti < t1 && !env.live(item, ti)) ti++;
+    return ti;
+  };
+  int ti = next_live(blockIdx.x * tiles_per_cta);
+  if (ti >= t1) return;
+  double *Cc = Cbase + (long long)item * stride + c_off;
 
   auto cp16 = [](double *dst, const double *src) {
     const unsigned d = (unsigned)__cvta_generic_to_shared(dst);
@@ -327,7 +334,7 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
     }
   }
   asm volatile("cp.async.commit_group;\n" ::: "memory");
-  prefetch_c(Ct);
+  prefetch_c(Cc + (long long)ti * TILE);
   asm volatile("cp.async.wait_group 0;\n" ::: "memory");
   __syncthreads();
   if (tid < TILE) invd[tid] = 1.0 / Lp[lpk_off(tid >> 3) + (tid & 7) * lpk_ld(tid >> 3) + (tid & 7)];
@@ -336,7 +343,7 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
   const unsigned FULL = 0xffffffffu;
   const int qbase = lane & ~3;
   const int r0 = warp * 8 * MT;
-  for (int ti = t0; ti < t1; ti++) {
+  while (ti < t1) {
     double acc[MT][16][2];
 #pragma unroll
     for (int mt = 0; mt < MT; mt++)
@@ -345,7 +352,8 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
 #pragma unroll
         for (int e = 0; e < 2; e++) acc[mt][nt][e] = Cb[(nt * 8 + 2 * t + e) * LD_CB + r0 + mt * 8 + g];
     __syncthreads();  // everybody has taken its rows out of the buffer
-    if (ti + 1 < t1) prefetch_c(Ct + TILE);  // next row tile, in flight during the arithmetic below
+    const int tn = next_live(ti + 1);
+    if (tn < t1) prefetch_c(Cc + (long long)tn * TILE);  // next live row tile, in flight during the arithmetic below
 
 #pragma unroll
     for (int cb = 0; cb < 16; cb++) {
@@ -394,6 +402,7 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
       }
     }
 
+    double *Ct = Cc + (long long)ti * TILE;
 #pragma unroll
     for (int mt = 0; mt < MT; mt++)
 #pragma unroll
@@ -402,7 +411,7 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
         Ct[r + (long long)c * ld] = acc[mt][nt][0];
         Ct[r + (long long)(c + 1) * ld] = acc[mt][nt][1];
       }
-    Ct += TILE;
+    ti = tn;
     asm volatile("cp.async.wait_group 0;\n" ::: "memory");
     __syncthreads();  // the next tile has landed for everybody
   }
@@ -1215,7 +1224,7 @@ int launch_potrf_tile(Handle *h, double *L, long long ld, long long stride, int 
 // X = C L^-T for `ntiles` consecutive 128-row tiles starting at element offset c_off (tile step = 128
 // rows), against the diagonal tile at element offset diag_off.
 int launch_trsm_tiles_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, long long c_off,
-                         int ntiles, int batch) {
+                         int ntiles, int batch, TrsmEnv env) {
   if (ntiles <= 0) return 0;
   const long long total = (long long)ntiles * batch;
   ProfScope ps__(h, PC_TRSM);
@@ -1234,13 +1243,16 @@ int launch_trsm_tiles_at(Handle *h, double *L, long long ld, long long stride, l
     // (an eight-warp, whole-tile form of the left-looking kernel was measured for this regime too: 611 us against 503 for
     // 128 x 31 tiles -- with the C tile in shared memory the DMMA operands cost two shared-memory loads each, where the
     // register-tile kernels feed A from registers; the round-1 kernels stay for batches)
-    const int tpc = total >= 148 * 16 ? 4 : (total >= 148 * 6 ? 2 : 1);
+    // With an envelope a block column has a few live row tiles per item (N = 4096, bench.py's draws: 176 of 496 per
+    // item), and two rows per CTA measured best there (B200, 1000 W, TRSM class per call: 7.52 ms with 2, 7.72 with
+    // 4 -- what the dense count picks -- 7.57 with 1).
+    const int tpc = env.F ? 2 : (total >= 148 * 16 ? 4 : (total >= 148 * 6 ? 2 : 1));
     if (tpc == 1 || h->trsm_pipelined == 0) {
       dim3 grid(ntiles, batch);
-      trsm_tile_kernel<0><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, 0, c_off, TILE);
+      trsm_tile_kernel<0><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, 0, c_off, TILE, env);
     } else {
       dim3 grid((ntiles + tpc - 1) / tpc, batch);
-      trsm_tiles_pipelined_kernel<2><<<grid, 256, TRSM_PIPE_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off, ntiles, tpc);
+      trsm_tiles_pipelined_kernel<2><<<grid, 256, TRSM_PIPE_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off, ntiles, tpc, env);
     }
   }
   GPB_LAUNCH_CHECK(h);
@@ -1253,7 +1265,7 @@ int launch_trsm_tiles(Handle *h, double *L, long long ld, long long stride, int 
 }
 
 int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base, int n,
-                         long long c_off, int ntiles, int batch, int *info) {
+                         long long c_off, int ntiles, int batch, int *info, TrsmEnv env) {
   // one launch when the diagonal CTAs and the 64-row (or 32-row) TRSM CTAs of all matrices fit one wave at one CTA per SM
   int mt = 0;
   if (h->panel_fused && h->panel_impl == 0 && ntiles > 0 && batch <= PANEL_FUSED_MAX_BATCH) {
@@ -1271,7 +1283,7 @@ int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, l
   if (mt == 0) {
     int rc = launch_potrf_tile_at(h, L, ld, stride, diag_off, index_base, n, batch, info);
     if (rc) return rc;
-    return launch_trsm_tiles_at(h, L, ld, stride, diag_off, c_off, ntiles, batch);
+    return launch_trsm_tiles_at(h, L, ld, stride, diag_off, c_off, ntiles, batch, env);
   }
   ProfScope ps__(h, PC_POTRF);
   const int chunks = ntiles * (4 / mt);
@@ -1287,9 +1299,11 @@ int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, l
 }
 
 int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int tile_col, int ntiles_below, int n, int batch,
-                      int *info) {
+                      int *info, const int *env) {
+  TrsmEnv te;
+  if (env) te = TrsmEnv{env + tile_col + 1, 2 * (int)(ld / TILE), tile_col};
   return launch_potrf_trsm_at(h, L, ld, stride, (long long)tile_col * TILE * (ld + 1), tile_col * TILE, n,
-                              (long long)(tile_col + 1) * TILE + (long long)tile_col * TILE * ld, ntiles_below, batch, info);
+                              (long long)(tile_col + 1) * TILE + (long long)tile_col * TILE * ld, ntiles_below, batch, info, te);
 }
 
 // inverse of `ntiles` diagonal tiles: L tiles at l_off + t*l_step, W tiles at w_off + t*w_step
@@ -1297,7 +1311,7 @@ int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l
                            long long w_off, long long w_step, long long stride, int ntiles, int batch) {
   dim3 grid(ntiles, batch);
   ProfScope ps__(h, PC_TRSM);
-  if (h->panel_impl == 1) trsm_tile_kernel<1><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step);
+  if (h->panel_impl == 1) trsm_tile_kernel<1><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step, TrsmEnv{});
   else tile_inverse_ll_kernel<<<grid, 256, TINV_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step);
   GPB_LAUNCH_CHECK(h);
   return 0;

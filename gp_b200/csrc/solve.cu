@@ -539,9 +539,11 @@ int launch_trsv_sweep(Handle *h, int np, const double *L, const double *Wdiag, l
 // env per item: F[0..nt) (first nonzero tile column of each tile row, filled by gram_se_batched; F_I <= I) and
 // E[0..nt): E_J = the last tile row I with F_I <= J.  F need not be monotone (x unsorted).  For K > J, E_K >= E_J,
 // which is what closes the selected-inverse recurrence over the contiguous range J+1..E_J.
-__global__ void __launch_bounds__(256) envelope_profile_kernel(int nt, int *__restrict__ env) {
+__global__ void __launch_bounds__(256) envelope_profile_kernel(int nt, int *__restrict__ env, int *__restrict__ band) {
   extern __shared__ int sF[];
+  __shared__ int s_band;
   int *F = env + (long long)blockIdx.x * 2 * nt, *E = F + nt;
+  if (threadIdx.x == 0) s_band = 0;
   for (int i = threadIdx.x; i < nt; i += blockDim.x) sF[i] = min(F[i], i);
   __syncthreads();
   for (int j = threadIdx.x; j < nt; j += blockDim.x) {
@@ -550,12 +552,48 @@ __global__ void __launch_bounds__(256) envelope_profile_kernel(int nt, int *__re
       if (sF[i] <= j) { e = i; break; }
     F[j] = sF[j];
     E[j] = e;
+    atomicMax(&s_band, j - sF[j]);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) band[blockIdx.x] = s_band;
+}
+
+// Dispatch order of the envelope GEMM launches: the items by descending bandwidth max_I (I - F_I), ties in item order.
+// A CTA's contraction length grows with its item's bandwidth, so the widest items go first and the narrow ones fill
+// the last wave.  One warp, a stable counting sort over the nt <= ENV_MAX_NT possible keys.
+__global__ void __launch_bounds__(32) envelope_order_kernel(int nt, int batch, const int *__restrict__ band,
+                                                            int *__restrict__ order) {
+  __shared__ int base[ENV_MAX_NT];
+  const int lane = threadIdx.x;
+  for (int k = lane; k < nt; k += 32) base[k] = 0;
+  __syncwarp();
+  for (int b = lane; b < batch; b += 32) atomicAdd(&base[band[b]], 1);
+  __syncwarp();
+  if (lane == 0)
+    for (int k = nt - 1, s = 0; k >= 0; k--) {
+      const int c = base[k];
+      base[k] = s;
+      s += c;
+    }
+  __syncwarp();
+  for (int b0 = 0; b0 < batch; b0 += 32) {
+    const int b = b0 + lane;
+    const int k = b < batch ? band[b] : -1 - lane;  // lanes past the batch: keys of their own
+    const unsigned peers = __match_any_sync(0xffffffffu, k);
+    const int rank = __popc(peers & ((1u << lane) - 1u));
+    if (b < batch) order[base[k] + rank] = b;
+    __syncwarp();
+    if (b < batch && rank == 0) base[k] += __popc(peers);
+    __syncwarp();
   }
 }
 
-int launch_envelope_profile(Handle *h, int nt, int *env, int batch) {
+int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch) {
   ProfScope ps__(h, PC_OTHER);
-  envelope_profile_kernel<<<batch, 256, nt * sizeof(int), h->stream>>>(nt, env);
+  int *band = order + batch;
+  envelope_profile_kernel<<<batch, 256, nt * sizeof(int), h->stream>>>(nt, env, band);
+  GPB_LAUNCH_CHECK(h);
+  envelope_order_kernel<<<1, 32, 0, h->stream>>>(nt, batch, band, order);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

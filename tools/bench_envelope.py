@@ -2,11 +2,17 @@
 
   python tools/bench_envelope.py --ref DIR [--runs 3] [--steps 10] [--warmup 3] [--out DIR]
   python tools/bench_envelope.py --sweep [--rounds 3]
+  python tools/bench_envelope.py --breakdown [--steps 10] [--warmup 3]
 
 Runs `bench.py --gpus 1` of this tree and of the tree at DIR (built the same way) in turn, `--runs` times each, and
 prints per run the headline evals/s, the LML-only `cholesky` ms, executed_tflops and the latency block; the last run
 of each dumps its outputs, and the maximum relative difference of lml and grad between the two is printed with the
-card name and power limit."""
+card name and power limit.
+
+`--breakdown` runs the bench.py workload of this tree (N = 4096, B = 256, bench.synth_inputs(0), device pointers) with
+the handle's per-class kernel timing on, once with the gradient and once LML-only, and prints per kernel class (gemm,
+potrf_tile, trsm_tile, gram, solve, other) the ms per call of each pass.  The GEMM time of the LML-only pass is that of
+the Cholesky; the difference to the other pass is the selected inverse's."""
 import argparse
 import json
 import os
@@ -89,10 +95,48 @@ def sweep(args):
         print(json.dumps({"shape": k, "ms_per_call": v}), flush=True)
 
 
+def breakdown(args):
+    import torch
+    sys.path.insert(0, HERE)
+    import bench
+    from gp_b200 import capi
+    dev = torch.device("cuda", 0)
+    stream = torch.cuda.current_stream(dev)
+    h = capi.Handle(0)
+    h.set_stream(stream.cuda_stream)
+    h.set_pointer_mode(True)
+    n, B = bench.N, bench.DRAWS_PER_GPU
+    dx, dy, dth = (torch.from_numpy(a).to(dev) for a in bench.synth_inputs(0))
+    lml = torch.empty(B, dtype=torch.float64, device=dev)
+    grad = torch.empty(B, 3, dtype=torch.float64, device=dev)
+    info = torch.zeros(B, dtype=torch.int32, device=dev)
+    for want_grad in (True, False):
+        def call():
+            h.lml_grad_batched_device(n, B, dx, 0, dy, 0, dth, 0.0, want_grad, lml, grad, info)
+        for _ in range(args.warmup):
+            call()
+        torch.cuda.synchronize(dev)
+        h.set_profiling(True)
+        e0 = torch.cuda.Event(enable_timing=True); e1 = torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(args.steps):
+            call()
+        e1.record(stream)
+        torch.cuda.synchronize(dev)
+        prof = h.get_profile()
+        h.set_profiling(False)
+        print(json.dumps({"pass": "lml+grad" if want_grad else "lml", "n": n, "B": B,
+                          "ms_per_call": round(e0.elapsed_time(e1) / args.steps, 3),
+                          "class_ms_per_call": {k: round(v[0] / args.steps, 3) for k, v in prof.items()},
+                          "class_launches_per_call": {k: v[1] // args.steps for k, v in prof.items()}}), flush=True)
+    h.close()
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--ref")
     ap.add_argument("--sweep", action="store_true")
+    ap.add_argument("--breakdown", action="store_true")
     ap.add_argument("--rounds", type=int, default=3)
     ap.add_argument("--runs", type=int, default=3)
     ap.add_argument("--steps", type=int, default=10)
@@ -104,8 +148,10 @@ def main():
     print(json.dumps({"gpu": smi}), flush=True)
     if args.sweep:
         return sweep(args)
+    if args.breakdown:
+        return breakdown(args)
     if not args.ref:
-        ap.error("--ref DIR or --sweep")
+        ap.error("--ref DIR, --sweep or --breakdown")
     if args.out is None:
         args.out = tempfile.mkdtemp(prefix="bench_envelope_")
     args.out = os.path.abspath(args.out)
