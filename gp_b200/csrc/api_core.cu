@@ -77,12 +77,8 @@ extern "C" int gpb200_create(gpb200_handle_t *out, int device) {
   if (gc && gc[0] >= '0' && gc[0] <= '3') h->gemm_cfg_override = gc[0] - '0';
   const char *tp = getenv("GPB200_TRSM_PIPELINED");
   if (tp && tp[0] == '0') h->trsm_pipelined = 0;
-  const char *pv = getenv("GPB200_PANEL_V1");
-  if (pv && pv[0] == '1') h->panel_impl = 1;
   const char *ds = getenv("GPB200_DIAG_SPLIT");
   if (ds && ds[0] == '0') h->diag_split = 0;
-  const char *tm = getenv("GPB200_TRSM_MT");
-  if (tm && (tm[0] == '1' || tm[0] == '2')) h->trsm_mt_override = tm[0] - '0';
   const char *fc = getenv("GPB200_FINE_CFG");
   if (fc && fc[0] == '0') h->fine_cfg = 0;
   const char *pf = getenv("GPB200_PANEL_FUSED");

@@ -173,7 +173,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       memcpy(&jbits, &jitter, sizeof(jbits));
       const std::vector<long long> key = {n, B, want_grad, xs, ys, jbits, (long long)(uintptr_t)h->ws, h->chol_panel_override,
                                           sp.deriv, sp.order0, sp.nblocks, h->gemm_cfg_override, h->lookahead, h->lookahead_max_batch,
-                                          h->panel_impl, h->trsm_mt_override, h->quarter_below_waves, h->trsm_pipelined, h->panel_fused, h->fine_cfg,
+                                          h->quarter_below_waves, h->trsm_pipelined, h->panel_fused, h->fine_cfg,
                                           h->envelope, h->sinv_min_batch, sp.ard_d};
       auto it = h->graphs.find(key);
       if (it == h->graphs.end()) {

@@ -97,8 +97,6 @@ struct Handle {
   int gemm_cfg_override = 0;  // 0 automatic, 1 one 128x128 CTA per SM, 2 two 128x64 half-tile CTAs per SM, 3 64x64 quarter-tile CTAs
   int quarter_below_waves = 2;  // automatic choice: quarter tiles while the half-tile grid is below this many waves of 2 x 148 CTAs
   int trsm_pipelined = 1;     // 0: one tile per CTA (the first TRSM tile kernel); env GPB200_TRSM_PIPELINED
-  int panel_impl = 0;         // 0: round-2 shared-memory panel kernels (POTRF with a panel warp); 1: the round-1 register-tile kernels; 2: round-2 POTRF without the panel warp (env GPB200_PANEL_V1 = 1 | 2)
-  int trsm_mt_override = 0;   // tuning knob: 8-row mma tiles per warp of trsm_ll_kernel (1, 2, 4); env GPB200_TRSM_MT
   int fine_cfg = 1;           // 64x64 CTAs of sixteen 16x16 warps for small chain launches (env GPB200_FINE_CFG)
   int panel_fused = 1;        // POTRF tile and the TRSM below it in one launch when one wave holds both (panel_fused_kernel); env GPB200_PANEL_FUSED
   int *panel_flags = nullptr; // 2 ints per matrix for panel_fused_kernel (visible column blocks, finished TRSM CTAs), zero between launches

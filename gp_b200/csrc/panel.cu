@@ -2,12 +2,16 @@
 // between the DMMA GEMM launches.  They replace the unblocked inner part of Eigen's LLT that runs
 // under Stan Math's cholesky_decompose (models/fit_hyperparameters.stan:25, covariance.cpp:29).
 //
-//   potrf_tile_kernel   in-register right-looking Cholesky of one 128x128 diagonal tile per CTA
-//                       (2-D cyclic ownership, one barrier per column, pivot check -> info)
-//   trsm_tile_kernel    X = C L^-T for a 128x128 tile below the diagonal: true substitution on 8x8
-//                       diagonal blocks with quad shuffles, DMMA (mma.sync m8n8k4 f64) for the
-//                       rank-8 updates.  The same kernel with C = I and a transposed store
-//                       produces the inverse of a diagonal tile (seed of the recursive TRTRI).
+//   trsm_tile_kernel             X = C L^-T for a 128x128 tile below the diagonal, tile in registers: true
+//                                substitution on 8x8 diagonal blocks with quad shuffles, DMMA (mma.sync m8n8k4
+//                                f64) for the rank-8 updates (batches)
+//   trsm_tiles_pipelined_kernel  the same for several row tiles per CTA, next C tile prefetched (large batches)
+//   potrf_tile_pw_kernel         left-looking Cholesky of one 128x128 diagonal tile per CTA in shared memory,
+//                                a panel warp carrying the chain of 8x8 diagonal blocks (pivot check -> info)
+//   trsm_ll_kernel<MT>           left-looking X = C L^-T, 32 MT rows per CTA (one or a few matrices)
+//   tile_inverse_ll_kernel       L^-1 of a diagonal tile (seed of the recursive TRTRI)
+//   panel_fused_kernel,          POTRF of the diagonal tile and the TRSM below it in one launch
+//   panel_fused_tile_kernel
 #include "common.cuh"
 #include "panel_ll.cuh"
 
@@ -20,162 +24,25 @@ __device__ __forceinline__ void dmma884p(double (&c)[2], double a, double b) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// POTRF of one 128x128 tile, blocked (v2): right-looking over sixteen 8-column blocks with the tile
-// register-resident in mma accumulator layout (warp w owns rows 16w..16w+15, like the TRSM kernel):
-//   1. the warp that owns the 8x8 diagonal block factors it with warp shuffles (8 dependent steps)
-//   2. every warp solves its rows of the 8-column panel against that block (quad shuffles)
-//   3. rank-8 SYRK update of the trailing lower triangle with DMMA (mma.sync m8n8k4 f64); the panel
-//      goes through shared memory once per block (B operand), the A operand comes from registers
-// Two block barriers per 8 columns instead of one per column, and the O(n^3) part on the tensor pipe.
-// ------------------------------------------------------------------------------------------------
-constexpr int LD_P = 12;  // panel row stride in doubles: conflict-free B-operand reads ((12g + t) mod 16 distinct)
-
-__global__ void __launch_bounds__(256, 1)
-potrf_tile_kernel_v2(double *__restrict__ Lbase, long long ld, long long stride, long long diag_off, int index_base,
-                     int n, int *info) {
-  __shared__ __align__(16) double Dsm[2][64];         // Dsm[c*8 + r] = D[r][c] (factored diagonal block)
-  __shared__ double dinv[2][8];
-  __shared__ __align__(16) double Psm[2][TILE * LD_P];  // solved panel rows: Psm[row*LD_P + c]
-  __shared__ int s_info;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int g = lane >> 2, t = lane & 3;
-  const unsigned FULL = 0xffffffffu;
-  const int qbase = lane & ~3;
-  double *T = Lbase + (long long)blockIdx.x * stride + diag_off;
-  const int r0 = warp * 16;
-  if (tid == 0) s_info = 0;
-
-  double acc[2][16][2];
-#pragma unroll
-  for (int mt = 0; mt < 2; mt++)
-#pragma unroll
-    for (int nt = 0; nt < 16; nt++)
-#pragma unroll
-      for (int e = 0; e < 2; e++) {
-        const int r = r0 + mt * 8 + g, c = nt * 8 + 2 * t + e;
-        acc[mt][nt][e] = (nt <= 2 * warp + mt) ? T[r + (long long)c * ld] : 0.0;  // tiles right of the diagonal are never used
-      }
-  __syncthreads();
-
-#pragma unroll
-  for (int cb = 0; cb < 16; cb++) {
-    const int buf = cb & 1;
-    // ---- 1. diagonal 8x8 block: rows 8cb..8cb+7 live in warp cb/2, m-tile cb%2 ------------------
-    if (warp == (cb >> 1)) {
-#pragma unroll
-      for (int mo = 0; mo < 2; mo++) {
-        if (mo == (cb & 1)) {
-          double a0 = acc[mo][cb][0], a1 = acc[mo][cb][1];  // element (row g, cols 2t, 2t+1)
-#pragma unroll
-          for (int k = 0; k < 8; k++) {
-            const double ak = (k & 1) ? a1 : a0;               // this lane's element in column k (valid if t == k/2)
-            const double piv = __shfl_sync(FULL, ak, 4 * k + (k >> 1));
-            if (!(piv > 0.0) && lane == 0 && s_info == 0) s_info = index_base + cb * 8 + k + 1;
-            const double inv = rsqrt(piv), dgl = piv * inv;  // shortest dependent chain on the critical path
-            const double lrow = __shfl_sync(FULL, ak, 4 * g + (k >> 1)) * inv;            // l[g][k]
-            const double lc0 = __shfl_sync(FULL, ak, 4 * (2 * t) + (k >> 1)) * inv;       // l[2t][k]
-            const double lc1 = __shfl_sync(FULL, ak, 4 * (2 * t + 1) + (k >> 1)) * inv;   // l[2t+1][k]
-            if (2 * t > k && g >= 2 * t) a0 = fma(-lrow, lc0, a0);
-            if (2 * t + 1 > k && g >= 2 * t + 1) a1 = fma(-lrow, lc1, a1);
-            if (t == (k >> 1)) {  // write the finished column k
-              const double v = (g > k) ? lrow : ((g == k) ? dgl : 0.0);
-              if (k & 1) a1 = v; else a0 = v;
-            }
-          }
-          // strict upper part of the block -> exact zeros
-          if (2 * t > g) a0 = 0.0;
-          if (2 * t + 1 > g) a1 = 0.0;
-          acc[mo][cb][0] = a0;
-          acc[mo][cb][1] = a1;
-          Dsm[buf][(2 * t) * 8 + g] = a0;
-          Dsm[buf][(2 * t + 1) * 8 + g] = a1;
-          if (g == 2 * t) dinv[buf][g] = 1.0 / a0;
-          if (g == 2 * t + 1) dinv[buf][g] = 1.0 / a1;
-        }
-      }
-    }
-    __syncthreads();
-    // ---- 2. panel solve for the m-tiles strictly below the diagonal block ------------------------
-    double af[2][2];
-#pragma unroll
-    for (int mt = 0; mt < 2; mt++) {
-      const bool below = (2 * warp + mt) > cb;  // warp-uniform
-      if (below) {
-#pragma unroll
-        for (int c = 0; c < 8; c++) {
-          double xv = acc[mt][cb][c & 1] * dinv[buf][c];
-          if (t == (c >> 1)) acc[mt][cb][c & 1] = xv;
-          xv = __shfl_sync(FULL, xv, qbase + (c >> 1));
-#pragma unroll
-          for (int e = 0; e < 2; e++) {
-            const int cp = 2 * t + e;
-            if (cp > c) acc[mt][cb][e] = fma(-xv, Dsm[buf][c * 8 + cp], acc[mt][cb][e]);
-          }
-        }
-        *reinterpret_cast<double2 *>(&Psm[buf][(r0 + mt * 8 + g) * LD_P + 2 * t]) =
-            make_double2(acc[mt][cb][0], acc[mt][cb][1]);
-      }
-#pragma unroll
-      for (int ks = 0; ks < 2; ks++) {
-        const int src = qbase + 2 * ks + (t >> 1);
-        const double v0 = __shfl_sync(FULL, acc[mt][cb][0], src);
-        const double v1 = __shfl_sync(FULL, acc[mt][cb][1], src);
-        af[mt][ks] = (t & 1) ? v1 : v0;
-      }
-    }
-    __syncthreads();
-    // ---- 3. trailing update, lower triangle only: C[i][j] -= X[i] . X[j], 8cb+7 < j <= i ---------
-#pragma unroll
-    for (int nt = 0; nt < 16; nt++) {
-      if (nt > cb && nt <= 2 * warp + 1) {
-#pragma unroll
-        for (int ks = 0; ks < 2; ks++) {
-          const double bfv = -Psm[buf][(nt * 8 + g) * LD_P + ks * 4 + t];
-          if (nt <= 2 * warp) dmma884p(acc[0][nt], af[0][ks], bfv);
-          dmma884p(acc[1][nt], af[1][ks], bfv);
-        }
-      }
-    }
-  }
-
-  // write back: lower triangle = L, strict upper = 0 (Eigen matrixL() convention)
-#pragma unroll
-  for (int mt = 0; mt < 2; mt++)
-#pragma unroll
-    for (int nt = 0; nt < 16; nt++)
-#pragma unroll
-      for (int e = 0; e < 2; e++) {
-        const int r = r0 + mt * 8 + g, c = nt * 8 + 2 * t + e;
-        T[r + (long long)c * ld] = (r >= c) ? acc[mt][nt][e] : 0.0;
-      }
-  __syncthreads();
-  if (tid == 0 && s_info != 0 && s_info <= n) {
-    if (info[blockIdx.x] == 0) info[blockIdx.x] = s_info;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // TRSM tile: X L^T = C with L the 128x128 lower-triangular diagonal tile, C a 128x128 tile.
 // 8 warps; warp w owns rows 16w..16w+15 as two m8 mma row tiles x sixteen n8 column tiles.
-// MODE 0: C read from / X written to the tile (in place).  MODE 1: C = I, X^T written to Wout
-// (Wout = L^-1, lower triangular, strict upper zero).
+// C is read from and X written to the tile (in place); blockIdx.x = row tile, blockIdx.y = batch item.
 // ------------------------------------------------------------------------------------------------
 constexpr int LD_L = TILE + 4;
 constexpr int TRSM_SMEM_BYTES = (TILE * LD_L + TILE) * (int)sizeof(double);
 
-template <int MODE>
 __global__ void __launch_bounds__(256, 1)
 trsm_tile_kernel(const double *Ldiag_base, double *Cbase, long long ld, long long stride, long long diag_off,
-                 long long diag_step, long long c_off, long long c_step, TrsmEnv env) {
+                 long long c_off, TrsmEnv env) {
   extern __shared__ __align__(16) double sm[];
   double *Ls = sm;                     // Ls[k*LD_L + n] = L[n][k]
   double *invd = sm + TILE * LD_L;     // 1 / L[n][n]
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int g = lane >> 2, t = lane & 3;
   const int item = blockIdx.y;
-  if (MODE == 0 && !env.live(item, blockIdx.x)) return;
-  const double *Ld = Ldiag_base + (long long)item * stride + diag_off + (long long)blockIdx.x * diag_step;
-  double *Ct = Cbase + (long long)item * stride + c_off + (long long)blockIdx.x * c_step;
+  if (!env.live(item, blockIdx.x)) return;
+  const double *Ld = Ldiag_base + (long long)item * stride + diag_off;
+  double *Ct = Cbase + (long long)item * stride + c_off + (long long)blockIdx.x * TILE;
 
   // stage the diagonal tile with cp.async (column-major copy, 16B vectors): all 32 copies of a thread are
   // in flight at once, together with the C-tile loads below (both tiles are 128 KB and this kernel runs
@@ -197,7 +64,7 @@ trsm_tile_kernel(const double *Ldiag_base, double *Cbase, long long ld, long lon
 #pragma unroll
       for (int e = 0; e < 2; e++) {
         const int r = r0 + mt * 8 + g, c = nt * 8 + 2 * t + e;
-        acc[mt][nt][e] = (MODE == 0) ? Ct[r + (long long)c * ld] : ((r == c) ? 1.0 : 0.0);
+        acc[mt][nt][e] = Ct[r + (long long)c * ld];
       }
 
   asm volatile("cp.async.wait_group 0;\n" ::: "memory");
@@ -258,26 +125,19 @@ trsm_tile_kernel(const double *Ldiag_base, double *Cbase, long long ld, long lon
 #pragma unroll
     for (int nt = 0; nt < 16; nt++) {
       const int r = r0 + mt * 8 + g, c = nt * 8 + 2 * t;
-      if (MODE == 0) {
-        Ct[r + (long long)c * ld] = acc[mt][nt][0];
-        Ct[r + (long long)(c + 1) * ld] = acc[mt][nt][1];
-      } else {
-        // W[c][r] = X[r][c]; X = L^-T is upper triangular (r <= c); emit exact zeros elsewhere
-        const double v0 = (r <= c) ? acc[mt][nt][0] : 0.0;
-        const double v1 = (r <= c + 1) ? acc[mt][nt][1] : 0.0;
-        *reinterpret_cast<double2 *>(Ct + c + (long long)r * ld) = make_double2(v0, v1);
-      }
+      Ct[r + (long long)c * ld] = acc[mt][nt][0];
+      Ct[r + (long long)(c + 1) * ld] = acc[mt][nt][1];
     }
 }
 
 // ------------------------------------------------------------------------------------------------
-// Pipelined TRSM over several row tiles of one block column (MODE 0 semantics).  Timing the kernel above
+// Pipelined TRSM over several row tiles of one block column.  Timing the kernel above
 // with its arithmetic removed showed 7.5 of its 18.1 ms per N=4096 step are exposed global-memory time
 // (one CTA per SM: load 256 KB, compute, store 128 KB, nothing overlaps).  Here one CTA keeps the diagonal
 // tile in shared memory for up to `tiles_per_cta` row tiles -- packed (only the lower triangle, in groups of
 // 8 columns: 72 KB instead of 135 KB) so that a full 128x128 prefetch buffer fits next to it -- and the
 // cp.async prefetch of the next C tile runs under the substitution + DMMA work of the current one.
-// The arithmetic per element is that of trsm_tile_kernel<0>.  What is left (14.4 of 17.3 ms with loads and stores
+// The arithmetic per element is that of trsm_tile_kernel.  What is left (14.4 of 17.3 ms with loads and stores
 // removed) is the substitution chain itself: its DMUL/DFMA steps queue behind the other warps' DMMAs on the one
 // FP64 pipe (ncu: 44.6 % DMMA-active, DFMA stalls 70 % short-scoreboard + 23 % math-pipe); 16 warps of 8 rows
 // instead of 8 warps of 16 rows measured the same.
@@ -420,9 +280,9 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
 // ------------------------------------------------------------------------------------------------
 // Round-2 panel kernels: left-looking over 8-column blocks with the tile resident in SHARED memory.
 //
-// The round-1 kernels keep the 128x128 tile in registers in mma accumulator layout, which forces the sixteen block
-// steps to be fully unrolled (register arrays need static indices): potrf_tile_kernel_v2 is 28 000 SASS instructions,
-// each executed once -- it runs at instruction-fetch speed (46 us per tile).  With the tile in shared memory every
+// A 128x128 tile kept in registers in mma accumulator layout forces the sixteen block steps to be fully unrolled
+// (register arrays need static indices): a register-resident POTRF in that form is 28 000 SASS instructions, each
+// executed once -- it runs at instruction-fetch speed (46 us per tile).  With the tile in shared memory every
 // index is dynamic, the block loop stays rolled, and the left-looking order needs no register-resident trailing matrix:
 //
 //   for cb = 0..15:   P  = T[:, 8cb:8cb+8] - T[:, 0:8cb] * T[8cb:8cb+8, 0:8cb]^T     DMMA, own rows
@@ -436,7 +296,7 @@ trsm_tiles_pipelined_kernel(const double *Ldiag_base, double *Cbase, long long l
 // trsm_ll_kernel        the rows of X = C L^-T are independent: each warp runs its rows through all sixteen steps with
 //                       no block barrier; a CTA takes 32 or 64 rows so that ONE matrix spreads a block column over the GPU
 // tile_inverse_ll_kernel  X = L^-T row block by row block into the unused upper triangle of the staged tile
-// panel_fused_kernel<MT>, panel_fused_tile_kernel   POTRF and TRSM of a block column in ONE launch: the TRSM CTAs follow
+// panel_fused_kernel, panel_fused_tile_kernel   POTRF and TRSM of a block column in ONE launch: the TRSM CTAs follow
 //                       the diagonal CTA's factorisation block by block through flags in global memory (64-row CTAs with
 //                       the staged L resident, or 128-row CTAs with a double-buffered row block of L)
 // Per-phase cycle counts (tools/panel_trace.py, instrumented build) are in profiles/panel_trace_r02.txt.
@@ -661,7 +521,7 @@ potrf_tile_pw_kernel(double *__restrict__ Lbase, long long ld, long long stride,
   potrf_pw_body<false>(sm, Lbase + (long long)blockIdx.x * stride + diag_off, ld, index_base, n, info + blockIdx.x, nullptr);
 }
 
-// X L^T = C for ROWS = 32 MT consecutive rows of a block column (MODE-0 semantics of trsm_tile_kernel), four warps
+// X L^T = C for ROWS = 32 MT consecutive rows of a block column (in place, like trsm_tile_kernel), four warps
 // of 8 MT rows each, no block barrier in the main loop.  blockIdx.x = row chunk, blockIdx.y = batch item.
 // The diagonal tile sits in shared memory as a full square (constant strides: every fragment address is one base
 // register plus an immediate), its sixteen 8x8 diagonal blocks once more row-major (Dall) for the substitution.
@@ -843,18 +703,13 @@ trsm_ll_kernel(const double *Ldiag_base, double *Cbase, long long ld, long long 
 
 // POTRF of the diagonal tile and the TRSM of the tiles below it in ONE launch (the latency path: one or a few matrices).
 // CTAs [0, batch) factor the diagonal tiles and publish them column block by column block; CTAs [batch, ...) take
-// 32 MT rows each of the block column below and trail the factorisation by about one 8-column block instead of
+// 64 rows each of the block column below and trail the factorisation by about one 8-column block instead of
 // starting when it has finished (16.5 us later and a launch gap).  The diagonal CTAs wait for nobody and have the
 // lowest block indices, so every waiting CTA waits for a CTA that is already resident.  flags[2 m] counts matrix m's
 // visible column blocks, flags[2 m + 1] its finished TRSM CTAs; the last one to finish clears both for the next launch.
-template <int MT>
-struct PanelFused {
-  static constexpr int SMEM_BYTES = TrsmLL<MT>::SMEM_BYTES > POTRF_PW_SMEM_BYTES ? TrsmLL<MT>::SMEM_BYTES : POTRF_PW_SMEM_BYTES;
-};
-
+constexpr int PANEL_FUSED_SMEM_BYTES = TrsmLL<2>::SMEM_BYTES > POTRF_PW_SMEM_BYTES ? TrsmLL<2>::SMEM_BYTES : POTRF_PW_SMEM_BYTES;
 constexpr int PANEL_FUSED_THREADS = POTRF_PW_THREADS + 32;
 
-template <int MT>
 __global__ void __launch_bounds__(PANEL_FUSED_THREADS, 1)
 panel_fused_kernel(double *__restrict__ Lbase, long long ld, long long stride, long long diag_off, long long c_off,
                    int chunks, int batch, int index_base, int n, int *info, int *flags) {
@@ -882,7 +737,7 @@ panel_fused_kernel(double *__restrict__ Lbase, long long ld, long long stride, l
     trsm_follow_loader(sm, base + diag_off, ld, flags + 2 * m, s_ready);
     return;
   }
-  trsm_ll_body<MT, true>(sm, base + diag_off, base + c_off + (long long)chunk * TrsmLL<MT>::ROWS, ld, s_ready);
+  trsm_ll_body<2, true>(sm, base + diag_off, base + c_off + (long long)chunk * TrsmLL<2>::ROWS, ld, s_ready);
   if (threadIdx.x == 0) {
     if (atomicAdd(flags + 2 * m + 1, 1) == chunks - 1) {
       flags[2 * m + 1] = 0;
@@ -1091,8 +946,7 @@ panel_fused_tile_kernel(double *__restrict__ Lbase, long long ld, long long stri
   }
 }
 
-// W = L^-1 of one 128x128 lower-triangular tile per CTA (MODE-1 semantics of trsm_tile_kernel: W lower triangular,
-// strict upper zero; in place allowed).  X = L^-T is computed row block by row block -- its rows are independent, so
+// W = L^-1 of one 128x128 lower-triangular tile per CTA (W lower triangular, strict upper zero; in place allowed).  X = L^-T is computed row block by row block -- its rows are independent, so
 // the eight warps never meet at a barrier -- left-looking over the column blocks at and right of the row block
 // (everything left of it is zero and is skipped).  X is upper triangular and lives in the UNUSED upper triangle of
 // the staged L tile; its 8x8 diagonal blocks, which would collide with L's, go to a side buffer.  Warp w takes row
@@ -1194,14 +1048,12 @@ int panel_trace_fetch(long long *out2048) {
 
 int panel_smem_setup(Handle *h) {
   GPB_CUDA(h, cudaFuncSetAttribute(trsm_tiles_pipelined_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_PIPE_SMEM_BYTES));
-  GPB_CUDA(h, cudaFuncSetAttribute(trsm_tile_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_SMEM_BYTES));
-  GPB_CUDA(h, cudaFuncSetAttribute(trsm_tile_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_SMEM_BYTES));
+  GPB_CUDA(h, cudaFuncSetAttribute(trsm_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TRSM_SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(tile_inverse_ll_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, TINV_SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(potrf_tile_pw_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, POTRF_PW_SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(trsm_ll_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrsmLL<1>::SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(trsm_ll_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrsmLL<2>::SMEM_BYTES));
-  GPB_CUDA(h, cudaFuncSetAttribute(panel_fused_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PanelFused<1>::SMEM_BYTES));
-  GPB_CUDA(h, cudaFuncSetAttribute(panel_fused_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PanelFused<2>::SMEM_BYTES));
+  GPB_CUDA(h, cudaFuncSetAttribute(panel_fused_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PANEL_FUSED_SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(panel_fused_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PANEL_FUSED_TILE_SMEM_BYTES));
   return 0;
 }
@@ -1209,10 +1061,7 @@ int panel_smem_setup(Handle *h) {
 int launch_potrf_tile_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base,
                          int n, int batch, int *info) {
   ProfScope ps__(h, PC_POTRF);
-  if (h->panel_impl == 1)
-    potrf_tile_kernel_v2<<<batch, 256, 0, h->stream>>>(L, ld, stride, diag_off, index_base, n, info);
-  else
-    potrf_tile_pw_kernel<<<batch, POTRF_PW_THREADS, POTRF_PW_SMEM_BYTES, h->stream>>>(L, ld, stride, diag_off, index_base, n, info);
+  potrf_tile_pw_kernel<<<batch, POTRF_PW_THREADS, POTRF_PW_SMEM_BYTES, h->stream>>>(L, ld, stride, diag_off, index_base, n, info);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }
@@ -1229,27 +1078,25 @@ int launch_trsm_tiles_at(Handle *h, double *L, long long ld, long long stride, l
   const long long total = (long long)ntiles * batch;
   ProfScope ps__(h, PC_TRSM);
   // Few tiles (one large matrix, batch 1..2: the latency path): the row-split left-looking kernel, 32 or 64 rows per
-  // CTA, so that one block column covers the GPU in a single wave.  Otherwise the DMMA-throughput kernels of round 1:
-  // one tile per CTA, or several row tiles per CTA pipelined when there are many.
-  int mt = h->trsm_mt_override;
-  if (mt != 1 && mt != 2) mt = (h->panel_impl == 1) ? 0 : (total * 4 <= 148 ? 1 : (total * 2 <= 148 ? 2 : 0));
-  if (mt == 1) {
+  // CTA, so that one block column covers the GPU in a single wave.  Otherwise the register-tile DMMA-throughput
+  // kernels: one tile per CTA, or several row tiles per CTA pipelined when there are many.
+  if (total * 4 <= 148) {
     dim3 grid(ntiles * 4, batch);
     trsm_ll_kernel<1><<<grid, 128, TrsmLL<1>::SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off);
-  } else if (mt == 2) {
+  } else if (total * 2 <= 148) {
     dim3 grid(ntiles * 2, batch);
     trsm_ll_kernel<2><<<grid, 128, TrsmLL<2>::SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off);
   } else {
     // (an eight-warp, whole-tile form of the left-looking kernel was measured for this regime too: 611 us against 503 for
     // 128 x 31 tiles -- with the C tile in shared memory the DMMA operands cost two shared-memory loads each, where the
-    // register-tile kernels feed A from registers; the round-1 kernels stay for batches)
+    // register-tile kernels feed A from registers; those stay for batches)
     // With an envelope a block column has a few live row tiles per item (N = 4096, bench.py's draws: 176 of 496 per
     // item), and two rows per CTA measured best there (B200, 1000 W, TRSM class per call: 7.52 ms with 2, 7.72 with
     // 4 -- what the dense count picks -- 7.57 with 1).
     const int tpc = env.F ? 2 : (total >= 148 * 16 ? 4 : (total >= 148 * 6 ? 2 : 1));
     if (tpc == 1 || h->trsm_pipelined == 0) {
       dim3 grid(ntiles, batch);
-      trsm_tile_kernel<0><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, 0, c_off, TILE, env);
+      trsm_tile_kernel<<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off, env);
     } else {
       dim3 grid((ntiles + tpc - 1) / tpc, batch);
       trsm_tiles_pipelined_kernel<2><<<grid, 256, TRSM_PIPE_SMEM_BYTES, h->stream>>>(L, L, ld, stride, diag_off, c_off, ntiles, tpc, env);
@@ -1266,36 +1113,26 @@ int launch_trsm_tiles(Handle *h, double *L, long long ld, long long stride, int 
 
 int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base, int n,
                          long long c_off, int ntiles, int batch, int *info, TrsmEnv env) {
-  // one launch when the diagonal CTAs and the 64-row (or 32-row) TRSM CTAs of all matrices fit one wave at one CTA per SM
-  int mt = 0;
-  if (h->panel_fused && h->panel_impl == 0 && ntiles > 0 && batch <= PANEL_FUSED_MAX_BATCH) {
-    if (h->trsm_mt_override == 1 && (long long)batch * (1 + 4 * ntiles) <= 148) mt = 1;
-    else if ((long long)batch * (1 + 2 * ntiles) <= 148) mt = 2;
+  // one launch when the diagonal CTAs and the 64-row (or 128-row) TRSM CTAs of all matrices fit one wave at one CTA per SM
+  const bool fused = h->panel_fused && ntiles > 0 && batch <= PANEL_FUSED_MAX_BATCH;
+  if (fused && (long long)batch * (1 + 2 * ntiles) <= 148) {
+    ProfScope ps__(h, PC_POTRF);
+    const int chunks = ntiles * 2;
+    panel_fused_kernel<<<batch * (1 + chunks), PANEL_FUSED_THREADS, PANEL_FUSED_SMEM_BYTES, h->stream>>>(
+        L, ld, stride, diag_off, c_off, chunks, batch, index_base, n, info, h->panel_flags);
+    GPB_LAUNCH_CHECK(h);
+    return 0;
   }
-  if (mt == 0 && h->panel_fused && h->panel_impl == 0 && ntiles > 0 && batch <= PANEL_FUSED_MAX_BATCH &&
-      (long long)batch * (1 + ntiles) <= 148) {
+  if (fused && (long long)batch * (1 + ntiles) <= 148) {
     ProfScope ps__(h, PC_POTRF);
     panel_fused_tile_kernel<<<batch * (1 + ntiles), POTRF_PW_THREADS + 32, PANEL_FUSED_TILE_SMEM_BYTES, h->stream>>>(
         L, ld, stride, diag_off, c_off, ntiles, batch, index_base, n, info, h->panel_flags);
     GPB_LAUNCH_CHECK(h);
     return 0;
   }
-  if (mt == 0) {
-    int rc = launch_potrf_tile_at(h, L, ld, stride, diag_off, index_base, n, batch, info);
-    if (rc) return rc;
-    return launch_trsm_tiles_at(h, L, ld, stride, diag_off, c_off, ntiles, batch, env);
-  }
-  ProfScope ps__(h, PC_POTRF);
-  const int chunks = ntiles * (4 / mt);
-  const int grid = batch * (1 + chunks);
-  if (mt == 1)
-    panel_fused_kernel<1><<<grid, PANEL_FUSED_THREADS, PanelFused<1>::SMEM_BYTES, h->stream>>>(L, ld, stride, diag_off, c_off, chunks,
-                                                                                          batch, index_base, n, info, h->panel_flags);
-  else
-    panel_fused_kernel<2><<<grid, PANEL_FUSED_THREADS, PanelFused<2>::SMEM_BYTES, h->stream>>>(L, ld, stride, diag_off, c_off, chunks,
-                                                                                          batch, index_base, n, info, h->panel_flags);
-  GPB_LAUNCH_CHECK(h);
-  return 0;
+  int rc = launch_potrf_tile_at(h, L, ld, stride, diag_off, index_base, n, batch, info);
+  if (rc) return rc;
+  return launch_trsm_tiles_at(h, L, ld, stride, diag_off, c_off, ntiles, batch, env);
 }
 
 int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int tile_col, int ntiles_below, int n, int batch,
@@ -1311,8 +1148,7 @@ int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l
                            long long w_off, long long w_step, long long stride, int ntiles, int batch) {
   dim3 grid(ntiles, batch);
   ProfScope ps__(h, PC_TRSM);
-  if (h->panel_impl == 1) trsm_tile_kernel<1><<<grid, 256, TRSM_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step, TrsmEnv{});
-  else tile_inverse_ll_kernel<<<grid, 256, TINV_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step);
+  tile_inverse_ll_kernel<<<grid, 256, TINV_SMEM_BYTES, h->stream>>>(L, W, ld, stride, l_off, l_step, w_off, w_step);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

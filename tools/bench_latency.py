@@ -2,7 +2,7 @@
 (stan/gp_lml_stan.hpp -> gpb200_lml_grad, one theta per leapfrog step; models/fit_hyperparameters.stan:18-31
 under pendulum_fit.R:206).  Device-resident inputs, CUDA events over `reps` back-to-back calls, results
 With arguments "variants" the same measurement is repeated
-under the tuning knobs (look-ahead off, round-1 panel kernels, panel widths) in child processes."""
+under the tuning knobs (look-ahead off, panel widths, GEMM configurations) in child processes."""
 import json
 import os
 import subprocess
@@ -49,7 +49,6 @@ def measure(sizes=((4096, 1), (2048, 1), (1024, 1), (100, 1), (4096, 4), (1024, 
 VARIANTS = [
     ("default", {}),
     ("no_lookahead", {"GPB200_LOOKAHEAD": "0"}),
-    ("panel_v1_no_lookahead", {"GPB200_PANEL_V1": "1", "GPB200_LOOKAHEAD": "0", "GPB200_GEMM_CFG": "2"}),
     ("lookahead_pt2", {"GPB200_CHOL_PANEL": "2"}),
     ("lookahead_pt4", {"GPB200_CHOL_PANEL": "4"}),
     ("half8_only", {"GPB200_GEMM_CFG": "2"}),

@@ -1,6 +1,5 @@
-"""Times the panel kernels in isolation (gpb200_debug_bench_panel): round-2 left-looking shared-memory
-kernels against the round-1 register-tile kernels, at the batch sizes of the latency path (1, 4) and of
-the batched headline step (256)."""
+"""Times the panel kernels in isolation (gpb200_debug_bench_panel), with and without the fused POTRF + TRSM
+launch, at the batch sizes of the latency path (1, 4) and of the batched headline step (256)."""
 import json
 import os
 import subprocess
@@ -11,7 +10,6 @@ sys.path.insert(0, ".")
 
 def run_variant():
     from gp_b200 import capi
-    label_skip_inverse = os.environ.get("GPB200_TRSM_MT") is not None
     h = capi.Handle(0)
     out = {}
     for what, name in ((0, "potrf_tile"), (1, "trsm_tiles"), (2, "tile_inverse"), (3, "potrf+trsm")):
@@ -19,8 +17,6 @@ def run_variant():
             if what == 0 and nt != 32:
                 continue
             if what != 3 and nt > 32:
-                continue
-            if what == 2 and label_skip_inverse:
                 continue
             out["%s nt=%d B=%d" % (name, nt, batch)] = round(h.debug_bench_panel(what, nt, batch, 5) * 1e3, 2)
     print(json.dumps(out))
@@ -31,8 +27,7 @@ if __name__ == "__main__":
         run_variant()
         sys.exit(0)
     res = {}
-    for label, env in (("round2_panel_warp", {}), ("round2_two_launches", {"GPB200_PANEL_FUSED": "0"}), ("round1_v1", {"GPB200_PANEL_V1": "1"}),
-                       ("ll_mt1", {"GPB200_TRSM_MT": "1"}), ("ll_mt2", {"GPB200_TRSM_MT": "2"})):
+    for label, env in (("round2_panel_warp", {}), ("round2_two_launches", {"GPB200_PANEL_FUSED": "0"})):
         e = dict(os.environ); e.update(env)
         r = subprocess.run([sys.executable, __file__, "child"], env=e, capture_output=True, text=True)
         if r.returncode != 0:

@@ -20,10 +20,8 @@ for name, base in (("panel warp", 512), ("helper warp 7", 0)):
         else:
             print("  %2d: %5d | %5d" % (cb, r[1] - r[0], r[2] - r[1]))
 buf[:] = 0
-import os
-os.environ["GPB200_TRSM_MT"] = "1"
 h2 = capi.Handle(0)
-h2.debug_bench_panel(1, 8, 1, 1)
+h2.debug_bench_panel(1, 8, 1, 1)   # seven row tiles: trsm_ll_kernel<1>
 assert h2.lib.gpb200_debug_panel_trace(h2._h, buf.ctypes.data) == 0
 t = buf[1024:1024 + 19 * 8].reshape(19, 8)
 print("trsm warp 0: load+setup", t[17, 0] - t[18, 0], "loop", t[16, 0] - t[0, 0])
