@@ -66,6 +66,8 @@ SIGNATURES = {
                                                 C.c_void_p, C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_lml_grad_ard_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, _ll, C.c_void_p,
                                               C.c_double, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gpb200_lml_grad_ragged": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_double, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_rbf_cov_chol": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_void_p, C.c_void_p]),
     "gpb200_rbf_cov_chol_batched": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                               C.c_void_p]),
@@ -374,6 +376,34 @@ class Handle:
         self._check(self.lib.gpb200_lml_grad_batched(self._h, n, B, _ptr(x), x_stride, _ptr(y), y_stride, _ptr(theta),
                                                      jitter, int(want_grad), _ptr(lml), _ptr(grad), _ptr(info)),
                     "lml_grad_batched")
+
+    def lml_grad_ragged(self, xs, ys, theta, jitter=0.0, want_grad=True):
+        """B GPs of different sizes in one call: xs, ys are lists of B 1-D arrays (group b has len(xs[b]) >= 1 points),
+        theta (B, 3).  Returns lml[B], grad[B,3], info[B]."""
+        th = np.ascontiguousarray(theta, dtype=np.float64).reshape(-1, 3)
+        B = th.shape[0]
+        if len(xs) != B or len(ys) != B:
+            raise GpB200Error("lml_grad_ragged: %d x groups and %d y groups for %d theta rows" % (len(xs), len(ys), B))
+        sizes = [np.asarray(v).size for v in xs]
+        if [np.asarray(v).size for v in ys] != sizes:
+            raise GpB200Error("lml_grad_ragged: every y group must have as many points as its x group")
+        offsets = np.zeros(B + 1, dtype=np.int64)
+        offsets[1:] = np.cumsum(sizes)
+        x = np.ascontiguousarray(np.concatenate([np.ravel(v) for v in xs]) if B else np.empty(0), dtype=np.float64)
+        y = np.ascontiguousarray(np.concatenate([np.ravel(v) for v in ys]) if B else np.empty(0), dtype=np.float64)
+        lml = np.empty(B); grad = np.empty((B, 3)); info = np.zeros(B, dtype=np.int32)
+        self._check(self.lib.gpb200_lml_grad_ragged(self._h, B, _ptr(offsets), _ptr(x), _ptr(y), _ptr(th), jitter,
+                                                    int(want_grad), _ptr(lml), _ptr(grad), _ptr(info)), "lml_grad_ragged")
+        return lml, grad, info
+
+    def lml_grad_ragged_device(self, B, offsets, x, y, theta, jitter, want_grad, lml, grad, info):
+        """Device-pointer variant: x, y (concatenated groups), theta, lml, grad, info are torch CUDA tensors (float64 /
+        int32); offsets is a host int64 array of B + 1 entries.  The handle must be in device-pointer mode.
+        Asynchronous on the handle's stream."""
+        assert self.device_pointers
+        off = np.ascontiguousarray(offsets, dtype=np.int64)
+        self._check(self.lib.gpb200_lml_grad_ragged(self._h, B, _ptr(off), _ptr(x), _ptr(y), _ptr(theta), jitter,
+                                                    int(want_grad), _ptr(lml), _ptr(grad), _ptr(info)), "lml_grad_ragged")
 
     def lml_grad_deriv_batched(self, t, y, theta, jitter=0.0, order0=0, nblocks=None, want_grad=True):
         """GP observed through derivative orders order0 .. order0+nblocks-1 on the grid t.

@@ -251,6 +251,219 @@ extern "C" int gpb200_lml_grad_ard_batched(gpb200_handle_t h, int n, int D, int 
   return lml_core(h, LmlSpec{false, n, 0, 1, D}, B, X, x_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info);
 }
 
+// ---- B GPs of different sizes in one call ---------------------------------------------------------------------------
+// Items are bucketed by tile count nt = ceil(n_b / 128); each bucket is a uniform lock-step batch at np = 128 nt whose
+// kernels read the per-item size nvec.  The padding is exact: y is zero there and K_b is [K_b 0; 0 I], so the
+// Cholesky, the inverses, the solves and the selected inverse run unchanged, and only the Gram, the trace epilogues and
+// finalize need n_b.  Every bucket takes the routes lml_core would take for a batch of its size at its np.
+namespace {
+struct RaggedBucket {
+  int nt, slot0, count, max_n;
+  long long dst0;  // first double of the bucket in the staged x / y
+  double work;     // count * nt^3: the bucket with the most work is dispatched first
+};
+
+// per-item workspace of the tiled SE route at np (the same terms as lml_core)
+size_t se_item_bytes(int np, int nparts, int zks, bool use_env) {
+  const long long mat = (long long)np * np;
+  return pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * 4 * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) +
+         64 + (use_env ? (size_t)(2 * (np / TILE) + 2) * sizeof(int) : 0);
+}
+}  // namespace
+
+extern "C" int gpb200_lml_grad_ragged(gpb200_handle_t h, int B, const long long *offsets, const double *x, const double *y,
+                                      const double *theta, double jitter, int want_grad, double *lml, double *grad, int *info) {
+  CHECK_H(h);
+  if (B < 0) BAD_ARG(h, 2, "lml_grad_ragged: B must be >= 0 (negative batch)");
+  if (B == 0) return 0;
+  if (!offsets) BAD_ARG(h, 3, "lml_grad_ragged: offsets is NULL");
+  if (offsets[0] != 0) BAD_ARG(h, 3, "lml_grad_ragged: offsets[0] must be 0");
+  for (int b = 0; b < B; b++) {
+    const long long nb = offsets[b + 1] - offsets[b];
+    const char *why = nb < 0 ? "offsets must be non-decreasing" : nb == 0 ? "every group needs n_b >= 1 point"
+                      : nb > MAX_DENSE_N ? "n_b above 65407" : nullptr;
+    if (why) {
+      snprintf(h->err, sizeof(h->err), "lml_grad_ragged: %s (offsets[%d] = %lld, offsets[%d] = %lld)", why, b, offsets[b], b + 1,
+               offsets[b + 1]);
+      return -3;
+    }
+  }
+  const long long ntot = offsets[B];
+
+  // ---- schedule: buckets by tile count, caller order inside a bucket, the most work first ----
+  std::map<int, std::vector<int>> by_nt;
+  for (int b = 0; b < B; b++) by_nt[(int)((offsets[b + 1] - offsets[b] + TILE - 1) / TILE)].push_back(b);
+  std::vector<RaggedBucket> bk;
+  for (const auto &kv : by_nt) bk.push_back({kv.first, 0, (int)kv.second.size(), 0, 0, (double)kv.second.size() * kv.first * kv.first * kv.first});
+  std::stable_sort(bk.begin(), bk.end(), [](const RaggedBucket &a, const RaggedBucket &c) {
+    return a.work != c.work ? a.work > c.work : a.nt > c.nt;
+  });
+  std::vector<RaggedSlot> meta(B);
+  int slot = 0;
+  long long dst = 0;
+  for (auto &k : bk) {
+    const int np = k.nt * TILE;
+    k.slot0 = slot;
+    k.dst0 = dst;
+    for (int b : by_nt[k.nt]) {
+      const int nb = (int)(offsets[b + 1] - offsets[b]);
+      meta[slot++] = RaggedSlot{offsets[b], dst, nb, np, b, 0};
+      k.max_n = std::max(k.max_n, nb);
+      dst += np;
+    }
+  }
+  const long long xtot = dst;
+
+  // ---- routes and workspace: per bucket as lml_core decides them for a uniform batch of the bucket's size ----
+  struct Route { bool small, use_env, sinv; int zks, ntasks, Bc; size_t per_item; };
+  std::vector<Route> rt(bk.size());
+  const bool host = !h->device_ptrs;
+  // staged x, y, theta, slot-order results, sizes, slot table; in host mode also the caller's inputs and the results
+  // in caller order
+  const size_t fixed = 2 * pad256((size_t)xtot * 8) + 2 * pad256((size_t)B * 3 * 8) + pad256((size_t)B * 8) + 2 * pad256((size_t)B * 4) +
+                       pad256((size_t)B * sizeof(RaggedSlot)) +
+                       (host ? 2 * pad256((size_t)ntot * 8) + 2 * pad256((size_t)B * 3 * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4)
+                             : 0) +
+                       4096;
+  size_t need = 0;
+  for (size_t k = 0; k < bk.size(); k++) {
+    Route &r = rt[k];
+    const int nt = bk[k].nt, np = nt * TILE, Bk = bk[k].count;
+    r.small = nt == 1 && lml_small_applies(h, bk[k].max_n);
+    r.use_env = h->envelope && !r.small && nt >= 16 && nt <= ENV_MAX_NT;
+    r.sinv = r.use_env && want_grad && (h->sinv_min_batch > 0 ? Bk >= h->sinv_min_batch : (long long)Bk * nt >= 256);
+    r.zks = trmv_split_chunks(np, Bk);
+    r.ntasks = 0;
+    if (!r.small) {
+      TaskList tl;
+      RC(tasks_lauum(h, nt, &tl));
+      r.ntasks = tl.count(0);
+    }
+    r.per_item = r.small ? 0 : se_item_bytes(np, r.ntasks * 4, r.zks, r.use_env);
+    r.Bc = Bk;
+    need = std::max(need, r.per_item * (size_t)Bk);
+  }
+  if (h->ws_limit > 0 || fixed + need + 8192 > h->ws_bytes) {
+    size_t limit = (size_t)h->ws_limit;
+    if (h->ws_limit <= 0) {
+      size_t freeb = 0, totalb = 0;
+      GPB_CUDA(h, cudaMemGetInfo(&freeb, &totalb));
+      limit = (size_t)((freeb + h->ws_bytes) * 0.85);
+    }
+    need = 0;
+    for (Route &r : rt) {
+      if (r.small) continue;
+      if (limit < fixed + r.per_item + 8192) BAD_ARG(h, 1002, "lml_grad_ragged: workspace limit too small for one item");
+      r.Bc = (int)std::min<size_t>((size_t)r.Bc, (limit - fixed - 8192) / r.per_item);
+      need = std::max(need, r.per_item * (size_t)r.Bc);
+    }
+  }
+  for (Route &r : rt)
+    if (!r.small) r.Bc = std::min(r.Bc, 65535);  // gridDim.y of the batched launches
+  Arena a;
+  RC(ws_reserve(h, fixed + need + 8192, &a));
+  double *sx = a.take<double>((size_t)xtot), *sy = a.take<double>((size_t)xtot), *sth = a.take<double>((size_t)B * 3);
+  double *slml = a.take<double>(B), *sgrad = a.take<double>((size_t)B * 3);
+  int *sinfo = a.take<int>(B), *snv = a.take<int>(B);
+  RaggedSlot *dmeta = a.take<RaggedSlot>(B);
+  const double *cx = x, *cy = y, *cth = theta;
+  double *olml = lml, *ograd = want_grad ? grad : nullptr;
+  int *oinfo = info;
+  if (host) {
+    double *hx = a.take<double>((size_t)ntot), *hy = a.take<double>((size_t)ntot), *hth = a.take<double>((size_t)B * 3);
+    olml = lml ? a.take<double>(B) : nullptr;
+    ograd = want_grad && grad ? a.take<double>((size_t)B * 3) : nullptr;
+    oinfo = info ? a.take<int>(B) : nullptr;
+    if (!hth) BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
+    RC(to_device(h, x, hx, (size_t)ntot));
+    RC(to_device(h, y, hy, (size_t)ntot));
+    RC(to_device(h, theta, hth, (size_t)B * 3));
+    cx = hx; cy = hy; cth = hth;
+  }
+  if (!dmeta) BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
+  // pageable source: the copy has taken the vector's contents when cudaMemcpyAsync returns
+  GPB_CUDA(h, cudaMemcpyAsync(dmeta, meta.data(), (size_t)B * sizeof(RaggedSlot), cudaMemcpyHostToDevice, h->stream));
+  RC(launch_ragged_stage(h, B, dmeta, cx, cy, cth, sx, sy, sth, snv));
+  GPB_CUDA(h, cudaMemsetAsync(sinfo, 0, (size_t)B * sizeof(int), h->stream));
+
+  for (size_t k = 0; k < bk.size(); k++) {
+    const RaggedBucket &K = bk[k];
+    const Route &r = rt[k];
+    const int nt = K.nt, np = nt * TILE;
+    const long long mat = (long long)np * np;
+    const double *bx = sx + K.dst0, *by = sy + K.dst0, *bth = sth + 3LL * K.slot0;
+    const int *bnv = snv + K.slot0;
+    double *blml = slml + K.slot0, *bgrad = sgrad + 3LL * K.slot0;
+    int *binfo = sinfo + K.slot0;
+    if (r.small) {
+      RC(launch_lml_small(h, K.max_n, bx, np, by, np, bth, jitter, want_grad, blml, bgrad, binfo, K.count, bnv));
+      continue;
+    }
+    TaskList tl;
+    RC(tasks_lauum(h, nt, &tl));
+    Arena ab = a;  // the buckets run one after the other on one stream: each reuses the same scratch
+    double *Lbuf = ab.take<double>((size_t)r.Bc * mat), *Sbuf = ab.take<double>((size_t)r.Bc * mat);
+    double *zbuf = ab.take<double>((size_t)r.Bc * np), *abuf = ab.take<double>((size_t)r.Bc * np), *dvec = ab.take<double>((size_t)r.Bc * np);
+    double *partial = ab.take<double>((size_t)r.Bc * r.ntasks * 4 * 4);
+    double *zpart = r.zks > 1 ? ab.take<double>((size_t)r.Bc * r.zks * np) : nullptr;
+    int *env = nullptr, *order = nullptr;
+    if (r.use_env && (!(env = ab.take<int>((size_t)r.Bc * 2 * nt)) || !(order = ab.take<int>((size_t)r.Bc * 2))))
+      BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
+    if (!partial || (r.zks > 1 && !zpart)) BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
+    for (int b0 = 0; b0 < K.count; b0 += r.Bc) {
+      const int bc = std::min(r.Bc, K.count - b0);
+      const double *ccx = bx + (long long)b0 * np, *ccy = by + (long long)b0 * np, *cct = bth + 3LL * b0;
+      const int *cnv = bnv + b0;
+      if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
+      RC(launch_gram_se_batched(h, np, np, ccx, np, cct, jitter, 1, Lbuf, mat, bc, env, cnv));
+      if (env) RC(launch_envelope_profile(h, nt, env, order, bc));
+      RC(chol_batched(h, Lbuf, np, mat, np, bc, binfo + b0, env, order));  // padded pivots are 1: info stays within n_b
+      RC(extract_diag(h, np, Lbuf, mat, dvec, bc));
+      int n1 = 0, n2 = 0;
+      if (r.sinv) {
+        RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
+        RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, ccy, np, nullptr, np, zbuf, np, bc, env));
+        RC(launch_backsub_band(h, np, Lbuf, Sbuf, mat, env, zbuf, abuf, bc));
+        RC(sinv_batched(h, Lbuf, Sbuf, np, mat, env, order, bc));
+        RC(launch_trace_sinv(h, np, np, Lbuf, mat, env, ccx, np, abuf, cct, partial, bc, cnv));
+        n1 = r.ntasks;
+      } else if (want_grad) {
+        RC(trtri_batched(h, Lbuf, Sbuf, np, mat, bc));
+        if (r.zks > 1) RC(launch_trmv_lower_n_split(h, np, r.zks, Lbuf, mat, ccy, np, np, zpart, zbuf, np, bc));
+        else RC(launch_trmv_lower_n(h, np, Lbuf, mat, ccy, np, np, zbuf, np, bc));
+        RC(launch_trmv_lower_t(h, np, Lbuf, mat, zbuf, np, abuf, np, bc));
+        GemmParams p{};
+        p.A = mref(Lbuf, np, mat);
+        p.B = mref(Lbuf, np, mat);
+        p.C = mref(nullptr, np, mat);
+        p.tasks = tl.at(0);
+        p.x = ccx; p.x_stride = np;
+        p.avec = abuf; p.a_stride = np;
+        p.theta = cct;
+        p.partial = partial;
+        p.n = np;
+        p.nvec = cnv;
+        p.ntasks = r.ntasks;
+        p.theta_stride = 3;
+        RC(launch_gemm(h, LAYOUT_TN, EPI_TRACE_RAGGED, p, r.ntasks, bc));
+      } else {
+        RC(launch_tile_inverse(h, Lbuf, Sbuf, np, mat, nt, bc));
+        if (bc >= 32) RC(launch_trsv_blocked(h, np, Lbuf, Sbuf, mat, ccy, np, nullptr, np, zbuf, np, bc, env));
+        else RC(launch_trsv_sweep(h, np, Lbuf, Sbuf, mat, ccy, np, nullptr, np, zbuf, abuf, np, bc));
+      }
+      if (!r.sinv) RC(gemm_partial_layout(h, tl.at(0), r.ntasks, bc, &n1, &n2));
+      RC(launch_finalize(h, np, np, want_grad, dvec, zbuf, abuf, partial, n1, n2, cct, blml + b0, bgrad + 3LL * b0, bc, cnv));
+    }
+  }
+  if (olml || ograd || oinfo) RC(launch_ragged_scatter(h, B, dmeta, slml, sgrad, sinfo, olml, ograd, oinfo));
+  if (host) {
+    if (lml) RC(from_device(h, olml, lml, (size_t)B * sizeof(double)));
+    if (ograd) RC(from_device(h, ograd, grad, (size_t)B * 3 * sizeof(double)));
+    if (info) RC(from_device(h, oinfo, info, (size_t)B * sizeof(int)));
+  }
+  return finish(h);
+}
+
 // number of CUDA-graph replays so far (small evaluations are replayed as one graph)
 extern "C" long long gpb200_graph_replays(gpb200_handle_t h) { return h ? h->graph_replays : 0; }
 

@@ -70,6 +70,7 @@ struct GemmParams {
   MatRef CT;                    // EPI_AXPBY: when CT.p is set the transpose of the output tile is written there too
   unsigned long long *flops;    // when set: every CTA adds the flops it executes (after all skipping)
   int ard_d;                    // EPI_TRACE_ARD: input dimensions D (x is n x D column-major per item, theta_stride = D + 2)
+  const int *nvec;              // EPI_TRACE_RAGGED: per-item sizes (the mask of item b is nvec[b] instead of n)
 };
 // envelope modes of the tile GEMM.  Only products with an exactly-zero operand tile are dropped, and the k order of
 // the rest is kept, so a result is bit-identical to the dense launch (up to the sign of an all-zero tile).
@@ -214,7 +215,9 @@ struct ProfScope {
 
 // ---- launchers implemented in the .cu files --------------------------------------------------
 enum GemmLayout { LAYOUT_NT = 0, LAYOUT_TN = 1, LAYOUT_NN = 2, LAYOUT_TT = 3 };  // TT: A k-contiguous, B n-contiguous
-enum GemmEpi { EPI_AXPBY = 0, EPI_TRACE = 1, EPI_TRACE_DERIV = 2, EPI_TRACE_ARD = 3 };
+// EPI_TRACE_RAGGED: the EPI_TRACE epilogue with a per-item size (gpb200_lml_grad_ragged), its own instantiation so that
+// the uniform one stays as it is
+enum GemmEpi { EPI_AXPBY = 0, EPI_TRACE = 1, EPI_TRACE_DERIV = 2, EPI_TRACE_ARD = 3, EPI_TRACE_RAGGED = 4 };
 constexpr int ARD_MAX_D = 8;  // input dimensions of the ARD covariance (gpb200_lml_grad_ard_batched)
 // doubles per CTA partial record of a trace epilogue: (S_se, S_d2, tr G, 0); (S_k, S_dk, tr G per block, ...);
 // (S_e, S_1 .. S_ARD_MAX_D, tr G)
@@ -254,7 +257,8 @@ int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l
 // launches to order[0..batch) (order[batch..2 batch) is its scratch)
 int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch);
 int launch_trace_sinv(Handle *h, int n, int np, const double *Z, long long stride, const int *env, const double *x,
-                      long long x_stride, const double *a, const double *theta, double *partial, int batch);
+                      long long x_stride, const double *a, const double *theta, double *partial, int batch,
+                      const int *nvec = nullptr);  // nvec: per-item sizes (device), nullptr = n for every item
 int launch_backsub_band(Handle *h, int np, const double *L, const double *Wdiag, long long stride, const int *env,
                         const double *z, double *a, int batch);
 int panel_smem_setup(Handle *h);

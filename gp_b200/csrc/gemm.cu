@@ -109,10 +109,18 @@ __global__ void __launch_bounds__(Cfg::NTHREADS, Cfg::MINB) gemm_trace_ard_kerne
 #include "gemm_tile_body.cuh"
 }
 
+// TN layout + the SE trace epilogue masked by a per-item size (gpb200_lml_grad_ragged), under its own name as well
+template <class Cfg, bool A_KC, bool B_KC, int EPI>
+__global__ void __launch_bounds__(Cfg::NTHREADS, Cfg::MINB) gemm_trace_ragged_kernel(const GemmParams p) {
+  static_assert(A_KC && B_KC && EPI == EPI_TRACE_RAGGED, "gemm_trace_ragged_kernel is the TN layout with the ragged SE epilogue");
+#include "gemm_tile_body.cuh"
+}
+
 template <class Cfg, bool A_KC, bool B_KC, int EPI>
 static int launch_one(Handle *h, const GemmParams &p, int ntasks, int batch) {
   void (*kern)(const GemmParams);
   if constexpr (EPI == EPI_TRACE_ARD) kern = gemm_trace_ard_kernel<Cfg, A_KC, B_KC, EPI>;
+  else if constexpr (EPI == EPI_TRACE_RAGGED) kern = gemm_trace_ragged_kernel<Cfg, A_KC, B_KC, EPI>;
   else kern = gemm_tile_kernel<Cfg, A_KC, B_KC, EPI>;
   dim3 grid(ntasks * Cfg::NSPLIT, batch);
   ProfScope ps__(h, PC_GEMM);
@@ -130,6 +138,7 @@ static int smem_setup_cfg(Handle *h) {
   GPB_CUDA(h, cudaFuncSetAttribute(gemm_tile_kernel<Cfg, true, true, EPI_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(gemm_tile_kernel<Cfg, false, false, EPI_TRACE>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(gemm_tile_kernel<Cfg, true, true, EPI_TRACE_DERIV>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
+  GPB_CUDA(h, cudaFuncSetAttribute(gemm_trace_ragged_kernel<Cfg, true, true, EPI_TRACE_RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   GPB_CUDA(h, cudaFuncSetAttribute(gemm_trace_ard_kernel<Cfg, true, true, EPI_TRACE_ARD>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM_BYTES));
   return 0;
 }
@@ -159,6 +168,7 @@ static int launch_cfg(Handle *h, GemmLayout layout, GemmEpi epi, const GemmParam
   } else if (layout == LAYOUT_TN) {
     if (epi == EPI_TRACE_DERIV) return launch_one<Cfg, true, true, EPI_TRACE_DERIV>(h, p, ntasks, batch);
     if (epi == EPI_TRACE_ARD) return launch_one<Cfg, true, true, EPI_TRACE_ARD>(h, p, ntasks, batch);
+    if (epi == EPI_TRACE_RAGGED) return launch_one<Cfg, true, true, EPI_TRACE_RAGGED>(h, p, ntasks, batch);
     return launch_one<Cfg, true, true, EPI_TRACE>(h, p, ntasks, batch);
   } else if (layout == LAYOUT_NT && epi == EPI_TRACE) {
     return launch_one<Cfg, false, false, EPI_TRACE>(h, p, ntasks, batch);  // G = X X^T of the distributed gradient (api_mg.cu)

@@ -1,7 +1,7 @@
 // Body of the tile GEMM kernels of gemm.cu (no include guard: it is included once inside each kernel definition,
-// where Cfg, A_KC, B_KC, EPI and the parameter block p are in scope).  The two kernels share it textually: moving it
-// into a __forceinline__ device function called by both changes the register allocation of the existing
-// gemm_tile_kernel instantiations, and the ARD epilogue runs under its own kernel name.
+// where Cfg, A_KC, B_KC, EPI and the parameter block p are in scope).  The kernels share it textually: moving it
+// into a __forceinline__ device function called by all of them changes the register allocation of the existing
+// gemm_tile_kernel instantiations, and the ARD and ragged epilogues run under their own kernel names.
   constexpr int WARPS_N = Cfg::WARPS_N, WM = Cfg::WM, WN = Cfg::WN, MI = Cfg::MI, NI = Cfg::NI;
   constexpr int NTHREADS = Cfg::NTHREADS, NCOPY_A = Cfg::NCOPY_A, NCOPY_B = Cfg::NCOPY_B;
   constexpr int STAGES = Cfg::STAGES, TN = Cfg::TN, LD_MC_B = Cfg::LD_MC_B;
@@ -389,12 +389,15 @@
     double *red = smem + 4 * TILE;
     const double *x = p.x + b * p.x_stride;
     const double *av = p.avec + b * p.a_stride;
+    // the item's true size, the mask of its padding (spelled out at each use: a local copy changes the SASS of the
+    // uniform EPI_TRACE instantiations)
+#define GPB_TRACE_N ((EPI == EPI_TRACE_RAGGED) ? p.nvec[b] : p.n)
     for (int q = tid; q < TM + TN; q += NTHREADS) {
       const bool row = q < TM;
       const int ql = row ? q : q - TM;
       const int i = (row ? task.c_r : task.c_c) + ql;
-      (row ? xr : xc)[ql] = (i < p.n) ? x[i] : 0.0;
-      (row ? ar : ac)[ql] = (i < p.n) ? av[i] : 0.0;
+      (row ? xr : xc)[ql] = (i < GPB_TRACE_N) ? x[i] : 0.0;
+      (row ? ar : ac)[ql] = (i < GPB_TRACE_N) ? av[i] : 0.0;
     }
     __syncthreads();
     const double rho = p.theta[b * 3 + 1];
@@ -413,7 +416,7 @@
           const int ml = wm + mi * 8 + 2 * t + e;
           const int i = task.c_r + ml;
           const double G = acc[ni][mi][e];
-          if (i < p.n && j < p.n) {
+          if (i < GPB_TRACE_N && j < GPB_TRACE_N) {
             const double d = xr[ml] - xc[nl];
             const double d2 = d * d;
             const double ek = exp_nonpos(d2 * nh);
@@ -458,4 +461,5 @@
       o[2] = r2;
       o[3] = 0.0;
     }
+#undef GPB_TRACE_N
   }

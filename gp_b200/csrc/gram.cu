@@ -72,14 +72,17 @@ __global__ void __launch_bounds__(256) gram_outer_kernel(int kind, int n, int m,
 // ---- batched padded SE Gram for the fused LML path: K = alpha^2 exp(-0.5 d^2/rho^2) + c I -------
 // Internal layout: np x np (np multiple of 128) per item, identity in the padding so that the
 // padded factor is [L 0; 0 I].  Only tiles with tile_row >= tile_col are produced when lower_only.
-__global__ void __launch_bounds__(256) gram_se_batched_kernel(int n, int np, const double *__restrict__ x,
+// RAGGED: item b has its own size nvec[b] <= np (gpb200_lml_grad_ragged), identity beyond it.
+template <bool RAGGED>
+__global__ void __launch_bounds__(256) gram_se_batched_kernel(int n_all, int np, const double *__restrict__ x,
                                                              long long x_stride, const double *__restrict__ theta,
                                                              double jitter, int lower_only,
                                                              double *__restrict__ K, long long stride,
-                                                             int *__restrict__ envF) {
+                                                             int *__restrict__ envF, const int *__restrict__ nvec) {
   const int nt = np / TILE;
   const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
   if (lower_only && tr < tc) return;
+  const int n = RAGGED ? nvec[blockIdx.y] : n_all;
   // envF (optional, item stride 2 nt, preset to INT_MAX per tile row): the first tile column of each tile row whose exp(-d^2/2rho^2) is
   // not exactly zero somewhere (NaN counts as nonzero).  That set holds the support of K and of dK/dtheta.
   bool nz = tr == tc;
@@ -538,11 +541,16 @@ int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const 
 }
 
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF) {
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF,
+                           const int *nvec) {
   const int nt = np / TILE;
   dim3 grid(nt * nt, batch);
   ProfScope ps__(h, PC_GRAM);
-  gram_se_batched_kernel<<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF);
+  if (nvec)
+    gram_se_batched_kernel<true><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF, nvec);
+  else
+    gram_se_batched_kernel<false><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF,
+                                                               nullptr);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

@@ -11,7 +11,8 @@ int launch_kernel_eval(Handle *h, int kind, long long len, const double *tj, con
 int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const double *y, double amp2, double l,
                       double *K, long long ldk);
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF = nullptr);
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF = nullptr,
+                           const int *nvec = nullptr);  // nvec: per-item sizes (device), nullptr = n for every item
 int launch_gram_tangent(Handle *h, int n, int np, const double *x, double alpha, const double *ls, double dadd, int mode,
                         double *S, double *Sdot, long long stride, int batch);
 int launch_gram_deriv(Handle *h, int n, int nblocks, const double *t, double alpha, double rho, const double *noise,
@@ -55,7 +56,8 @@ int launch_trsv_sweep(Handle *h, int np, const double *L, const double *Wdiag, l
                       long long y_stride, const double *mu, int n_valid, double *z, double *acc, long long z_stride,
                       int batch);
 int launch_finalize(Handle *h, int n, int np, int want_grad, const double *dvec, const double *z, const double *a,
-                    const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch);
+                    const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch,
+                    const int *nvec = nullptr);
 int launch_finalize_ard(Handle *h, int n, int D, int np, int want_grad, const double *dvec, const double *z, const double *a,
                         const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch);
 int launch_finalize_deriv(Handle *h, int n_grid, int nblocks, int np, int want_grad, const double *dvec, const double *z,
@@ -78,8 +80,18 @@ int launch_sumsq_logdiag(Handle *h, int n, const double *z, const double *L, lon
 // small.cu
 int small_smem_setup(Handle *h);
 bool lml_small_applies(const Handle *h, int n);
+// nvec (device, optional): per-item sizes <= n; n then only sizes the shared-memory tile
 int launch_lml_small(Handle *h, int n, const double *x, long long x_stride, const double *y, long long y_stride,
-                     const double *theta, double jitter, int want_grad, double *lml, double *grad, int *info, int batch);
+                     const double *theta, double jitter, int want_grad, double *lml, double *grad, int *info, int batch,
+                     const int *nvec = nullptr);
+// ragged staging (gpb200_lml_grad_ragged): slot s of the bucketed batch gets item meta[s].idx's slices of x and y,
+// zero-padded to meta[s].np, its theta and its size
+struct RaggedSlot { long long src, dst; int n, np, idx, pad_; };
+int launch_ragged_stage(Handle *h, int slots, const RaggedSlot *meta, const double *x, const double *y,
+                        const double *theta, double *dx, double *dy, double *dth, int *nvec);
+// results of slot s to the caller's index meta[s].idx (grad / info skipped when null)
+int launch_ragged_scatter(Handle *h, int slots, const RaggedSlot *meta, const double *lml_s, const double *grad_s,
+                          const int *info_s, double *lml, double *grad, int *info);
 
 // rng.cu
 int launch_normal_fill(Handle *h, unsigned long long seed, unsigned long long offset, long long len, long long rows,

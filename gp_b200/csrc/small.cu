@@ -35,10 +35,13 @@ __device__ __forceinline__ double warp_sum_s(double v) {
   return v;
 }
 
+// RAGGED: item b has its own size nvec[b] <= n8 (gpb200_lml_grad_ragged); rows and columns from it to n8 are identity
+template <bool RAGGED>
 __global__ void __launch_bounds__(256, 2)
-lml_small_kernel(int n, int n8, const double *__restrict__ x, long long x_stride, const double *__restrict__ y,
+lml_small_kernel(int n_all, int n8, const double *__restrict__ x, long long x_stride, const double *__restrict__ y,
                  long long y_stride, const double *__restrict__ theta, double jitter, int want_grad,
-                 double *__restrict__ lml, double *__restrict__ grad, int *__restrict__ info) {
+                 double *__restrict__ lml, double *__restrict__ grad, int *__restrict__ info, const int *__restrict__ nvec) {
+  const int n = RAGGED ? nvec[blockIdx.x] : n_all;
   extern __shared__ __align__(16) double sm[];
   const int ld = n8 + 4, nb = n8 >> 3;
   double *T = sm;                          // T[c * ld + r]
@@ -328,18 +331,24 @@ static size_t small_smem_bytes(int n8) {
 }
 
 int small_smem_setup(Handle *h) {
-  GPB_CUDA(h, cudaFuncSetAttribute(lml_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem_bytes(SMALL_MAX_N)));
+  GPB_CUDA(h, cudaFuncSetAttribute(lml_small_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem_bytes(SMALL_MAX_N)));
+  GPB_CUDA(h, cudaFuncSetAttribute(lml_small_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)small_smem_bytes(SMALL_MAX_N)));
   return 0;
 }
 
 bool lml_small_applies(const Handle *h, int n) { return h->small_kernel && n <= SMALL_MAX_N; }
 
 int launch_lml_small(Handle *h, int n, const double *x, long long x_stride, const double *y, long long y_stride,
-                     const double *theta, double jitter, int want_grad, double *lml, double *grad, int *info, int batch) {
+                     const double *theta, double jitter, int want_grad, double *lml, double *grad, int *info, int batch,
+                     const int *nvec) {
   const int n8 = round_up(n, 8);
   ProfScope ps__(h, PC_OTHER);
-  lml_small_kernel<<<batch, 256, small_smem_bytes(n8), h->stream>>>(n, n8, x, x_stride, y, y_stride, theta, jitter, want_grad,
-                                                                   lml, grad, info);
+  if (nvec)
+    lml_small_kernel<true><<<batch, 256, small_smem_bytes(n8), h->stream>>>(n, n8, x, x_stride, y, y_stride, theta, jitter,
+                                                                           want_grad, lml, grad, info, nvec);
+  else
+    lml_small_kernel<false><<<batch, 256, small_smem_bytes(n8), h->stream>>>(n, n8, x, x_stride, y, y_stride, theta, jitter,
+                                                                            want_grad, lml, grad, info, nullptr);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

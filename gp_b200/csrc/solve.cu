@@ -245,14 +245,16 @@ __global__ void __launch_bounds__(256) trsv_update_kernel(long long ld, long lon
   if (half == 0) acc[b * z_stride + acc_row0 + blockIdx.x * TILE + r] += ssum + part[r];
 }
 
-// Deterministic finalisation, one CTA per batch item.
-__global__ void __launch_bounds__(256) finalize_kernel(int n, int np, int want_grad, const double *__restrict__ dvec,
+// Deterministic finalisation, one CTA per batch item.  RAGGED: item b has its own size nvec[b].
+template <bool RAGGED>
+__global__ void __launch_bounds__(256) finalize_kernel(int n_all, int np, int want_grad, const double *__restrict__ dvec,
                                                       const double *__restrict__ z, const double *__restrict__ a,
                                                       const double *__restrict__ partial, int ntasks, int ntasks2,
                                                       const double *__restrict__ theta, double *__restrict__ lml,
-                                                      double *__restrict__ grad) {
+                                                      double *__restrict__ grad, const int *__restrict__ nvec) {
   __shared__ double red[8][6];
   const long long b = blockIdx.x;
+  const int n = RAGGED ? nvec[b] : n_all;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   double ld = 0.0, qf = 0.0, aa = 0.0, p0 = 0.0, p1 = 0.0, p2 = 0.0;
   for (int i = tid; i < n; i += 256) {
@@ -602,14 +604,17 @@ int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch) 
 // the envelope): one CTA per lower tile (I, J) of one item, the same sums as the EPI_TRACE epilogue of the dense route
 //   [0] w sum (a_i a_j - Z_ij) e_ij,  [1] w sum (a_i a_j - Z_ij) e_ij d_ij^2,  [2] tr Z on diagonal tiles
 // with w = 2 off the diagonal (the tile stands for its transpose too).  Outside the envelope e_ij is exactly zero:
-// those CTAs only write zeros.
-__global__ void __launch_bounds__(256) trace_sinv_kernel(int n, int np, const double *__restrict__ Z, long long stride,
+// those CTAs only write zeros.  RAGGED: item b has its own size nvec[b].
+template <bool RAGGED>
+__global__ void __launch_bounds__(256) trace_sinv_kernel(int n_all, int np, const double *__restrict__ Z, long long stride,
                                                         const int *__restrict__ env, const double *__restrict__ x,
                                                         long long x_stride, const double *__restrict__ a,
-                                                        const double *__restrict__ theta, double *__restrict__ partial) {
+                                                        const double *__restrict__ theta, double *__restrict__ partial,
+                                                        const int *__restrict__ nvec) {
   __shared__ double xr[TILE], xc[TILE], ar[TILE], ac[TILE], red[8][3];
   const int nt = np / TILE, q = blockIdx.x, tid = threadIdx.x;
   const long long b = blockIdx.y;
+  const int n = RAGGED ? nvec[b] : n_all;
   int I = (int)((sqrt(8.0 * q + 1.0) - 1.0) * 0.5);
   while (I * (I + 1) / 2 > q) I--;
   while ((I + 1) * (I + 2) / 2 <= q) I++;
@@ -662,11 +667,12 @@ __global__ void __launch_bounds__(256) trace_sinv_kernel(int n, int np, const do
 }
 
 int launch_trace_sinv(Handle *h, int n, int np, const double *Z, long long stride, const int *env, const double *x,
-                      long long x_stride, const double *a, const double *theta, double *partial, int batch) {
+                      long long x_stride, const double *a, const double *theta, double *partial, int batch, const int *nvec) {
   const int nt = np / TILE;
   dim3 grid(nt * (nt + 1) / 2, batch);
   ProfScope ps__(h, PC_OTHER);
-  trace_sinv_kernel<<<grid, 256, 0, h->stream>>>(n, np, Z, stride, env, x, x_stride, a, theta, partial);
+  if (nvec) trace_sinv_kernel<true><<<grid, 256, 0, h->stream>>>(n, np, Z, stride, env, x, x_stride, a, theta, partial, nvec);
+  else trace_sinv_kernel<false><<<grid, 256, 0, h->stream>>>(n, np, Z, stride, env, x, x_stride, a, theta, partial, nullptr);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }
@@ -722,9 +728,61 @@ int launch_backsub_band(Handle *h, int np, const double *L, const double *Wdiag,
 }
 
 int launch_finalize(Handle *h, int n, int np, int want_grad, const double *dvec, const double *z, const double *a,
-                    const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch) {
+                    const double *partial, int ntasks, int ntasks2, const double *theta, double *lml, double *grad, int batch,
+                    const int *nvec) {
   ProfScope ps__(h, PC_OTHER);
-  finalize_kernel<<<batch, 256, 0, h->stream>>>(n, np, want_grad, dvec, z, a, partial, ntasks, ntasks2, theta, lml, grad);
+  if (nvec)
+    finalize_kernel<true><<<batch, 256, 0, h->stream>>>(n, np, want_grad, dvec, z, a, partial, ntasks, ntasks2, theta, lml, grad,
+                                                        nvec);
+  else
+    finalize_kernel<false><<<batch, 256, 0, h->stream>>>(n, np, want_grad, dvec, z, a, partial, ntasks, ntasks2, theta, lml,
+                                                         grad, nullptr);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+// ---- ragged batches (gpb200_lml_grad_ragged) ---------------------------------------------------------------------------
+// Gather: one CTA per slot (blockIdx.x: gridDim.x holds any batch size).  Item meta[s].idx's n points of x and y go to the slot's np-long rows of dx / dy with zeros
+// after them: with y zero there and the Gram the identity, z = L^-1 y and a = K^-1 y are exactly zero in the padding.
+__global__ void __launch_bounds__(256) ragged_stage_kernel(const RaggedSlot *__restrict__ meta, const double *__restrict__ x,
+                                                           const double *__restrict__ y, const double *__restrict__ theta,
+                                                           double *__restrict__ dx, double *__restrict__ dy,
+                                                           double *__restrict__ dth, int *__restrict__ nvec) {
+  const long long s = blockIdx.x;
+  const RaggedSlot m = meta[s];
+  for (int i = threadIdx.x; i < m.np; i += blockDim.x) {
+    dx[m.dst + i] = i < m.n ? x[m.src + i] : 0.0;
+    dy[m.dst + i] = i < m.n ? y[m.src + i] : 0.0;
+  }
+  if (threadIdx.x < 3) dth[3 * s + threadIdx.x] = theta[3LL * m.idx + threadIdx.x];
+  if (threadIdx.x == 0) nvec[s] = m.n;
+}
+
+// Scatter: the results of slot s go to the caller's item meta[s].idx
+__global__ void ragged_scatter_kernel(int slots, const RaggedSlot *__restrict__ meta, const double *__restrict__ lml_s,
+                                      const double *__restrict__ grad_s, const int *__restrict__ info_s,
+                                      double *__restrict__ lml, double *__restrict__ grad, int *__restrict__ info) {
+  const int s = blockIdx.x * blockDim.x + threadIdx.x;
+  if (s >= slots) return;
+  const long long b = meta[s].idx;
+  if (lml) lml[b] = lml_s[s];
+  if (grad)
+    for (int k = 0; k < 3; k++) grad[3 * b + k] = grad_s[3LL * s + k];
+  if (info) info[b] = info_s[s];
+}
+
+int launch_ragged_stage(Handle *h, int slots, const RaggedSlot *meta, const double *x, const double *y,
+                        const double *theta, double *dx, double *dy, double *dth, int *nvec) {
+  ProfScope ps__(h, PC_OTHER);
+  ragged_stage_kernel<<<slots, 256, 0, h->stream>>>(meta, x, y, theta, dx, dy, dth, nvec);
+  GPB_LAUNCH_CHECK(h);
+  return 0;
+}
+
+int launch_ragged_scatter(Handle *h, int slots, const RaggedSlot *meta, const double *lml_s, const double *grad_s,
+                          const int *info_s, double *lml, double *grad, int *info) {
+  ProfScope ps__(h, PC_OTHER);
+  ragged_scatter_kernel<<<(slots + 255) / 256, 256, 0, h->stream>>>(slots, meta, lml_s, grad_s, info_s, lml, grad, info);
   GPB_LAUNCH_CHECK(h);
   return 0;
 }

@@ -59,6 +59,12 @@ def gp_lml_grad_ard_draws(X, y, theta, jitter=0.0, want_grad=True, handle=None):
     return (handle or capi.default_handle()).lml_grad_ard_batched(X, y, theta, jitter, want_grad)
 
 
+def gp_lml_grad_groups(xs, ys, theta, jitter=0.0, want_grad=True, handle=None):
+    """One GP per group with the group's own size (multiple_players.stan:59-63): xs, ys lists of B 1-D arrays,
+    theta (B, 3).  All B LMLs and gradients in one call; returns lml[B], grad[B,3], info[B]."""
+    return (handle or capi.default_handle()).lml_grad_ragged(xs, ys, theta, jitter, want_grad)
+
+
 def fit_hyperparameters_lp(x, y, log_rho, log_alpha, log_sigma, handle=None):
     """lp__ and its gradient w.r.t. the unconstrained (log rho, log alpha, log sigma) for
     models/fit_hyperparameters.stan: `~` likelihood (constant dropped, :31), gamma(4,4) and

@@ -187,6 +187,19 @@ GPB200_API int gpb200_lml_grad_ard_batched(gpb200_handle_t h, int n, int D, int 
                                            const double *y, long long y_stride, const double *theta, double jitter,
                                            int want_grad, double *lml, double *grad, int *info);
 
+/* B independent GPs of different sizes (per-group GPs, multiple_players.stan:59-63), the model of
+ * gpb200_lml_grad_batched for each: item b owns x[offsets[b] .. offsets[b+1]) and the same slice of y,
+ * n_b = offsets[b+1] - offsets[b] >= 1 (at most 65407).  offsets: HOST array of B + 1 int64, offsets[0] = 0,
+ * non-decreasing (sizes are scheduling information, as ls of gpb200_rbf_cov_chol_batched).  x, y, theta (B x 3
+ * row-major), lml[B], grad[B*3], info[B] follow the pointer mode; any of lml, grad, info may be NULL and is then
+ * not written (grad is not written when want_grad = 0).  B has no limit beyond memory.  info[b] in 1..n_b as in gpb200_lml_grad_batched; the other items are unaffected by a failing one.
+ * Item b gives, to rounding, what gpb200_lml_grad_batched(h, n_b, 1, x + offsets[b], 0, y + offsets[b], 0,
+ * theta + 3b, ...) gives.  The items run as one lock-step batch per tile count ceil(n_b / 128), zero-padded to
+ * 128 * that count (the padding is exact), the bucket with the most work first. */
+GPB200_API int gpb200_lml_grad_ragged(gpb200_handle_t h, int B, const long long *offsets, const double *x,
+                                      const double *y, const double *theta, double jitter, int want_grad,
+                                      double *lml, double *grad, int *info);
+
 /* ---- a1-a3: the reference's one native entry point ----------------------------------------- */
 /* Exact twin of rbf_cov_chol (covariance.cpp:9-47): Sigma = exp(-(xi-xj)^2/(2 l^2)) + 1e-10 I,
  * L = chol(Sigma), dLdl = d L / d l (forward mode); both n x n column-major with zero strict

@@ -80,6 +80,12 @@ gp_lml_grad_draws <- function(x, y, theta, jitter = 0) .Call("gp_lml_grad_draws"
 # (D + 2) x B, one (alpha, rho_1 .. rho_D, sigma) per column; grad has the same layout
 gp_lml_grad_ard_draws <- function(X, y, theta, jitter = 0) .Call("gp_lml_grad_ard_draws", as.matrix(X), y, theta, jitter)
 
+# ---- one GP per group, groups of different sizes (multiple_players.stan:59-63) ----
+# x_list, y_list: lists of numeric vectors, one per group; theta: 3 x G matrix, one (alpha, rho, sigma) per COLUMN.
+# All G LMLs and gradients in one call; list(lml = G, grad = 3 x G, info = G)
+gp_lml_grad_groups <- function(x_list, y_list, theta, jitter = 0)
+  .Call("gp_lml_grad_groups", as.list(x_list), as.list(y_list), as.matrix(theta), jitter)
+
 # ---- GP observed through derivatives (the Stan model inside gpderivs.py:25-133; design_notes.Rmd:25-46) ----
 # theta: (2 + nblocks) x B matrix, columns (alpha, rho, noise_1..noise_nblocks); y = c(y, yp, ypp) stacked
 gp_lml_grad_deriv_draws <- function(t, y, theta, order0 = 0L, jitter = 0)

@@ -24,6 +24,7 @@ SEXP Rf_allocVector(int, R_xlen_t);
 SEXP Rf_duplicate(SEXP);
 SEXP Rf_coerceVector(SEXP, int);
 int Rf_isNull(SEXP);
+int TYPEOF(SEXP);
 SEXP Rf_mkChar(const char *);
 SEXP Rf_setAttrib(SEXP, SEXP, SEXP);
 SEXP VECTOR_ELT(SEXP, R_xlen_t);

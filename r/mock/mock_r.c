@@ -93,6 +93,7 @@ int *INTEGER(SEXP s) {
   return (int *)s->data;
 }
 int Rf_isNull(SEXP s) { return s == R_NilValue || s->type == NILSXP; }
+int TYPEOF(SEXP s) { return s->type; }
 int Rf_nrows(SEXP s) { return s->nrow >= 0 ? s->nrow : (int)s->len; }
 int Rf_ncols(SEXP s) { return s->ncol >= 0 ? s->ncol : 1; }
 

@@ -312,6 +312,48 @@ SEXP gp_lml_grad_draws(SEXP x_, SEXP y_, SEXP theta_, SEXP jitter) {
   return out;
 }
 
+/* LML + gradient of one GP per group, groups of different sizes (per-player GPs, multiple_players.stan:59-63):
+ * x_list, y_list are lists of B numeric vectors (group b has length(x_list[[b]]) >= 1 points), theta a 3 x B matrix
+ * (alpha, rho, sigma per column); returns list(lml =, grad = 3 x B, info =) */
+SEXP gp_lml_grad_groups(SEXP xl, SEXP yl, SEXP theta_, SEXP jitter) {
+  int np = 0;
+  if (TYPEOF(xl) != VECSXP || TYPEOF(yl) != VECSXP)
+    Rf_error("gp_lml_grad_groups: x_list and y_list must be lists of numeric vectors, one per group");
+  const int B = LENGTH(xl);
+  if (LENGTH(yl) != B) Rf_error("gp_lml_grad_groups: length(y_list) = %d must equal length(x_list) = %d", LENGTH(yl), B);
+  SEXP theta = as_real(theta_, &np, "theta");
+  if (Rf_nrows(theta) != 3 || Rf_ncols(theta) != B)
+    Rf_error("gp_lml_grad_groups: theta must be a 3 x B matrix, one (alpha, rho, sigma) per COLUMN, B = length(x_list) = %d "
+             "(got %d x %d)", B, Rf_nrows(theta), Rf_ncols(theta));
+  long long *off = (long long *)R_alloc((size_t)B + 1, sizeof(long long));
+  off[0] = 0;
+  for (int b = 0; b < B; b++) {
+    const int nx = LENGTH(VECTOR_ELT(xl, b)), ny = LENGTH(VECTOR_ELT(yl, b));
+    if (nx < 1) Rf_error("gp_lml_grad_groups: x_list[[%d]] is empty (every group needs at least one point)", b + 1);
+    if (ny != nx) Rf_error("gp_lml_grad_groups: length(y_list[[%d]]) = %d must equal length(x_list[[%d]]) = %d", b + 1, ny, b + 1, nx);
+    off[b + 1] = off[b] + nx;
+  }
+  double *x = (double *)R_alloc((size_t)off[B], sizeof(double)), *y = (double *)R_alloc((size_t)off[B], sizeof(double));
+  for (int b = 0; b < B; b++) {  /* coerced one group at a time: the PROTECT stack stays flat for any number of groups */
+    int k = 0;
+    SEXP xb = as_real(VECTOR_ELT(xl, b), &k, "x_list[[b]]"), yb = as_real(VECTOR_ELT(yl, b), &k, "y_list[[b]]");
+    memcpy(x + off[b], REAL(xb), sizeof(double) * (size_t)(off[b + 1] - off[b]));
+    memcpy(y + off[b], REAL(yb), sizeof(double) * (size_t)(off[b + 1] - off[b]));
+    UNPROTECT(k);
+  }
+  SEXP lml = PROTECT(Rf_allocVector(REALSXP, B));
+  SEXP grad = PROTECT(Rf_allocMatrix(REALSXP, 3, B));
+  SEXP info = PROTECT(Rf_allocVector(INTSXP, B));
+  np += 3;
+  check(gpb200_lml_grad_ragged(handle(), B, off, x, y, REAL(theta), Rf_asReal(jitter), 1, REAL(lml), REAL(grad),
+                               INTEGER(info)), "lml_grad_groups");
+  SEXP elts[3] = {lml, grad, info};
+  static const char *const names[3] = {"lml", "grad", "info"};
+  SEXP out = named_list(3, elts, names);
+  UNPROTECT(np);
+  return out;
+}
+
 /* LML + gradient for B draws with the ARD covariance (QQard of R/kernels.R:19) on the n x D matrix X (1 <= D <= 8):
  * theta is a (D + 2) x B matrix (alpha, rho_1 .. rho_D, sigma per column), grad has the same layout */
 SEXP gp_lml_grad_ard_draws(SEXP X_, SEXP y_, SEXP theta_, SEXP jitter) {
@@ -514,6 +556,7 @@ static const R_CallMethodDef call_methods[] = {
     {"gp_gram_ard", (DL_FUNC)&gp_gram_ard, 4},         {"gp_gram_deriv", (DL_FUNC)&gp_gram_deriv, 7},
     {"gp_potrf", (DL_FUNC)&gp_potrf, 1},               {"gp_potrs", (DL_FUNC)&gp_potrs, 2},
     {"gp_lml_grad_draws", (DL_FUNC)&gp_lml_grad_draws, 4}, {"gp_lml_grad_ard_draws", (DL_FUNC)&gp_lml_grad_ard_draws, 4},
+    {"gp_lml_grad_groups", (DL_FUNC)&gp_lml_grad_groups, 4},
     {"gp_condition", (DL_FUNC)&gp_condition, 6},       {"gp_cond_mvn", (DL_FUNC)&gp_cond_mvn, 4},
     {"gp_rbf_cov_chol_grid", (DL_FUNC)&gp_rbf_cov_chol_grid, 2}, {"gp_approx_L_basis", (DL_FUNC)&gp_approx_L_basis, 5},
     {"gp_se_chol_tangent", (DL_FUNC)&gp_se_chol_tangent, 5},

@@ -171,3 +171,85 @@ inline double gp_lml_joint(const Eigen::Matrix<double, Eigen::Dynamic, 1>& t,
   gpb200_stan::eval_joint(t, y_stack, alpha, rho, noise.data(), (int)noise.size(), lml, nullptr);
   return lml;
 }
+
+// ---- one GP per group, groups of different sizes: the per-player GPs of multiple_players.stan:59-63, all groups'
+// LMLs and gradients in one call at every leapfrog step.  x and y hold the groups one after the other, sizes[g] >= 1
+// points each (sum(sizes) == size(x) == rows(y)); alpha, rho, sigma hold one entry per group:
+//
+//   functions { real gp_lml_groups(real[] x, vector y, int[] sizes, vector alpha, vector rho, vector sigma); }
+//   model     { target += gp_lml_groups(x, y, sizes, alpha, rho, sigma); ... priors ... }
+//
+// Returns sum_g lml_g (with constants) with a partial for every group's three parameters; a group whose covariance
+// is not positive definite throws std::domain_error, so NUTS rejects the proposal.
+namespace gpb200_stan {
+inline void eval_groups(const std::vector<double>& x, const Eigen::VectorXd& y, const std::vector<int>& sizes,
+                        const std::vector<double>& theta, double& total, std::vector<double>* grad) {
+  const int G = (int)sizes.size();
+  if ((int)theta.size() != 3 * G) throw std::domain_error("gp_lml_groups: alpha, rho and sigma need one entry per group");
+  std::vector<long long> off(G + 1, 0);
+  for (int g = 0; g < G; g++) {
+    if (sizes[g] < 1) throw std::domain_error("gp_lml_groups: every group size must be >= 1");
+    off[g + 1] = off[g] + sizes[g];
+  }
+  if (off[G] != (long long)x.size() || off[G] != (long long)y.size())
+    throw std::domain_error("gp_lml_groups: sum(sizes) must equal the length of x and of y");
+  total = 0.0;
+  if (G == 0) return;
+  std::vector<double> lml(G), g3(3 * G);
+  std::vector<int> info(G);
+  const int rc = gpb200_lml_grad_ragged(handle(), G, off.data(), x.data(), y.data(), theta.data(), 0.0, grad != nullptr,
+                                        lml.data(), g3.data(), info.data());
+  if (rc < 0) throw std::runtime_error(std::string("gp_lml_groups: ") + gpb200_last_error(handle()));
+  for (int g = 0; g < G; g++)
+    if (info[g] > 0)
+      throw std::domain_error("gp_lml_groups: covariance of group " + std::to_string(g + 1) + " is not positive definite (pivot " +
+                              std::to_string(info[g]) + ")");
+  for (int g = 0; g < G; g++) total += lml[g];
+  if (grad) *grad = g3;
+}
+}  // namespace gpb200_stan
+
+template <typename T0__, typename T1__, typename T2__>
+typename boost::math::tools::promote_args<T0__, T1__, T2__>::type
+gp_lml_groups(const std::vector<double>& x, const Eigen::Matrix<double, Eigen::Dynamic, 1>& y, const std::vector<int>& sizes,
+              const Eigen::Matrix<T0__, Eigen::Dynamic, 1>& alpha, const Eigen::Matrix<T1__, Eigen::Dynamic, 1>& rho,
+              const Eigen::Matrix<T2__, Eigen::Dynamic, 1>& sigma, std::ostream* pstream__) {
+  using stan::math::value_of;
+  const int G = (int)sizes.size();
+  if (alpha.size() != G || rho.size() != G || sigma.size() != G)
+    throw std::domain_error("gp_lml_groups: alpha, rho and sigma need one entry per group");
+  std::vector<double> theta(3 * G), grad;
+  for (int g = 0; g < G; g++) {
+    theta[3 * g] = value_of(alpha.data()[g]);
+    theta[3 * g + 1] = value_of(rho.data()[g]);
+    theta[3 * g + 2] = value_of(sigma.data()[g]);
+  }
+  double total;
+  gpb200_stan::eval_groups(x, y, sizes, theta, total, &grad);
+  std::vector<stan::math::var> operands;
+  std::vector<double> partials;
+  for (int g = 0; g < G; g++) {
+    gpb200_stan::add_operand(operands, partials, alpha.data()[g], grad[3 * g]);
+    gpb200_stan::add_operand(operands, partials, rho.data()[g], grad[3 * g + 1]);
+    gpb200_stan::add_operand(operands, partials, sigma.data()[g], grad[3 * g + 2]);
+  }
+  return stan::math::precomputed_gradients(total, operands, partials);
+}
+
+inline double gp_lml_groups(const std::vector<double>& x, const Eigen::Matrix<double, Eigen::Dynamic, 1>& y,
+                            const std::vector<int>& sizes, const Eigen::Matrix<double, Eigen::Dynamic, 1>& alpha,
+                            const Eigen::Matrix<double, Eigen::Dynamic, 1>& rho,
+                            const Eigen::Matrix<double, Eigen::Dynamic, 1>& sigma, std::ostream* pstream__) {
+  const int G = (int)sizes.size();
+  if (alpha.size() != G || rho.size() != G || sigma.size() != G)
+    throw std::domain_error("gp_lml_groups: alpha, rho and sigma need one entry per group");
+  std::vector<double> theta(3 * G);
+  for (int g = 0; g < G; g++) {
+    theta[3 * g] = alpha.data()[g];
+    theta[3 * g + 1] = rho.data()[g];
+    theta[3 * g + 2] = sigma.data()[g];
+  }
+  double total;
+  gpb200_stan::eval_groups(x, y, sizes, theta, total, nullptr);
+  return total;
+}
