@@ -41,7 +41,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
     return launch_lml_small(h, n, x, x_stride, y, y_stride, theta, jitter, want_grad, lml, grad, info, B);
   }
   const int zks = trmv_split_chunks(np, B);  // k-chunks of the split z = W y (small batches only)
-  // SE covariance: the tile envelope of every item (F, E; solve.cu) bounds the Cholesky, and larger batches compute the
+  // SE covariance: the envelope of every item (common.cuh, ENV_BLK) bounds the Cholesky, and larger batches compute the
   // gradient from the selected inverse instead of the explicit inverse + W^T W.  Measured on a B200 (1000 W), LML +
   // gradient per call on the bench.py family, dense / envelope + explicit inverse / envelope + selected inverse, ms:
   //   N = 1024: B = 1 0.452 / 0.458 / 0.85,  B = 32 2.10 / 1.98 / 2.12   (nt = 8: the band covers the matrix, the
@@ -52,7 +52,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
   const bool use_env = !sp.deriv && !ard && h->envelope && !small && nt >= 16 && nt <= ENV_MAX_NT;
   const bool sinv = use_env && want_grad && (h->sinv_min_batch > 0 ? B >= h->sinv_min_batch : (long long)B * nt >= 256);
   const size_t per_item = small ? 0 : pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * pw * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) + 64 +
-                                      (use_env ? (size_t)(2 * nt + 2) * sizeof(int) : 0);
+                                      (use_env ? (size_t)(env_record_ints(nt) + 2) * sizeof(int) : 0);
   const size_t fixed = pad256((size_t)B * (x_stride ? xl : 0) * 8 + (size_t)xl * 8) + pad256((size_t)B * (y_stride ? n : 0) * 8 + n * 8) +
                        2 * pad256((size_t)B * ts * 8) + pad256((size_t)B * 8) + pad256((size_t)B * 4) + 4096 + (use_env ? 512 : 0);
   int Bc = B;
@@ -83,7 +83,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
     zbuf = a.take<double>((size_t)Bc * np); abuf = a.take<double>((size_t)Bc * np); dvec = a.take<double>((size_t)Bc * np);
     partial = a.take<double>((size_t)Bc * nparts * pw);
     zpart = zks > 1 ? a.take<double>((size_t)Bc * zks * np) : nullptr;
-    if (use_env && (!(env = a.take<int>((size_t)Bc * 2 * nt)) || !(order = a.take<int>((size_t)Bc * 2))))
+    if (use_env && (!(env = a.take<int>((size_t)Bc * env_record_ints(nt))) || !(order = a.take<int>((size_t)Bc * 2))))
       BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
     if (!partial) BAD_ARG(h, 1002, "lml_grad_batched: workspace arithmetic error");
   }
@@ -99,7 +99,7 @@ int lml_core(gpb200_handle_t h, const LmlSpec &sp, int B, const double *x, long 
       if (sp.deriv) RC(launch_gram_deriv_batched(h, ng, sp.order0, sp.nblocks, np, cx, xs, cth, ts, jitter, 1, Lbuf, mat, bc));
       else if (ard) RC(launch_gram_ard_batched(h, n, sp.ard_d, np, cx, xs, cth, jitter, Lbuf, mat, bc));
       else {
-        if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
+        if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0xff, (size_t)bc * env_record_ints(nt) * sizeof(int), h->stream));  // fb UINT_MAX, er -1
         RC(launch_gram_se_batched(h, n, np, cx, xs, cth, jitter, 1, Lbuf, mat, bc, env));
         if (env) RC(launch_envelope_profile(h, nt, env, order, bc));
       }
@@ -267,7 +267,7 @@ struct RaggedBucket {
 size_t se_item_bytes(int np, int nparts, int zks, bool use_env) {
   const long long mat = (long long)np * np;
   return pad256(mat * 8) * 2 + 3 * pad256(np * 8) + pad256((size_t)nparts * 4 * 8) + (zks > 1 ? pad256((size_t)zks * np * 8) : 0) +
-         64 + (use_env ? (size_t)(2 * (np / TILE) + 2) * sizeof(int) : 0);
+         64 + (use_env ? (size_t)(env_record_ints(np / TILE) + 2) * sizeof(int) : 0);
 }
 }  // namespace
 
@@ -407,14 +407,14 @@ extern "C" int gpb200_lml_grad_ragged(gpb200_handle_t h, int B, const long long 
     double *partial = ab.take<double>((size_t)r.Bc * r.ntasks * 4 * 4);
     double *zpart = r.zks > 1 ? ab.take<double>((size_t)r.Bc * r.zks * np) : nullptr;
     int *env = nullptr, *order = nullptr;
-    if (r.use_env && (!(env = ab.take<int>((size_t)r.Bc * 2 * nt)) || !(order = ab.take<int>((size_t)r.Bc * 2))))
+    if (r.use_env && (!(env = ab.take<int>((size_t)r.Bc * env_record_ints(nt))) || !(order = ab.take<int>((size_t)r.Bc * 2))))
       BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
     if (!partial || (r.zks > 1 && !zpart)) BAD_ARG(h, 1002, "lml_grad_ragged: workspace arithmetic error");
     for (int b0 = 0; b0 < K.count; b0 += r.Bc) {
       const int bc = std::min(r.Bc, K.count - b0);
       const double *ccx = bx + (long long)b0 * np, *ccy = by + (long long)b0 * np, *cct = bth + 3LL * b0;
       const int *cnv = bnv + b0;
-      if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0x7f, (size_t)bc * 2 * nt * sizeof(int), h->stream));  // F = "no tile yet"
+      if (env) GPB_CUDA(h, cudaMemsetAsync(env, 0xff, (size_t)bc * env_record_ints(nt) * sizeof(int), h->stream));  // fb UINT_MAX, er -1
       RC(launch_gram_se_batched(h, np, np, ccx, np, cct, jitter, 1, Lbuf, mat, bc, env, cnv));
       if (env) RC(launch_envelope_profile(h, nt, env, order, bc));
       RC(chol_batched(h, Lbuf, np, mat, np, bc, binfo + b0, env, order));  // padded pivots are 1: info stays within n_b

@@ -11,7 +11,15 @@ namespace gpb {
 
 constexpr int PANEL_FUSED_MAX_BATCH = 148;  // matrices per panel_fused_kernel launch (flag slots in the handle)
 constexpr int TILE = 128;  // tile edge of every tiled algorithm (internal matrices are padded to it)
-constexpr int ENV_MAX_NT = 512;  // tile rows of a matrix with a tile envelope (the GEMM stages one half of it in shared memory)
+constexpr int ENV_MAX_NT = 512;  // tile rows of a matrix with a tile envelope (the GEMM stages one part of it in shared memory)
+// Envelope record of one item of the SE route, ints at these offsets (nt tile rows):
+//   F  [0, nt)      first tile column of each tile row that holds a nonzero (F_I <= I)
+//   E  [nt, 2nt)    per tile column J, the last tile row I with F_I <= J
+//   fb [2nt, 4nt)   per 64-row block, the first column any of its rows has a nonzero in (the element profile)
+//   er [4nt, 5nt)   per tile column J, the last row with a nonzero in column 128 J + 127 or left of it (E_J = er_J / 128)
+// "Nonzero": exp(-d^2 / 2 rho^2) not exactly zero, NaN included, and every diagonal element.
+constexpr int ENV_BLK = 64;  // rows per fb block: the smallest CTA extent of the tile GEMM
+__host__ __device__ constexpr int env_record_ints(int nt) { return 5 * nt; }
 
 inline int round_up(int n, int m) { return (n + m - 1) / m * m; }
 
@@ -62,8 +70,7 @@ struct GemmParams {
   // n_grid x n_grid; block b carries derivative order order0 + b; theta is B x theta_stride
   int n_grid, order0, theta_stride;
   int latency_hint;   // 1: this launch sits on a dependent chain (look-ahead Cholesky): small launches take the 16-warp fine tiles
-  // tile envelope of a banded covariance (ENV_* below): per item env[0..nt) = F (first nonzero tile column of each
-  // tile row), env[nt..2nt) = E (last tile row I with F_I <= J, per tile column J); item stride 2 * env_nt
+  // envelope of a banded covariance (ENV_* below): the records of env_record_ints(env_nt) ints per item
   const int *env;
   int env_nt, env_mode;
   const int *order;             // envelope launches: item of blockIdx.y (envelope_order_kernel); nullptr: blockIdx.y itself
@@ -72,11 +79,15 @@ struct GemmParams {
   int ard_d;                    // EPI_TRACE_ARD: input dimensions D (x is n x D column-major per item, theta_stride = D + 2)
   const int *nvec;              // EPI_TRACE_RAGGED: per-item sizes (the mask of item b is nvec[b] instead of n)
 };
-// envelope modes of the tile GEMM.  Only products with an exactly-zero operand tile are dropped, and the k order of
-// the rest is kept, so a result is bit-identical to the dense launch (up to the sign of an all-zero tile).
+// envelope modes of the tile GEMM.  Only products with an exactly-zero operand are dropped, and the k order of the rest
+// is kept, so a result is bit-identical to the dense launch (up to the sign of an all-zero tile).  The bounds move in
+// 16-wide k-chunks (KC), so every DMMA that remains reads the same k as in the dense launch.
 enum { ENV_NONE = 0,
-       ENV_CHOL = 1,   // C(I,J) -= L(I,k) L(J,k)^T: exit when J < F_I (tile outside the profile), k starts at max(F_I, F_J)
-       ENV_BAND = 2 }; // selected inverse: exit when I > E_J, the contraction ends at tile E_J
+       ENV_CHOL = 1,       // C(I,J) -= L(I,k) L(J,k)^T: exit when J < F_I (tile outside the profile), k starts at max(F_I, F_J)
+       ENV_CHOL_FINE = 2,  // the same update, k starts at the first column where a row of this CTA's A and one of its B
+                           // can both be nonzero (fb over the CTA's rows and over its columns, rounded down to 16)
+       ENV_BAND = 3 };     // selected inverse: exit when I > E_J; row k of Y[S,J] = L[S,J] W_JJ is zero past er_J, so the
+                           // contraction ends at er_J + 1 rounded up to 16
 
 // Tile envelope of the batched TRSM below diagonal tile `col` (the throughput TRSM kernels of panel.cu): F points at the
 // F entry of the first row tile of item 0, item stride `stride`.  Row tile r (counted from the first) is live when
@@ -247,12 +258,12 @@ int launch_trsm_tiles_at(Handle *h, double *L, long long ld, long long stride, l
 // latency path, otherwise the two launches above (whose TRSM solves only the tiles live under `env`)
 int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, long long diag_off, int index_base, int n,
                          long long c_off, int ntiles, int batch, int *info, TrsmEnv env = TrsmEnv{});
-// env: the tile envelope of each item (F, E with item stride 2 * ld / TILE, see GemmParams), or nullptr
+// env: the envelope record of each item (env_record_ints(ld / TILE) ints, see ENV_BLK), or nullptr
 int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int tile_col, int ntiles_below, int n, int batch,
                       int *info, const int *env = nullptr);
 int launch_tile_inverse_at(Handle *h, const double *L, long long ld, long long l_off, long long l_step, double *W,
                            long long w_off, long long w_step, long long stride, int ntiles, int batch);
-// tile envelope of the SE path (solve.cu): E from F (F filled by gram_se_batched), the trace of the selected inverse
+// tile envelope of the SE path (solve.cu): F, E and er from the element profile gram_se_batched records, the trace of the selected inverse
 // and the band-limited back substitution.  launch_envelope_profile also writes the dispatch order of the envelope GEMM
 // launches to order[0..batch) (order[batch..2 batch) is its scratch)
 int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch);

@@ -172,9 +172,10 @@ static void set_env(GemmParams &p, const int *env, const int *order, int nt, int
   p.env_mode = env ? mode : ENV_NONE;
 }
 
-// Batched tiled Cholesky, in place on Lbuf (np x np per item, lower tiles valid on entry).  With a tile envelope
-// (env, see ENV_CHOL) every update CTA starts its contraction at the first tile where both operand rows can be nonzero
-// and exits when its output tile lies left of the profile: L is bit-identical to the dense factorisation.
+// Batched tiled Cholesky, in place on Lbuf (np x np per item, lower tiles valid on entry).  With an envelope (env, see
+// ENV_CHOL_FINE) every update CTA starts its contraction at the first 16-column chunk where a row of both its operands
+// can be nonzero and exits when nothing is left: L is bit-identical to the dense factorisation.  The look-ahead
+// schedule keeps the tile rule (ENV_CHOL): its launches are bound by the panel chain, not by their flops.
 // Panel width: pure left-looking when the batch alone fills the GPU, 8-tile (1024-column) panels
 // with right-looking trailing updates otherwise.
 int chol_panel_tiles(int nt, int batch) {
@@ -294,7 +295,7 @@ int chol_batched(Handle *h, double *Lbuf, int np, long long stride, int n, int b
   p.C0 = mref(Lbuf, np, stride);
   p.alpha = -1.0;
   p.beta = 1.0;
-  set_env(p, env, order, nt, ENV_CHOL);
+  set_env(p, env, order, nt, ENV_CHOL_FINE);
   for (int j = 0; j < nt; j++) {
     if (tl.count(j) > 0) {
       p.tasks = tl.at(j);
@@ -352,7 +353,8 @@ int trtri_batched(Handle *h, double *Lbuf, double *Sbuf, int np, long long strid
 // J <= I <= E_J, which hold every tile where the SE covariance or its derivatives are nonzero.  With Y = L W
 // (W_JJ = L_JJ^-1, the block column scaled by its diagonal inverse) and S = J+1..E_J:
 //   Z[S,J] = -Z[S,S] Y[S,J],    Z[J,J] = W_JJ^T W_JJ - Y[S,J]^T Z[S,J]
-// For K in S, E_K >= E_J, so every Z[S,S] tile the contraction reads was produced by an earlier step.
+// For K in S, E_K >= E_J, so every Z[S,S] tile the contraction reads was produced by an earlier step.  Rows of Y[S,J]
+// past er_J are zero (ENV_BAND), so both contractions end there.
 //   Y    all block columns in one launch (Sbuf, lower tiles)
 //   D    W_JJ^T W_JJ over the diagonal tiles of Lbuf (full tiles)
 //   per J from the last: Z[S,J] into Lbuf (lower tiles) and its transpose into the upper tiles, so that Z[S,S] is

@@ -9,13 +9,16 @@
   extern __shared__ __align__(16) double smem[];
   constexpr int TM = Cfg::TM, LD_MC = Cfg::LD_MC_A;
   TileTask task = p.tasks[blockIdx.x / Cfg::NSPLIT];
-  // the half of the item's envelope this launch uses (F for ENV_CHOL, E for ENV_BAND), read beside the task rather
-  // than after it: on the dependent chain of the look-ahead Cholesky a second dependent load is a visible latency
-  __shared__ int s_env[ENV_MAX_NT];
+  // the part of the item's envelope record this launch uses (F for ENV_CHOL, fb for ENV_CHOL_FINE, er for ENV_BAND),
+  // read beside the task rather than after it: on the dependent chain of the look-ahead Cholesky a second dependent
+  // load is a visible latency
+  __shared__ int s_env[2 * ENV_MAX_NT];
   const long long b = p.order ? p.order[blockIdx.y] : blockIdx.y;  // the batch item
   if (p.env_mode != ENV_NONE) {
-    const int *src = p.env + b * 2 * p.env_nt + (p.env_mode == ENV_CHOL ? 0 : p.env_nt);
-    for (int q = threadIdx.x; q < p.env_nt; q += Cfg::NTHREADS) s_env[q] = src[q];
+    const int nt = p.env_nt;
+    const int *src = p.env + b * env_record_ints(nt) + (p.env_mode == ENV_CHOL ? 0 : (p.env_mode == ENV_CHOL_FINE ? 2 * nt : 4 * nt));
+    const int cnt = p.env_mode == ENV_CHOL_FINE ? 2 * nt : nt;
+    for (int q = threadIdx.x; q < cnt; q += Cfg::NTHREADS) s_env[q] = src[q];
     __syncthreads();
   }
   const int split = (Cfg::NSPLIT > 1) ? (int)(blockIdx.x % Cfg::NSPLIT) : 0;
@@ -42,24 +45,32 @@
     if (skip_last) task.k_len -= TILE / 2;
     if (sym_skip) task.k_len = 0;
   }
-  if (p.env_mode != ENV_NONE) {  // the item's tile envelope: leave out the contraction over exactly-zero operand tiles
-    const int *F = s_env, *E = s_env;
+  if (p.env_mode != ENV_NONE) {  // the item's envelope: leave out the contraction over exactly-zero operand rows
     const int ti = task.c_r / TILE, tj = task.c_c / TILE;
     int k0 = A_KC ? task.a_r : task.a_c, k1 = k0 + task.k_len;
-    bool out;
+    bool out = false;
     if (p.env_mode == ENV_CHOL) {
+      const int *F = s_env;
       out = tj < F[ti];
       k0 = max(k0, max(F[ti], F[tj]) * TILE);
+    } else if (p.env_mode == ENV_CHOL_FINE) {
+      // A is L(rows of C, :) and B is L(columns of C, :): a CTA whose C block lies left of the profile ends with k_len 0
+      const int *fb = s_env;
+      int ka = fb[task.c_r / ENV_BLK], kb = fb[task.c_c / ENV_BLK];
+      if (TM > ENV_BLK) ka = min(ka, fb[task.c_r / ENV_BLK + 1]);
+      if (TN > ENV_BLK) kb = min(kb, fb[task.c_c / ENV_BLK + 1]);
+      k0 = max(k0, max(ka, kb) & ~(KC - 1));
     } else {
-      out = ti > E[tj];
-      k1 = min(k1, (E[tj] + 1) * TILE);
+      const int er = s_env[tj];
+      out = ti > er / TILE;
+      k1 = min(k1, (er + KC) & ~(KC - 1));
     }
     const int shift = k0 - (A_KC ? task.a_r : task.a_c);
     if (A_KC) task.a_r += shift; else task.a_c += shift;
     if (B_KC) task.b_r += shift; else task.b_c += shift;
     task.k_len = max(k1 - k0, 0);
     // an update of the factor in place with nothing left to add leaves C as it is
-    if (out || (p.env_mode == ENV_CHOL && task.k_len == 0)) {
+    if (out || (p.env_mode != ENV_BAND && task.k_len == 0)) {
       if (EPI != EPI_AXPBY && threadIdx.x < epi_partial_width(EPI))
         p.partial[((long long)b * gridDim.x + blockIdx.x) * epi_partial_width(EPI) + threadIdx.x] = 0.0;
       return;

@@ -73,19 +73,31 @@ __global__ void __launch_bounds__(256) gram_outer_kernel(int kind, int n, int m,
 // Internal layout: np x np (np multiple of 128) per item, identity in the padding so that the
 // padded factor is [L 0; 0 I].  Only tiles with tile_row >= tile_col are produced when lower_only.
 // RAGGED: item b has its own size nvec[b] <= np (gpb200_lml_grad_ragged), identity beyond it.
+// Element profile for the envelope record (common.cuh, ENV_BLK) of item b: fcol / lrow are the first nonzero column
+// and the last nonzero row among this thread's elements of tile (tr, tc) (INT_MAX / -1: none).  Warp w holds the rows of
+// 64-row block (w & 1) of the tile row (rl = 2 (tid & 63)).
+__device__ __forceinline__ void record_profile(int *rec, int nt, int tr, int tc, int fcol, int lrow) {
+  const unsigned fw = __reduce_min_sync(0xffffffffu, (unsigned)fcol);
+  const int lw = __reduce_max_sync(0xffffffffu, lrow);
+  if ((threadIdx.x & 31) == 0) {
+    if (fw != (unsigned)INT_MAX) atomicMin(reinterpret_cast<unsigned *>(rec + 2 * nt) + 2 * tr + ((threadIdx.x >> 5) & 1), fw);
+    if (lw >= 0) atomicMax(rec + 4 * nt + tc, lw);
+  }
+}
+
 template <bool RAGGED>
 __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n_all, int np, const double *__restrict__ x,
                                                              long long x_stride, const double *__restrict__ theta,
                                                              double jitter, int lower_only,
                                                              double *__restrict__ K, long long stride,
-                                                             int *__restrict__ envF, const int *__restrict__ nvec) {
+                                                             int *__restrict__ env, const int *__restrict__ nvec) {
   const int nt = np / TILE;
   const int tr = blockIdx.x % nt, tc = blockIdx.x / nt;
   if (lower_only && tr < tc) return;
   const int n = RAGGED ? nvec[blockIdx.y] : n_all;
-  // envF (optional, item stride 2 nt, preset to INT_MAX per tile row): the first tile column of each tile row whose exp(-d^2/2rho^2) is
-  // not exactly zero somewhere (NaN counts as nonzero).  That set holds the support of K and of dK/dtheta.
-  bool nz = tr == tc;
+  // env (optional, records of env_record_ints(nt) ints, fb preset to UINT_MAX and er to -1): the element profile of the
+  // tile, where an element is nonzero when its exp(-d^2/2rho^2) is not exactly zero (NaN counts) or it is on the
+  // diagonal.  That set holds the support of K and of dK/dtheta, and the diagonal of the identity padding.
   __shared__ double xs[TILE], ys[TILE];
   const long long b = blockIdx.y;
   const double *xb = x + b * x_stride;
@@ -97,20 +109,29 @@ __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n_all, int np,
   const double a2 = alpha * alpha, nh = -0.5 / (rho * rho), dadd = sigma * sigma + jitter;
   double *Kb = K + b * stride;
   const int rl = 2 * (tid & 63), cq = tid >> 6;
+  int fcol = INT_MAX, lrow = -1;
   if (tr != tc && r0 + TILE <= n && c0 + TILE <= n) {
     // interior off-diagonal tile (all but O(nt) of the nt^2/2 tiles): no masks, no diagonal
     const double x0 = xs[rl], x1 = xs[rl + 1];
     double *dst = Kb + (r0 + rl) + (long long)(c0 + cq) * np;
+    int s0 = 32;  // the first column step with a nonzero
+    bool nz0 = false, nz1 = false;
 #pragma unroll 4
     for (int s = 0; s < 32; s++) {
       const double yc = ys[cq + 4 * s];
       const double d0 = x0 - yc, d1 = x1 - yc;
       const double e0 = exp_nonpos(d0 * d0 * nh), e1 = exp_nonpos(d1 * d1 * nh);
-      nz |= e0 != 0.0 || e1 != 0.0;
+      nz0 |= e0 != 0.0;
+      nz1 |= e1 != 0.0;
+      s0 = min(s0, (e0 != 0.0 || e1 != 0.0) ? s : 32);
       *reinterpret_cast<double2 *>(dst) = make_double2(a2 * e0, a2 * e1);
       dst += 4LL * np;
     }
-    if (envF && __syncthreads_or(nz) && tid == 0) atomicMin(envF + b * 2 * nt + tr, tc);
+    if (env) {
+      if (s0 < 32) fcol = c0 + cq + 4 * s0;
+      lrow = nz1 ? r0 + rl + 1 : (nz0 ? r0 + rl : -1);
+      record_profile(env + b * env_record_ints(nt), nt, tr, tc, fcol, lrow);
+    }
     return;
   }
 #pragma unroll 2
@@ -121,6 +142,7 @@ __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n_all, int np,
 #pragma unroll
     for (int e = 0; e < 2; e++) {
       const int i = r0 + rl + e;
+      bool nz = i == j;
       if (i < n && j < n) {
         const double d = xs[rl + e] - ys[cl];
         const double ek = exp_nonpos(d * d * nh);
@@ -129,10 +151,14 @@ __global__ void __launch_bounds__(256) gram_se_batched_kernel(int n_all, int np,
       } else {
         v[e] = (i == j) ? 1.0 : 0.0;
       }
+      if (nz) {
+        fcol = min(fcol, j);
+        lrow = max(lrow, i);
+      }
     }
     *reinterpret_cast<double2 *>(Kb + (r0 + rl) + (long long)j * np) = make_double2(v[0], v[1]);
   }
-  if (envF && __syncthreads_or(nz) && tid == 0) atomicMin(envF + b * 2 * nt + tr, tc);
+  if (env) record_profile(env + b * env_record_ints(nt), nt, tr, tc, fcol, lrow);
 }
 
 // ---- block-column panel of the padded SE Gram for the block-cyclic multi-GPU Cholesky ----------
@@ -541,15 +567,15 @@ int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const 
 }
 
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF,
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *env,
                            const int *nvec) {
   const int nt = np / TILE;
   dim3 grid(nt * nt, batch);
   ProfScope ps__(h, PC_GRAM);
   if (nvec)
-    gram_se_batched_kernel<true><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF, nvec);
+    gram_se_batched_kernel<true><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, env, nvec);
   else
-    gram_se_batched_kernel<false><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, envF,
+    gram_se_batched_kernel<false><<<grid, 256, 0, h->stream>>>(n, np, x, x_stride, theta, jitter, lower_only, K, stride, env,
                                                                nullptr);
   GPB_LAUNCH_CHECK(h);
   return 0;

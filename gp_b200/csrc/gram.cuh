@@ -11,7 +11,7 @@ int launch_kernel_eval(Handle *h, int kind, long long len, const double *tj, con
 int launch_gram_outer(Handle *h, int kind, int n, int m, const double *x, const double *y, double amp2, double l,
                       double *K, long long ldk);
 int launch_gram_se_batched(Handle *h, int n, int np, const double *x, long long x_stride, const double *theta,
-                           double jitter, int lower_only, double *K, long long stride, int batch, int *envF = nullptr,
+                           double jitter, int lower_only, double *K, long long stride, int batch, int *env = nullptr,
                            const int *nvec = nullptr);  // nvec: per-item sizes (device), nullptr = n for every item
 int launch_gram_tangent(Handle *h, int n, int np, const double *x, double alpha, const double *ls, double dadd, int mode,
                         double *S, double *Sdot, long long stride, int batch);

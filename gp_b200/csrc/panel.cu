@@ -1138,7 +1138,7 @@ int launch_potrf_trsm_at(Handle *h, double *L, long long ld, long long stride, l
 int launch_potrf_trsm(Handle *h, double *L, long long ld, long long stride, int tile_col, int ntiles_below, int n, int batch,
                       int *info, const int *env) {
   TrsmEnv te;
-  if (env) te = TrsmEnv{env + tile_col + 1, 2 * (int)(ld / TILE), tile_col};
+  if (env) te = TrsmEnv{env + tile_col + 1, env_record_ints((int)(ld / TILE)), tile_col};
   return launch_potrf_trsm_at(h, L, ld, stride, (long long)tile_col * TILE * (ld + 1), tile_col * TILE, n,
                               (long long)(tile_col + 1) * TILE + (long long)tile_col * TILE * ld, ntiles_below, batch, info, te);
 }

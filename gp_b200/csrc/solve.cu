@@ -152,7 +152,7 @@ __global__ void __launch_bounds__(TILE * TRSV_KSPLIT) trsv_blocked_kernel(int np
   for (int j = 0; j < nt; j++) {
     const int i = j * TILE + r;
     const int kmax = j * TILE;  // multiple of 128, so every group's strided range has the same length
-    const int kmin = env ? env[b * 2 * nt + j] * TILE : 0;
+    const int kmin = env ? env[b * env_record_ints(nt) + j] * TILE : 0;
     double s0 = 0.0, s1 = 0.0, s2 = 0.0, s3 = 0.0;
     const double *lp = Lb + i + (long long)(kmin + grp) * np;
     for (int k = kmin + grp; k < kmax; k += 4 * KS) {
@@ -538,22 +538,32 @@ int launch_trsv_sweep(Handle *h, int np, const double *L, const double *Wdiag, l
 }
 
 // ---- tile envelope of the SE covariance ------------------------------------------------------------------------------
-// env per item: F[0..nt) (first nonzero tile column of each tile row, filled by gram_se_batched; F_I <= I) and
-// E[0..nt): E_J = the last tile row I with F_I <= J.  F need not be monotone (x unsorted).  For K > J, E_K >= E_J,
-// which is what closes the selected-inverse recurrence over the contiguous range J+1..E_J.
+// The record of each item (common.cuh, ENV_BLK) from the element profile gram_se_batched left in it: fb (first nonzero
+// column per 64-row block) and, in er, per tile column the last row with a nonzero in it.  Here
+//   F_I = min(fb_2I, fb_2I+1) / 128,  E_J = the last tile row I with F_I <= J,  er_J = max over J' <= J of er_J'.
+// F need not be monotone (x unsorted).  For K > J, E_K >= E_J, which is what closes the selected-inverse recurrence
+// over the contiguous range J+1..E_J.  E_J = er_J / 128: both name the last row whose profile reaches column 128 J + 127.
 __global__ void __launch_bounds__(256) envelope_profile_kernel(int nt, int *__restrict__ env, int *__restrict__ band) {
-  extern __shared__ int sF[];
+  extern __shared__ int sF[];  // F, then the per-column last rows as recorded
+  int *sL = sF + nt;
   __shared__ int s_band;
-  int *F = env + (long long)blockIdx.x * 2 * nt, *E = F + nt;
+  int *F = env + (long long)blockIdx.x * env_record_ints(nt), *E = F + nt, *er = F + 4 * nt;
+  const unsigned *fb = reinterpret_cast<const unsigned *>(F + 2 * nt);
   if (threadIdx.x == 0) s_band = 0;
-  for (int i = threadIdx.x; i < nt; i += blockDim.x) sF[i] = min(F[i], i);
+  for (int i = threadIdx.x; i < nt; i += blockDim.x) {
+    sF[i] = min((int)(min(fb[2 * i], fb[2 * i + 1]) / TILE), i);
+    sL[i] = er[i];
+  }
   __syncthreads();
   for (int j = threadIdx.x; j < nt; j += blockDim.x) {
     int e = j;
     for (int i = nt - 1; i > j; i--)
       if (sF[i] <= j) { e = i; break; }
+    int last = sL[0];
+    for (int i = 1; i <= j; i++) last = max(last, sL[i]);
     F[j] = sF[j];
     E[j] = e;
+    er[j] = last;
     atomicMax(&s_band, j - sF[j]);
   }
   __syncthreads();
@@ -593,7 +603,7 @@ __global__ void __launch_bounds__(32) envelope_order_kernel(int nt, int batch, c
 int launch_envelope_profile(Handle *h, int nt, int *env, int *order, int batch) {
   ProfScope ps__(h, PC_OTHER);
   int *band = order + batch;
-  envelope_profile_kernel<<<batch, 256, nt * sizeof(int), h->stream>>>(nt, env, band);
+  envelope_profile_kernel<<<batch, 256, 2 * nt * sizeof(int), h->stream>>>(nt, env, band);
   GPB_LAUNCH_CHECK(h);
   envelope_order_kernel<<<1, 32, 0, h->stream>>>(nt, batch, band, order);
   GPB_LAUNCH_CHECK(h);
@@ -620,7 +630,7 @@ __global__ void __launch_bounds__(256) trace_sinv_kernel(int n_all, int np, cons
   while ((I + 1) * (I + 2) / 2 <= q) I++;
   const int J = q - I * (I + 1) / 2;
   double *o = partial + (b * gridDim.x + q) * 4;
-  if (J < env[b * 2 * nt + I]) {
+  if (J < env[b * env_record_ints(nt) + I]) {
     if (tid < 4) o[tid] = 0.0;
     return;
   }
@@ -688,7 +698,7 @@ __global__ void __launch_bounds__(1024) backsub_band_kernel(int np, const double
   const long long b = blockIdx.x;
   const int nt = np / TILE, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const double *Lb = L + b * stride, *Wb = Wdiag + b * stride, *zb = z + b * np;
-  const int *E = env + b * 2 * nt + nt;
+  const int *E = env + b * env_record_ints(nt) + nt;
   double *ab = a + b * np;
   for (int J = nt - 1; J >= 0; J--) {
     const int i0 = (J + 1) * TILE, i1 = (E[J] + 1) * TILE;
