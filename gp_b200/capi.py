@@ -76,6 +76,9 @@ SIGNATURES = {
     "gpb200_latent_forward": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_int, C.c_void_p, C.c_void_p]),
     "gpb200_latent_backward": (C.c_int, [_h, C.c_int, C.c_void_p, C.c_double, C.c_double, C.c_double, C.c_int, C.c_void_p,
                                          C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gpb200_latent_forward_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, _ll, C.c_void_p, C.c_double,
+                                                C.c_void_p, C.c_void_p, C.c_void_p]),
+    "gpb200_latent_backward_batched": (C.c_int, [_h, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]),
     "gpb200_approx_L": (C.c_int, [_h, C.c_int, C.c_double, C.c_int, C.c_void_p, C.POINTER(C.c_void_p),
                                   C.POINTER(C.c_void_p), C.c_void_p]),
     "gpb200_approx_Lz": (C.c_int, [_h, C.c_int, C.c_double, C.c_int, C.c_void_p, C.POINTER(C.c_void_p),
@@ -505,6 +508,56 @@ class Handle:
         self._check(self.lib.gpb200_latent_backward(self._h, n, _ptr(x), alpha, rho, diag_add, nvec, _ptr(z2), _ptr(fb), _ptr(tb),
                                                     _ptr(zbar)), "latent_backward")
         return tb, (zbar[0] if np.ndim(z) == 1 else zbar)
+
+    def latent_forward_batched(self, x, theta, diag_add, z):
+        """f_{b,m} = L_b z_{b,m} for B states at once, L_b = chol(cov_exp_quad(x_b, alpha_b, rho_b) + diag_add I).
+        x: (n,) shared or (B, n); theta: (B, 2) = (alpha, rho); z: (B, n) or (B, nvec, n).  Returns f (shaped like z) and
+        info (B,); failed items (info != 0) get NaN in f and do not raise.  The handle records the batch (factors and
+        copies of the inputs) for latent_backward_batched."""
+        th = np.ascontiguousarray(theta, dtype=np.float64)
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        z = np.asarray(z, dtype=np.float64)
+        if th.ndim != 2 or th.shape[1] != 2:
+            raise ValueError("theta must be (B, 2) = (alpha, rho) per row")
+        B = th.shape[0]
+        if z.ndim not in (2, 3) or z.shape[0] != B:
+            raise ValueError("z must be (B, n) or (B, nvec, n)")
+        n = z.shape[-1]
+        nvec = z.shape[1] if z.ndim == 3 else 1
+        if x.ndim not in (1, 2) or x.shape[-1] != n or (x.ndim == 2 and x.shape[0] != B):
+            raise ValueError("x must be (n,) or (B, n) with the n of z")
+        z3 = np.ascontiguousarray(z.reshape(B, nvec, n))
+        f = np.empty((B, nvec, n)); info = np.zeros(B, dtype=np.int32)
+        self._check(self.lib.gpb200_latent_forward_batched(self._h, n, B, nvec, _ptr(x), n if x.ndim == 2 else 0, _ptr(th),
+                                                           float(diag_add), _ptr(z3), _ptr(f), _ptr(info)),
+                    "latent_forward_batched")
+        self._latent_shape = (n, B, nvec, z.ndim)
+        return f.reshape(z.shape), info
+
+    def latent_backward_batched(self, fbar):
+        """Reverse sweep of the batch recorded by the last latent_forward_batched: fbar has the shape of that call's z.
+        Returns theta_bar (B, 2) = d lp / d (alpha_b, rho_b) and zbar (the shape of z); failed items get NaN."""
+        n, B, nvec, zdim = getattr(self, "_latent_shape", (0, 0, 0, 2))
+        fb = np.ascontiguousarray(fbar, dtype=np.float64)
+        if fb.size != B * nvec * n:
+            raise ValueError("fbar must have the shape of the recorded z")
+        tb = np.empty((B, 2)); zbar = np.empty((B, nvec, n))
+        self._check(self.lib.gpb200_latent_backward_batched(self._h, n, B, nvec, _ptr(fb), _ptr(tb), _ptr(zbar)),
+                    "latent_backward_batched")
+        return tb, zbar.reshape(fb.shape)
+
+    def latent_forward_batched_device(self, n, B, nvec, x, x_stride, theta, diag_add, z, f, info):
+        """Device-pointer variant: x, theta (B x 2), z, f (B*nvec vectors of n) and info (int32) are torch CUDA tensors;
+        the handle must be in device-pointer mode.  Asynchronous on the handle's stream."""
+        assert self.device_pointers
+        self._check(self.lib.gpb200_latent_forward_batched(self._h, n, B, nvec, _ptr(x), x_stride, _ptr(theta), float(diag_add),
+                                                           _ptr(z), _ptr(f), _ptr(info)), "latent_forward_batched")
+
+    def latent_backward_batched_device(self, n, B, nvec, fbar, theta_bar, zbar):
+        """Device-pointer variant of latent_backward_batched (torch CUDA tensors).  Asynchronous on the handle's stream."""
+        assert self.device_pointers
+        self._check(self.lib.gpb200_latent_backward_batched(self._h, n, B, nvec, _ptr(fbar), _ptr(theta_bar), _ptr(zbar)),
+                    "latent_backward_batched")
 
     def _tables(self, Ls, dLdls):
         Ls = [_f(a) for a in Ls]; dLs = [_f(a) for a in dLdls]

@@ -25,6 +25,7 @@ void free_handle(gpb200_handle_s *h) {
   if (h->stream_switch) cudaEventDestroy(h->stream_switch);
   if (h->ws) cudaFree(h->ws);
   if (h->latent_L) cudaFree(h->latent_L);
+  if (h->latent_rec) cudaFree(h->latent_rec);
   if (h->info_slot) cudaFree(h->info_slot);
   if (h->panel_flags) cudaFree(h->panel_flags);
   if (h->flops_dev) cudaFree(h->flops_dev);

@@ -152,6 +152,13 @@ struct Handle {
   double latent_key[4] = {0, 0, 0, 0};
   int latent_n = 0;
   unsigned long long latent_xhash = 0;
+  // record of the last gpb200_latent_forward_batched, read by gpb200_latent_backward_batched (api_latent.cu): the B
+  // padded factors, per-item info and device copies of x, theta and z (diag_add enters the backward sweep only
+  // through L) in one grow-only allocation (not the workspace)
+  void *latent_rec = nullptr;
+  size_t latent_rec_bytes = 0;
+  int latent_rec_valid = 0, latent_rec_n = 0, latent_rec_B = 0, latent_rec_nvec = 0;
+  long long latent_rec_xs = 0;  // x stride in the record: 0 shared, n per item
   int *info_slot = nullptr;     // persistent device word for the single-evaluation entry point in device-pointer mode
   cudaEvent_t stream_switch = nullptr;
   int small_kernel = 1;         // one-CTA whole-evaluation kernel for n <= 128 (env GPB200_SMALL_KERNEL=0 disables)

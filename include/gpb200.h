@@ -231,6 +231,28 @@ GPB200_API int gpb200_latent_forward(gpb200_handle_t h, int n, const double *x, 
 GPB200_API int gpb200_latent_backward(gpb200_handle_t h, int n, const double *x, double alpha, double rho, double diag_add,
                                       int nvec, const double *z, const double *fbar, double *theta_bar, double *zbar);
 
+/* B states of the non-centred latent model in one call (multi-chain samplers, f over a set of posterior draws).  Item b:
+ *   K_b = cov_exp_quad(x_b, alpha_b, rho_b) + diag_add I,  L_b = chol(K_b),  f_{b,m} = L_b z_{b,m}  (m < nvec)
+ * x: per item n doubles, x_stride in doubles (0 = shared, else >= n); theta: B x 2 row-major (alpha, rho);
+ * z, f: B*nvec vectors of length n, vector m of item b at offset (b*nvec + m)*n; info[B] as in
+ * gpb200_lml_grad_batched (items with info != 0 get NaN in f; the others are unaffected).
+ * The handle keeps a record of this call: the B factors and device copies of x, theta and z, so the caller may
+ * overwrite its buffers before the backward call.  All B factors stay on the device (B * 8 * np^2 bytes, np = 128 *
+ * ceil(n / 128)); when they do not fit the call fails.  A call that fails for any reason leaves no record.
+ * gpb200_latent_backward_batched uses that record. */
+GPB200_API int gpb200_latent_forward_batched(gpb200_handle_t h, int n, int B, int nvec, const double *x,
+                                             long long x_stride, const double *theta, double diag_add,
+                                             const double *z, double *f, int *info);
+/* Reverse sweep of the batch recorded by the last gpb200_latent_forward_batched on this handle:
+ * zbar_{b,m} = L_b^T fbar_{b,m};  theta_bar[b] = d lp / d (alpha_b, rho_b) through f and the Cholesky.
+ * n, B, nvec must equal the record's (else, or with no record, a negative status and nothing is launched).
+ * fbar and zbar use the layout of z; theta_bar is B x 2.  Items whose forward info != 0 get NaN.
+ * The record is left unchanged, so backward may be called again.  The single-item gpb200_latent_forward / _backward
+ * neither read nor change the record.  Both batched calls follow the pointer mode; in device-pointer mode neither
+ * synchronises the host. */
+GPB200_API int gpb200_latent_backward_batched(gpb200_handle_t h, int n, int B, int nvec, const double *fbar,
+                                              double *theta_bar, double *zbar);
+
 /* approx_L (covariance.cpp:49-96): cubic-Hermite interpolation in l between tabulated factors;
  * Ls / dLdls are P pointers to n x n column-major tables, lp the P grid points. */
 GPB200_API int gpb200_approx_L(gpb200_handle_t h, int n, double l, int P, const double *lp,
